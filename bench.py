@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # CUDA path (this repo)
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on host cores
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/<name>.npy
 
 Workload (config.workload): Computers-shaped synthetic graph (13,752 nodes / 245,861 edges, seeded
 Chung-Lu, curvature on a 1/1024 grid), target = graph edges, 2-hop vicinity, descriptor 'sum',
@@ -56,7 +57,16 @@ def parse():
                          "nccl = pad + NCCL all-gather + un-permute (torch.distributed)")
     ap.add_argument("--secondary", type=int, default=int(os.environ.get("TLC_BENCH_SECONDARY", "1")),
                     help="1: also measure the other BASELINE.json configurations (a few steps each) into the `secondary` object")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last timed step as DIR/<name>.npy (float32 / "
+                         "float64, at most 64 MB in all): the inputs are seeded, so two builds can be compared output "
+                         "for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl cuda)")
+    return args
 
 
 def make_workload(name, mode="edge", negatives=0):
@@ -99,6 +109,29 @@ def batch_targets(ne, perm, step, rank, world, batch):
     start = ((step * world + rank) * batch) % len(perm)
     idx = perm[np.arange(start, start + batch) % len(perm)]
     return np.ascontiguousarray(ne[idx].astype(np.int32))
+
+
+DUMP_LIMIT = 64 << 20   # bytes of all dumped .npy files together
+
+
+def dump_outputs(path, arrays, seed=0):
+    """{name: array with one row per target} -> path/<name>.npy: float64 stays float64, everything else (fp32 rows,
+    uint8 status) is written as float32.  If the rows do not fit DUMP_LIMIT, the same seeded sample of rows is kept
+    in every array and the sampled row indices are written too (rows.npy)."""
+    os.makedirs(path, exist_ok=True)
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        out[name] = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+    rows = len(next(iter(out.values())))
+    row_bytes = sum(a.nbytes for a in out.values()) / max(rows, 1)
+    budget = DUMP_LIMIT - 4096 * (len(out) + 1)   # (.npy headers)
+    if row_bytes * rows > budget:
+        keep = np.sort(np.random.default_rng(seed).choice(rows, int(budget // (row_bytes + 8)), replace=False))
+        out = {name: a[keep] for name, a in out.items()}
+        out["rows"] = keep.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def config_dict(args, world):
@@ -476,10 +509,12 @@ def run_cuda(args):
             return sv.prepare(global_targets(s))
         return torch.from_numpy(batch_targets(ne, perm, s, rank, world, B)).to(dev)
 
-    def run(x):
+    def run(x):  # -> {name: device array} what the caller receives
         if world > 1:
-            return sv.run(x)   # this rank's shard through the C-ABI, NCCL all-gather of the fp32 rows, un-permute
+            pi, st = sv.run(x)   # this rank's shard through the C-ABI, NCCL all-gather of the fp32 rows, un-permute
+            return {"pi_f32": pi, "status": st}
         g.vicinity_pi_dev(x, out_pi, out_f32, out_st, hop=args.hop, mode=cmode, flags=flags)
+        return {"pi": out_pi, "pi_f32": out_f32, "status": out_st}
 
     def barrier():
         torch.cuda.synchronize()
@@ -504,7 +539,7 @@ def run_cuda(args):
     ev0.record()
     t_wall0 = time.perf_counter()
     for s in range(args.warmup, args.warmup + args.steps):
-        run(batches[s])
+        last = run(batches[s])
         for k, v in stage_ms_of(g).items():
             stage_acc[k] = stage_acc.get(k, 0.0) + v
         alg_bytes += g.last_algorithmic_bytes()
@@ -515,6 +550,8 @@ def run_cuda(args):
     barrier()
     t_wall = time.perf_counter() - t_wall0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:   # (every rank holds the whole table of the step)
+        dump_outputs(args.dump_outputs, last)
     launches = api.launch_count() - launches0
     ks_last = g.last_small()
     table_rows_last = g.last_counts().get("table_route", 0)

@@ -1,7 +1,6 @@
 """TEST INFRASTRUCTURE -- generates tests/golden/*.npz by running the REAL reference
-(/root/reference, imported in place through oracle/ref_harness.py) on small seeded inputs.
-
-Run in the build container only (the GPU box has no /root/reference):
+(a checkout of pkuyzy/TLC-GNN at oracle/_ref/ or $TLC_REFERENCE_ROOT, imported in place through
+oracle/ref_harness.py) on small seeded inputs; needs no GPU:
     python oracle/make_golden.py
 
 Each fixture stores the inputs, the unmodified reference's batch output
@@ -267,5 +266,98 @@ def pimg_cases():
     print("wrote pimg_vectors")
 
 
+# (8) tests/test_oracle_vs_reference.py: its inputs (seeded graphs and targets the other fixtures do not hold: self,
+# repeated, reversed, unknown and far pairs, hop 3, min / max, the KD node generator on a PPI-shaped graph) and what the
+# oracle computes on them.  The tests hold the oracle to these records everywhere and, where a checkout of the original
+# exists, also compare it with the original live on the same inputs.  Written by `--vs-reference-pins` (no checkout
+# needed: the records are the oracle's, not the original's).
+VS_REF_FILE = os.path.join(OUT, "vs_reference_pins.npz")
+VS_REF_BATCH = [("cora", 0.25, 2, False, True), ("pubmed", 0.04, 2, True, True), ("pubmed", 0.04, 2, False, False),
+                ("computers", 0.02, 1, True, True)]
+VS_REF_EDGE = [(3, "sum", True), (1, "max", True), (2, "min", False)]
+VS_REF_STAGE_FIELDS = ("status", "vert", "fval", "pkind", "pbirth", "pdeath", "elo", "ehi", "pos", "neg")
+VS_REF_KD_FIELDS = ("status", "vert", "fval", "pkind", "pbirth", "pdeath", "img")
+
+
+def vs_ref_key(*parts):
+    return "_".join(str(int(p) if isinstance(p, bool) else p) for p in parts)
+
+
+def vs_ref_inputs():
+    """{key: (graph key, graph config, targets or nodes in the graph's own labels)} of every test in
+    test_oracle_vs_reference.py"""
+    def case(name, scale, cont, seed, ntargets):
+        c = gg.make_config(name, scale=scale, continuous=cont)
+        rng = np.random.default_rng(seed)
+        e = c["edges"]
+        tg = e[rng.choice(len(e), ntargets, replace=False)]
+        far = rng.integers(0, c["N"], size=(4, 2))
+        return vs_ref_key("graph", name, scale, cont), c, np.concatenate([tg, far])
+    out = {}
+    for name, scale, hop, cont, ext in VS_REF_BATCH:
+        out[vs_ref_key("batch", name, scale, hop, cont, ext)] = case(name, scale, cont, 11, 24)
+    gk, c, tg = case("pubmed", 0.04, True, 5, 10)
+    out["stages"] = (gk, c, tg[:10])
+    c = gg.make_config("ppi", scale=0.06, continuous=True)
+    labels, _ = gg.relabel_first_appearance(c["edges"])
+    out["kd"] = (vs_ref_key("graph", "ppi", 0.06, True), c, np.random.default_rng(5).choice(labels, 6, replace=False))
+    c = gg.make_config("pubmed", scale=0.04, continuous=True)
+    e = c["edges"]
+    rng = np.random.default_rng(23)
+    pick = e[rng.choice(len(e), 10, replace=False)]
+    un = np.unique(e)
+    tg = np.concatenate([pick, pick[:3], pick[:3, ::-1], np.stack([un[:4], un[:4]], 1), rng.choice(un, size=(6, 2)),
+                         np.array([[10 ** 7, int(un[0])], [int(un[1]), 10 ** 7 + 1]])])
+    out["edge"] = (vs_ref_key("graph", "pubmed", 0.04, True), c, tg)
+    return out
+
+
+def vs_ref_graph(edges, kappa):
+    """-> (oracle graph in first-appearance numbering, label -> id)"""
+    import oracle as orc
+    labels, ne = gg.relabel_first_appearance(edges)
+    return orc.OracleGraph(*gg.build_csr(len(labels), ne, kappa)), {int(l): i for i, l in enumerate(labels)}
+
+
+def vs_ref_map(lut, targets):
+    return np.array([[lut.get(int(a), -1), lut.get(int(b), -1)] for a, b in targets], dtype=np.int32)
+
+
+def vs_reference_pins():
+    import oracle as orc
+    out = {"source": np.array("oracle/tlc_oracle.c, not the original")}
+    for key, (gk, c, tg) in vs_ref_inputs().items():
+        out[gk + "__edges"], out[gk + "__kappa"] = c["edges"].astype(np.int32), c["kappa"]   # (graphs shared by cases: once)
+        out[key + "__graph"], out[key + "__targets"] = np.array(gk), tg
+        og, lut = vs_ref_graph(c["edges"], c["kappa"])
+        if key.startswith("batch"):
+            _, name, scale, hop, cont, ext = key.split("_")
+            r = og.run_batch(vs_ref_map(lut, tg), hop=int(hop), flags=orc.F_NORM | (orc.F_EXTENDED if int(ext) else 0))
+            out[key + "__pi"], out[key + "__cnt"] = r["pi"], np.int64(r["cnt_compute"])
+        elif key == "edge":
+            for hop, desc, ext in VS_REF_EDGE:
+                r = og.run_batch(vs_ref_map(lut, tg), hop=hop, descriptor=desc, flags=orc.F_NORM | (orc.F_EXTENDED if ext else 0))
+                kk = vs_ref_key("edge", hop, desc, ext)
+                out[kk + "__pi"], out[kk + "__cnt"] = r["pi"], np.int64(r["cnt_compute"])
+        elif key == "stages":
+            for i, (a, b) in enumerate(tg):
+                if int(a) in lut and int(b) in lut:
+                    o = og.run_one(lut[int(a)], lut[int(b)], hop=2, flags=orc.F_NORM | orc.F_EXTENDED)
+                    for f in VS_REF_STAGE_FIELDS:
+                        out["stages__%d__%s" % (i, f)] = np.asarray(o[f])
+        else:
+            fl = orc.F_NORM | orc.F_EXTENDED | orc.F_KEEP_ZERO | orc.F_NORM_EPS
+            for i, u in enumerate(tg):
+                for hop in (1, 2):
+                    o = og.run_one(lut[int(u)], lut[int(u)], hop=hop, mode=orc.MODE_NODE, flags=fl)
+                    for f in VS_REF_KD_FIELDS:
+                        out["kd__%d_%d__%s" % (i, hop, f)] = np.asarray(o[f])
+    np.savez_compressed(VS_REF_FILE, **out)
+    print("wrote", os.path.basename(VS_REF_FILE), len(out), "arrays")
+
+
 if __name__ == "__main__":
-    main()
+    if "--vs-reference-pins" in sys.argv:
+        vs_reference_pins()
+    else:
+        main()

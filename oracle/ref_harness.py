@@ -1,10 +1,11 @@
 """TEST INFRASTRUCTURE ONLY -- in-container harness around the *real* reference.
 
-Imports pkuyzy/TLC-GNN in place from /root/reference (read-only) so that
+Imports pkuyzy/TLC-GNN in place from a checkout of it (read-only): oracle/_ref/, which git ignores, or the
+directory named by TLC_REFERENCE_ROOT, so that
   * the C restatement in oracle/tlc_oracle.c can be pinned against it, and
   * golden vectors under tests/golden/ can be generated (oracle/make_golden.py).
 
-/root/reference does not exist on the GPU box, so nothing in the `-m gpu`
+The reference is not part of this repository, so nothing in the `-m gpu`
 tests, smoke() or bench.py imports this module; only `-m "not gpu"` tests that
 skip when the reference tree is absent, and make_golden.py, do.
 
@@ -23,7 +24,7 @@ import types
 
 import numpy as np
 
-REF_ROOT = os.environ.get("TLC_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("TLC_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def available():
@@ -49,7 +50,8 @@ def load():
     if _loaded:
         return types.SimpleNamespace(**_loaded)
     if not available():
-        raise RuntimeError("reference tree not present at %s" % REF_ROOT)
+        raise RuntimeError("no checkout of pkuyzy/TLC-GNN at %s: clone it there or point TLC_REFERENCE_ROOT at one"
+                           % REF_ROOT)
     # The reference's package is called `sg2dgm`, and so is our drop-in mirror.
     # Load the reference under a private package name so both can coexist.
     if "dionysus" not in sys.modules:

@@ -1,5 +1,6 @@
 import os, sys, time
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tlc-gnn_b200')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tlc-gnn_b200"))
 import numpy as np, bench
 from tlc_b200 import _lib as L, api
 c, labels, ne, csr, perm = bench.make_workload("computers")

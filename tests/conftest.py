@@ -9,4 +9,4 @@ for p in (os.path.join(ROOT, "tlc-gnn_b200"), os.path.join(ROOT, "oracle"), os.p
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the reference tree at /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs a checkout of the reference at oracle/_ref/ or $TLC_REFERENCE_ROOT")

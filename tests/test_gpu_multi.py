@@ -60,6 +60,33 @@ def _worker(rank, world, port, out_path, exchange):
     dist.destroy_process_group()
 
 
+@pytest.mark.timeout(900)
+@pytest.mark.parametrize("exchange", ["peer", "nccl"])
+def test_two_gpu_bench_dumps_the_last_timed_step(tmp_path, exchange):
+    """bench.py --dump-outputs on two ranks: rank 0 writes the whole table of the last timed step (both ranks' rows,
+    in the step's target order) and it equals the oracle's rows"""
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two GPUs")
+    import subprocess
+    import sys
+    import bench
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    steps, warmup, batch, world = 3, 1, 256, 2
+    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--standalone", "--nproc_per_node", str(world),
+                          os.path.join(root, "bench.py"), "--workload", "cora", "--batch", str(batch), "--steps", str(steps),
+                          "--warmup", str(warmup), "--secondary", "0", "--no-cpu-baseline", "--exchange", exchange,
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=800)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert sorted(os.listdir(tmp_path)) == ["pi_f32.npy", "status.npy"]
+    _, _, ne, csr, perm = bench.make_workload("cora")
+    s = warmup + steps - 1
+    tg = np.concatenate([bench.batch_targets(ne, perm, s, r, world, batch) for r in range(world)])
+    ref = orc.OracleGraph(*csr).run_batch(tg, hop=2, flags=orc.F_NORM)
+    assert np.array_equal(np.load(tmp_path / "status.npy"), ref["status"].astype(np.float32))
+    den = np.where(ref["pi"] != 0, np.abs(ref["pi"]), 1.0)
+    assert float(np.max(np.abs(np.load(tmp_path / "pi_f32.npy") - ref["pi"]) / den)) < 1e-5
+
+
 @pytest.mark.timeout(600)
 @pytest.mark.parametrize("exchange", ["peer", "nccl"])
 def test_two_gpu_exchange_matches_oracle(tmp_path, exchange):
