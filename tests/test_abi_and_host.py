@@ -64,22 +64,28 @@ def test_call_level_errors_without_gpu():
 
 def test_graph_create_validates_the_csr():
     """a malformed CSR would mean out-of-bounds device accesses: every precondition is checked on the host, before any
-    CUDA call (so this runs without a GPU), and reported through rc / tlc_last_error"""
+    CUDA call (so this runs without a GPU), and reported through rc / tlc_last_error.  tlc_ollivier_ricci shares the
+    validator; it takes no curvatures, so the curvature cases are tlc_graph_create's alone."""
     lib = L.lib()
     h = C.c_void_p()
 
-    def create(rp, col, kap):
+    def create(rp, col, kap, entry="tlc_graph_create"):
         rp = np.asarray(rp, np.int32); col = np.asarray(col, np.int32); kap = np.asarray(kap, np.float64)
-        rc = lib.tlc_graph_create(len(rp) - 1, len(col), rp.ctypes.data, col.ctypes.data, kap.ctypes.data, 0, 0, C.byref(h))
+        if entry == "tlc_graph_create":
+            rc = lib.tlc_graph_create(len(rp) - 1, len(col), rp.ctypes.data, col.ctypes.data, kap.ctypes.data, 0, 0, C.byref(h))
+        else:
+            out = np.zeros(len(col))
+            rc = lib.tlc_ollivier_ricci(0, len(rp) - 1, len(col), rp.ctypes.data, col.ctypes.data, 0.5, out.ctypes.data, None)
         return rc, lib.tlc_last_error().decode()
 
     # path 0 - 1 - 2, well formed except for the one defect under test
-    rc, msg = create([0, 3, 1, 4], [1, 0, 2, 1], [0, 0, 0, 0]);            assert rc == -1 and "monotone" in msg
-    rc, msg = create([0, 1, 3, 4], [1, 0, 7, 1], [0, 0, 0, 0]);            assert rc == -1 and "out of range" in msg
-    rc, msg = create([0, 1, 3, 4], [0, 0, 2, 1], [0, 0, 0, 0]);            assert rc == -1 and "self-loop" in msg
-    rc, msg = create([0, 1, 3, 4], [1, 2, 0, 1], [0, 0, 0, 0]);            assert rc == -1 and "ascending" in msg
-    rc, msg = create([0, 2, 4, 4], [1, 1, 0, 0], [0, 0, 0, 0]);            assert rc == -1 and "ascending" in msg   # duplicate entry
-    rc, msg = create([0, 1, 2, 3], [1, 2, 1], [0, 0, 0]);                  assert rc == -1 and "symmetric" in msg
+    for e in ("tlc_graph_create", "tlc_ollivier_ricci"):
+        rc, msg = create([0, 3, 1, 4], [1, 0, 2, 1], [0, 0, 0, 0], e);         assert rc == -1 and "monotone" in msg, e
+        rc, msg = create([0, 1, 3, 4], [1, 0, 7, 1], [0, 0, 0, 0], e);         assert rc == -1 and "out of range" in msg, e
+        rc, msg = create([0, 1, 3, 4], [0, 0, 2, 1], [0, 0, 0, 0], e);         assert rc == -1 and "self-loop" in msg, e
+        rc, msg = create([0, 1, 3, 4], [1, 2, 0, 1], [0, 0, 0, 0], e);         assert rc == -1 and "ascending" in msg, e
+        rc, msg = create([0, 2, 4, 4], [1, 1, 0, 0], [0, 0, 0, 0], e);         assert rc == -1 and "ascending" in msg, e  # duplicate entry
+        rc, msg = create([0, 1, 2, 3], [1, 2, 1], [0, 0, 0], e);               assert rc == -1 and "symmetric" in msg, e
     rc, msg = create([0, 1, 3, 4], [1, 0, 2, 1], [0.5, 0.25, 0, 0]);       assert rc == -1 and "mirror" in msg      # kappa(0,1) != kappa(1,0)
     rc, msg = create([0, 1, 3, 4], [1, 0, 2, 1], [-1.0, -1.0, 0, 0]);      assert rc == -1 and "kappa + 1" in msg   # weight 0
     rc, msg = create([0, 1, 3, 4], [1, 0, 2, 1], [0, 0, np.nan, np.nan]);  assert rc == -1 and "kappa + 1" in msg

@@ -351,6 +351,7 @@ def test_handed_back_targets_on_the_graph_row_route(monkeypatch):
     pi_c, status_c, cnt_c = g.vicinity_pi(tg, hop=2, flags=L.F_NORM | L.F_DIRECT)
     assert np.array_equal(pi_c, pi) and np.array_equal(status_c, status) and cnt_c == cnt
     assert cn["handed_back"] > 0 and 0 < cn["graph_row_route"] < cn["live"]      # some redone, the rest stayed on the route
+    assert 0 < cn["table_route"] <= cn["graph_row_route"]                       # (the redone targets leave both counts)
     assert np.array_equal(status, o["status"]) and cnt == o["cnt_compute"] and rel_err(pi, o["pi"]) < IMG_TOL
     pi_m, status_m, cnt_m = g.vicinity_pi(tg, hop=2, flags=L.F_NORM | L.F_NO_DIRECT)
     assert np.array_equal(pi, pi_m) and np.array_equal(status, status_m) and cnt == cnt_m

@@ -866,7 +866,7 @@ static void launch_class(const SmallArgs& a, int grid, cudaStream_t st) {
 void launch_small(const GraphView& g, const Params& p, const int32_t* targets, int64_t E, const VicinityScratch& vs,
                   double* out_pi, float* out_pi32, uint8_t* out_status, int32_t* list_b, int32_t* list_c, int32_t* list_big,
                   int* counters, int32_t* out_n, int32_t* out_m, const SmallDiag* diag, SmallStats* stats, int sm_count,
-                  int phases, cudaStream_t st, cudaEvent_t ev_mid2, int32_t* list_b2) {
+                  int phases, cudaStream_t st, int32_t* list_b2) {
   SmallArgs a{};
   a.stats = stats; a.ball_acc = vs.ball_acc;
 #ifdef SMALL_PROFILE
@@ -909,7 +909,6 @@ void launch_small(const GraphView& g, const Params& p, const int32_t* targets, i
       const int grid = (int)std::min<int64_t>(E, (int64_t)sm_count * 3);
       launch_class<128, 256, 4096>(a, std::max(grid, 1), st);
     }
-    if (ev_mid2) cudaEventRecord(ev_mid2, st);
     // class C over the rows class B deferred; what it cannot take either goes back into list_b for the staged pipeline
     a.cls = 2;
     a.list = list_c; a.list_count = counters + 1; a.defer_list = list_b; a.defer_count = counters + 2;

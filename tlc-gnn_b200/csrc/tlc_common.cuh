@@ -265,7 +265,7 @@ struct SmallStats {  // device accumulators of one call
 void launch_small(const GraphView& g, const Params& p, const int32_t* targets, int64_t E, const VicinityScratch& vs,
                   double* out_pi, float* out_pi32, uint8_t* out_status, int32_t* list_b, int32_t* list_c, int32_t* list_big,
                   int* counters, int32_t* out_n, int32_t* out_m, const SmallDiag* diag, SmallStats* stats, int sm_count,
-                  int phases, cudaStream_t st, cudaEvent_t ev_mid2, int32_t* list_b2 = nullptr);
+                  int phases, cudaStream_t st, int32_t* list_b2 = nullptr);
 // rows of a sub-list: sub[i] = targets[list[i]], idx[i] = list[i]
 void launch_gather_targets(const int32_t* targets, const int32_t* list, int64_t k, int32_t* sub, int64_t* idx, cudaStream_t st);
 
