@@ -188,6 +188,31 @@ int tlc_small_diagrams(tlc_graph *g, const int32_t *targets, int64_t E, const tl
                        int32_t *npairs, int32_t *pkind, int32_t *pbv, int32_t *pdv, double *pbirth, double *pdeath,
                        double *out_pi, uint8_t *out_status, int32_t *out_n, int32_t *out_m);
 
+/* Persistence diagrams of a whole batch, on every route the batch call takes (kernel S, the materialised and the
+ * graph-row route, chunking, sub-calls): graph2pi.get_pimg_for_all_edges' diagrams before the imager.  Target t's diagram
+ * is np.array(PD0 + PD1) of riccidist2dgm.py:323-328 in that order -- PD_up, [min,max], PD_down, [max,min], then PD_one
+ * with TLC_F_EXTENDED -- at poff[t] .. poff[t+1], in TARGET order.  TLC_F_ASC_ONLY (not with TLC_F_EXTENDED) keeps PD_up and
+ * [min,max], the pairs of nonzero image weight without extended persistence, and lets the call take the graph-row route.
+ * Every other flag keeps its batch-call meaning.  bv / dv are GRAPH ids (tlc_graph_create numbering).  Targets whose
+ * status is neither OK, TRIVIAL nor NO_TREE_EDGES have no pairs.
+ * Capacity: poff, npairs, *total_pairs, the image rows and the statuses are always written; if *total_pairs > cap the
+ * call returns TLC_E_CAPACITY and leaves the pair arrays untouched (cap = 0: a sizing call; again with cap = *total_pairs
+ * it succeeds).  Output is bit-identical from run to run; image rows and statuses equal tlc_vicinity_pi_dev's. */
+typedef struct {
+  int64_t cap;            /* capacity of the pair arrays, in pairs                                   */
+  int64_t *poff;          /* [E+1] exclusive offsets, target order (required)                        */
+  int32_t *npairs;        /* [E]   pairs per target (may be NULL)                                    */
+  uint8_t *kind;          /* [cap] TLC_K_*                                  any of these may be NULL */
+  int32_t *bv, *dv;       /* [cap] birth / death vertex, graph ids                                   */
+  double *birth, *death;  /* [cap]                                                                   */
+} tlc_diagrams;
+/* DEVICE buffers: targets, every array of *out, dev_out_pi float64[E][res*res] (may be NULL), dev_out_status (may be NULL) */
+int tlc_vicinity_diagrams_dev(tlc_graph *g, const int32_t *dev_targets, int64_t E, const tlc_params *p, tlc_diagrams *out,
+                              double *dev_out_pi, uint8_t *dev_out_status, int64_t *total_pairs);
+/* same, HOST buffers */
+int tlc_vicinity_diagrams(tlc_graph *g, const int32_t *targets, int64_t E, const tlc_params *p, tlc_diagrams *out,
+                          double *out_pi, uint8_t *out_status, int64_t *total_pairs);
+
 /* compute_ricci_curvature (loaddatas.py:105-123): OllivierRicci(G, alpha, method="Sinkhorn").compute_ricci_curvature() on the
  * unweighted graph given as a symmetric CSR (ascending rows, no self-loops) -- the step BEFORE the path, whose output is
  * the `kappa` of tlc_graph_create.  out_kappa[nnz] receives the curvature of every directed entry (both directions of an

@@ -144,6 +144,7 @@ struct SmallArgs {
   int32_t *dbv, *ddv;
   double *dbirth, *ddeath;
   int want_desc;            // run the descending sweep although no loops are wanted (diagram output)
+  int graph_ids;            // diagram output: vertices as graph ids (vert[lid]) instead of local ids
   SmallStats* stats;        // device accumulators (handled rows, sum n, sum m, algorithmic bytes) or nullptr
   const unsigned long long* ball_acc;  // [N][2] per ball: expanded degree sum, rowptr pairs read (byte accounting)
   int cls;                  // 0: class A, 1: class B, 2: class C
@@ -278,6 +279,7 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
   const bool ext = (p.flags & TLC_F_EXTENDED) != 0;
   const bool norm = (p.flags & TLC_F_NORM) != 0;
   const bool do_desc = ext || a.want_desc != 0;
+  auto vid = [&](int x) { return a.graph_ids ? vert[x] : x; };  // diagram output: local -> graph id
   const int W = a.W;
   const int64_t count = a.list ? (int64_t)*a.list_count : a.E;
   const int64_t nteams = (int64_t)gridDim.x * TEAMS;
@@ -603,7 +605,7 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
                 const int max_node = fa > fb ? xa : xb;  // :64
                 if (keep0 || fv[large] < fv[max_node]) {  // :65 (KD :68-69: always)
                   if (lane == 0) {
-                    if (a.poff) { const int64_t o = dpo + np; a.dkind[o] = TLC_K_UP; a.dbv[o] = large; a.ddv[o] = max_node; a.dbirth[o] = fv[large]; a.ddeath[o] = fv[max_node]; }
+                    if (a.poff) { const int64_t o = dpo + np; a.dkind[o] = TLC_K_UP; a.dbv[o] = vid(large); a.ddv[o] = vid(max_node); a.dbirth[o] = fv[large]; a.ddeath[o] = fv[max_node]; }
                     if (((p.img_mask >> TLC_K_UP) & 1u) && fv[max_node] > fv[large]) { pb[2 * npb] = fv[large]; pb[2 * npb + 1] = fv[max_node]; }
                   }
                   if (((p.img_mask >> TLC_K_UP) & 1u) && fv[max_node] > fv[large]) npb++;
@@ -615,7 +617,7 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
               } else {
                 const int min_node = fa < fb ? xa : xb;  // :103-104
                 if (keep0 || fv[small] > fv[min_node]) {  // :105 (KD :108-109: always)
-                  if (lane == 0 && a.poff) { const int64_t o = dpo + np; a.dkind[o] = TLC_K_DOWN; a.dbv[o] = small; a.ddv[o] = min_node; a.dbirth[o] = fv[small]; a.ddeath[o] = fv[min_node]; }
+                  if (lane == 0 && a.poff) { const int64_t o = dpo + np; a.dkind[o] = TLC_K_DOWN; a.dbv[o] = vid(small); a.ddv[o] = vid(min_node); a.dbirth[o] = fv[small]; a.ddeath[o] = fv[min_node]; }
                   np++;  // (PD_down has death <= birth: weight 0 in the image, SURVEY.md F6)
                 }
                 if (lane == 0) { par[small] = (LID)large; negl[nneg] = (uint16_t)el; }  // :107, Neg_edges += [edge]  :99
@@ -651,7 +653,7 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
         // essential pair of the sweep   :110
         if (tid == 0) {
           const int bvx = sweep == 0 ? minv : maxv, dvx = sweep == 0 ? maxv : minv;
-          if (a.poff) { const int64_t o = dpo + np; a.dkind[o] = sweep == 0 ? TLC_K_ESS : TLC_K_ESS_REV; a.dbv[o] = bvx; a.ddv[o] = dvx; a.dbirth[o] = fv[bvx]; a.ddeath[o] = fv[dvx]; }
+          if (a.poff) { const int64_t o = dpo + np; a.dkind[o] = sweep == 0 ? TLC_K_ESS : TLC_K_ESS_REV; a.dbv[o] = vid(bvx); a.ddv[o] = vid(dvx); a.dbirth[o] = fv[bvx]; a.ddeath[o] = fv[dvx]; }
           if (sweep == 0 && ((p.img_mask >> TLC_K_ESS) & 1u) && fv[dvx] > fv[bvx]) { pb[2 * npb] = fv[bvx]; pb[2 * npb + 1] = fv[dvx]; }
         }
         if (sweep == 0 && ((p.img_mask >> TLC_K_ESS) & 1u) && fv[maxv] > fv[minv]) npb++;
@@ -727,7 +729,7 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
                 const int lvv = fv[la] >= fv[lb] ? la : lb;   // large_value = max(old[large_edge])
                 const int lov = fv[p0] <= fv[p1] ? p0 : p1;   // low_value   = min(old[pos_edge])
                 if (keep0 || fv[lvv] > fv[lov]) {  // :160-165 (KD :169-170: always)
-                  if (a.poff) { const int64_t o = dpo + np; a.dkind[o] = TLC_K_ONE; a.dbv[o] = lov; a.ddv[o] = lvv; a.dbirth[o] = fv[lov]; a.ddeath[o] = fv[lvv]; }
+                  if (a.poff) { const int64_t o = dpo + np; a.dkind[o] = TLC_K_ONE; a.dbv[o] = vid(lov); a.ddv[o] = vid(lvv); a.dbirth[o] = fv[lov]; a.ddeath[o] = fv[lvv]; }
                   np++;
                   if (((p.img_mask >> TLC_K_ONE) & 1u) && fv[lvv] > fv[lov]) { pb[2 * npb] = fv[lov]; pb[2 * npb + 1] = fv[lvv]; npb++; }
                 }
@@ -887,7 +889,7 @@ void launch_small(const GraphView& g, const Params& p, const int32_t* targets, i
   a.out_n = out_n; a.out_m = out_m;
   if (diag) {
     a.poff = diag->poff; a.dnp = diag->np; a.dkind = diag->kind; a.dbv = diag->bv; a.ddv = diag->dv;
-    a.dbirth = diag->birth; a.ddeath = diag->death; a.want_desc = 1;
+    a.dbirth = diag->birth; a.ddeath = diag->death; a.want_desc = diag->want_desc; a.graph_ids = diag->graph_ids;
   }
   if (phases & 1) {
     cudaMemsetAsync(counters, 0, 8 * sizeof(int), st);

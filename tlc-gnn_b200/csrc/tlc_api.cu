@@ -100,6 +100,48 @@ struct CallStats {
   }
 };
 
+// grow b to `need` bytes keeping its first `used` bytes (DevBuf::reserve frees before it allocates and loses them)
+static cudaError_t grow_keep(DevBuf& b, size_t used, size_t need, cudaStream_t st) {
+  if (b.p && need <= b.bytes) return cudaSuccess;
+  DevBuf nb;
+  cudaError_t e = nb.reserve(need);
+  if (e == cudaSuccess && used) e = cudaMemcpyAsync(nb.p, b.p, used, cudaMemcpyDeviceToDevice, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e == cudaSuccess) b = std::move(nb);
+  return e;
+}
+
+// a pair array set owned by the graph: capacity in pairs, grow-only
+struct PairBufs {
+  DevBuf kind, bv, dv, birth, death;
+  int64_t cap = 0;
+  DiagArea view() const {
+    return DiagArea{kind.as<uint8_t>(), bv.as<int32_t>(), dv.as<int32_t>(), birth.as<double>(), death.as<double>()};
+  }
+  // room for `need` pairs; the first `used` pairs are kept
+  cudaError_t grow(int64_t used, int64_t need, cudaStream_t st) {
+    if (need <= cap && kind.p) return cudaSuccess;
+    const int64_t n = std::max<int64_t>(need, cap + cap / 2);
+    cudaError_t e = cudaSuccess;
+    DevBuf* bufs[5] = {&kind, &bv, &dv, &birth, &death};
+    const size_t sz[5] = {1, 4, 4, 8, 8};
+    for (int i = 0; i < 5 && e == cudaSuccess; i++) e = grow_keep(*bufs[i], (size_t)used * sz[i], (size_t)n * sz[i] + 16, st);
+    if (e == cudaSuccess) cap = n;
+    return e;
+  }
+};
+
+// the pairs of a tlc_vicinity_diagrams call while it runs.  Every target's diagram is one contiguous segment of the
+// staging: kernel S writes its rows into `small` at offsets fixed before it runs, the staged pipeline's chunks are
+// exported into `staged` (staging offsets >= small_total); np / soff record count and offset per target of the call.
+struct DiagCollect {
+  bool on = false;
+  DevBuf np, soff, poff;  // [E] int32, [E] int64, [E + 1] int64 (host entry point: the final offsets)
+  PairBufs small, staged, out;  // out: the host entry point's gathered arrays before they are copied back
+  int64_t small_total = 0, staged_used = 0;
+  DevBuf chunk;  // per chunk: staging offset and call row of each target
+};
+
 struct tlc_graph {
   int device = 0;
   GraphView gv{};  // views of rowptr / col / kappa / rec
@@ -164,6 +206,7 @@ struct tlc_graph {
   int64_t px_cap = 0;
   std::vector<cudaEvent_t> ev_pool;  // stage-timing events, reused from call to call
   int sm_count = 0;
+  DiagCollect dg;
 
   ~tlc_graph() {
     for (void* q : peer_opened) cudaIpcCloseMemHandle(q);
@@ -718,13 +761,42 @@ static int copy_detail(tlc_detail* detail, const ChunkView& c, const Packed& k, 
 
 static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const tlc_params* up, double* d_pi,
                       float* d_pi32, uint8_t* d_status, int64_t* cnt_compute, tlc_detail* detail, CallStats& s,
-                      size_t ev_base);
+                      size_t ev_base, const int64_t* drow = nullptr);
+
+// diagram call: the pairs of a finished chunk into the staging area.  tidx: the chunk's rows of this (sub-)call, drow:
+// their rows in the diagram call (NULL: the same); skip[t] != 0: target t is redone by a later sub-call, not exported.
+static int export_chunk(tlc_graph* g, const ChunkView& c, int64_t T, const int64_t* tidx, const int64_t* drow,
+                        const std::vector<uint8_t>& skip) {
+  DiagCollect& d = g->dg;
+  cudaStream_t st = g->stream;
+  std::vector<int32_t> tnp((size_t)T);
+  std::vector<uint8_t> tst((size_t)T);
+  CK(cudaMemcpyAsync(tnp.data(), c.tnp, (size_t)T * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(tst.data(), c.tstatus, (size_t)T, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  std::vector<int64_t> h((size_t)T * 2);  // [T] staging offsets | [T] rows of the diagram call
+  int64_t sum = 0;
+  for (int64_t t = 0; t < T; t++) {
+    const bool redone = !skip.empty() && skip[(size_t)t];
+    h[(size_t)t] = d.small_total + d.staged_used + sum;
+    h[(size_t)(T + t)] = redone ? -1 : (drow ? drow[tidx[t]] : tidx[t]);
+    if (!redone) sum += diag_pairs(tst[(size_t)t], tnp[(size_t)t]);
+  }
+  CK(d.staged.grow(d.staged_used, d.staged_used + sum, st));
+  CK(d.chunk.reserve((size_t)T * 16));
+  CK(cudaMemcpyAsync(d.chunk.p, h.data(), (size_t)T * 16, cudaMemcpyHostToDevice, st));
+  launch_export_pairs(c, d.chunk.as<int64_t>(), d.chunk.as<int64_t>() + T, d.staged.view(), d.small_total,
+                      d.np.as<int32_t>(), d.soff.as<int64_t>(), g->sm_count, st);
+  CK(cudaStreamSynchronize(st));
+  d.staged_used += sum;
+  return TLC_OK;
+}
 
 // the targets kernel 3v handed back on a graph-row batch call, as their own call on the materialised route; rows scattered
 // back.  The targets are counted already: of the redo's statistics only its chunks and stage times are added to s.
 static int redo_handed_back(tlc_graph* g, const int32_t* d_targets, int64_t E, const std::vector<int64_t>& redo,
                             const tlc_params* up, double* d_pi, float* d_pi32, uint8_t* d_status, size_t ev_base,
-                            CallStats& s) {
+                            CallStats& s, const int64_t* drow) {
   cudaStream_t st = g->stream;
   const int r2 = up->resolution * up->resolution;
   const int64_t k = (int64_t)redo.size();
@@ -745,9 +817,11 @@ static int redo_handed_back(tlc_graph* g, const int32_t* d_targets, int64_t E, c
   CK(cudaStreamSynchronize(st));
   tlc_params up2 = *up;
   up2.flags = (up2.flags | TLC_F_NO_DIRECT) & ~TLC_F_DIRECT;
+  std::vector<int64_t> rows((size_t)k);  // diagram call: the redone targets' rows in it
+  for (int64_t i = 0; i < k; i++) rows[(size_t)i] = drow ? drow[redo[i]] : redo[i];
   CallStats sub;
   const int rc = run_staged(g, b_sub.as<int32_t>(), k, &up2, b_pi.as<double>(), b_pi32.as<float>(), b_st.as<uint8_t>(),
-                            nullptr, nullptr, sub, ev_base);
+                            nullptr, nullptr, sub, ev_base, rows.data());
   if (rc) return rc;
   launch_scatter_rows(b_pi.as<double>(), d_pi32 ? b_pi32.as<float>() : nullptr, d_status ? b_st.as<uint8_t>() : nullptr,
                       b_idx.as<int64_t>(), k, r2, d_pi, d_pi32, d_status, g->sm_count, st);
@@ -762,7 +836,7 @@ static int redo_handed_back(tlc_graph* g, const int32_t* d_targets, int64_t E, c
 // (a nested call's live behind its caller's).
 static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const tlc_params* up, double* d_pi,
                       float* d_pi32, uint8_t* d_status, int64_t* cnt_compute, tlc_detail* detail, CallStats& s,
-                      size_t ev_base) {
+                      size_t ev_base, const int64_t* drow) {
   s = CallStats();
   if (E < 0 || E >= ((int64_t)1 << 32)) return fail(TLC_E_INVALID, "E must be in [0, 2^32)");
   CK(cudaSetDevice(g->device));
@@ -785,7 +859,9 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
 
   // ---- route, one per call ----
   const int64_t Wd = ((int64_t)g->gv.N + 31) / 32;
-  const bool want_desc_call = ((p.flags & TLC_F_EXTENDED) != 0 || detail != nullptr) && !(p.flags & TLC_F_ASC_ONLY);
+  // (pair output -- detail or diagram call -- wants PD_down and [max,min] unless TLC_F_ASC_ONLY)
+  const bool want_pairs = detail != nullptr || g->dg.on;
+  const bool want_desc_call = ((p.flags & TLC_F_EXTENDED) != 0 || want_pairs) && !(p.flags & TLC_F_ASC_ONLY);
   const bool direct_ok = g->ball_cache.p != nullptr && g->gminw.p != nullptr && !want_desc_call && !bad_desc &&
                          p.mode <= TLC_MODE_NODE && !(p.flags & TLC_F_FILT_ANY_STRUCT) &&
                          !(p.flags & (TLC_F_NO_DIRECT | TLC_F_EDGE_SORTED)) && (size_t)Wd * 8 <= 64 * 1024;
@@ -856,13 +932,14 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
     CK(cudaMemcpyAsync((void*)(c.voff + k.T), &k.Nv, 8, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync((void*)(c.eoff + k.T), &k.Ne, 8, cudaMemcpyHostToDevice, st));
     const std::vector<SubRange> subs = split_subranges(g, order, pos, k.T, h.n);
+    std::vector<uint8_t> fbv;  // graph-row batch call: targets kernel 3v handed back (redone below)
     if (direct) {
       c.count_m = light ? 1 : 0;
       // tm: counted by kernel 1b (batch call) or known from the full counting pass (detail call)
       if (!light) CK(cudaMemcpyAsync((void*)c.tm, h.tm + pos, (size_t)k.T * 4, cudaMemcpyHostToDevice, st));
       int fb0 = 0, fb1 = 0;
       CK(cudaMemcpyAsync(&fb0, fb_counters, sizeof(int), cudaMemcpyDeviceToHost, st));
-      s.table += run_stages(g, p, c, k.n_max, k.m_max, subs, d_pi, d_pi32, d_status, detail != nullptr, tm, use_table);
+      s.table += run_stages(g, p, c, k.n_max, k.m_max, subs, d_pi, d_pi32, d_status, want_pairs, tm, use_table);
       CK(cudaMemcpyAsync(&fb1, fb_counters, sizeof(int), cudaMemcpyDeviceToHost, st));
       if (light) CK(cudaMemcpyAsync(h.tm + pos, c.tm, (size_t)k.T * 4, cudaMemcpyDeviceToHost, st));
       CK(cudaStreamSynchronize(st));
@@ -873,7 +950,7 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
       if (fb1 != fb0) {
         // kernel 3v handed targets back: their edge-sorted sweep needs the adjacency
         if (light) {  // no adjacency space was reserved: those targets are redone on the materialised route below
-          std::vector<uint8_t> fbv((size_t)k.T);
+          fbv.resize((size_t)k.T);
           CK(cudaMemcpyAsync(fbv.data(), c.tfb, (size_t)k.T, cudaMemcpyDeviceToHost, st));
           CK(cudaStreamSynchronize(st));
           for (const SubRange& r : subs)
@@ -888,14 +965,15 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
           c.dbm = nullptr;
           c.W = 0;
           s.direct -= k.T;
-          run_stages(g, p, c, k.n_max, k.m_max, subs, d_pi, d_pi32, d_status, detail != nullptr, tm, use_table);
+          run_stages(g, p, c, k.n_max, k.m_max, subs, d_pi, d_pi32, d_status, want_pairs, tm, use_table);
         }
       }
     } else {
-      run_stages(g, p, c, k.n_max, k.m_max, subs, d_pi, d_pi32, d_status, detail != nullptr, tm, use_table);
+      run_stages(g, p, c, k.n_max, k.m_max, subs, d_pi, d_pi32, d_status, want_pairs, tm, use_table);
     }
     s.chunks++;
     CK(cudaStreamSynchronize(st));
+    if (g->dg.on && (rc = export_chunk(g, c, k.T, h.tidx + pos, drow, fbv))) return rc;
     if (detail) {
       g->detail_chunk = c;
       if ((rc = copy_detail(detail, c, k, h.voff + pos, h.eoff + pos, p))) return rc;
@@ -904,7 +982,7 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
   }
   if (!redo.empty()) {
     tm.collect(s.stage_ms);
-    if ((rc = redo_handed_back(g, d_targets, E, redo, up, d_pi, d_pi32, d_status, tm.used, s))) return rc;
+    if ((rc = redo_handed_back(g, d_targets, E, redo, up, d_pi, d_pi32, d_status, tm.used, s, drow))) return rc;
   }
   if (tm.on) {
     cudaEventRecord(ev_total1, st);
@@ -968,8 +1046,8 @@ static constexpr size_t SM_STATS_OFF = 32;  // SmallStats behind the eight list 
 static bool small_applicable(const tlc_graph* g, const tlc_params* up, int64_t E, const tlc_detail* detail) {
   if (detail || E <= 0 || E >= ((int64_t)1 << 31)) return false;
   if (up->resolution != 5 || up->descriptor < 0 || up->descriptor > 2) return false;
-  if (up->flags & (TLC_F_FILT_ANY_STRUCT | TLC_F_EDGE_SORTED | TLC_F_DIRECT |
-                   TLC_F_NO_DIRECT | TLC_F_NO_SMALL | TLC_F_ASC_ONLY)) return false;
+  if (up->flags & (TLC_F_FILT_ANY_STRUCT | TLC_F_EDGE_SORTED | TLC_F_DIRECT | TLC_F_NO_DIRECT | TLC_F_NO_SMALL |
+                   (g->dg.on ? 0u : TLC_F_ASC_ONLY))) return false;  // (the diagram call: kernel S skips the descending sweep)
   if (getenv("TLC_NO_SMALL")) return false;
   return true;
 }
@@ -988,13 +1066,51 @@ static int run_staged_list(tlc_graph* g, const int32_t* d_targets, const int32_t
   float* pi32 = g->sm_pi32.as<float>();
   uint8_t* sst = g->sm_st.as<uint8_t>();
   launch_gather_targets(d_targets, d_list, k, sub, idx, st);
+  std::vector<int64_t> rows;  // diagram call: the sub-list's rows in it
+  if (g->dg.on) {
+    rows.resize((size_t)k);
+    CK(cudaMemcpyAsync(rows.data(), idx, (size_t)k * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+  }
   tlc_params up2 = *up;
   up2.flags |= TLC_F_NO_SMALL;
   CallStats part;
-  if ((rc = run_staged(g, sub, k, &up2, pi, pi32, sst, nullptr, nullptr, part, ev_base))) return rc;
+  if ((rc = run_staged(g, sub, k, &up2, pi, pi32, sst, nullptr, nullptr, part, ev_base, g->dg.on ? rows.data() : nullptr)))
+    return rc;
   launch_scatter_rows(pi, d_pi32 ? pi32 : nullptr, d_status ? sst : nullptr, idx, k, r2, d_pi, d_pi32, d_status, g->sm_count, st);
   CK(cudaStreamSynchronize(st));
   s += part;
+  return TLC_OK;
+}
+
+// diagram call: kernel S's staging area.  The counting pass bounds the pairs of every row kernel S can finish (<= 1024
+// vertices, <= 4096 edges) by n + m + 2 (ascending sweep only: n + 2), the other rows by 0; the row's segment starts at
+// the exclusive prefix of those bounds (dg.soff, which the staged export overwrites for the rows it takes)
+static int small_diagram_area(tlc_graph* g, const Params& p, const int32_t* d_targets, int64_t E, const VicinityScratch& vs,
+                              SmallDiag* out) {
+  DiagCollect& d = g->dg;
+  cudaStream_t st = g->stream;
+  launch_vicinity_sizes(g->gv, p, d_targets, E, g->d_n.as<int32_t>(), g->d_m.as<int32_t>(), g->d_ds.as<int32_t>(),
+                        g->d_st.as<uint8_t>(), g->d_bytes.as<double>(), vs, g->work_counter.as<int>(), st);
+  std::vector<int32_t> n((size_t)E), m((size_t)E);
+  CK(cudaMemcpyAsync(n.data(), g->d_n.p, (size_t)E * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(m.data(), g->d_m.p, (size_t)E * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  const bool asc = (p.flags & TLC_F_ASC_ONLY) != 0;
+  std::vector<int64_t> off((size_t)E);
+  int64_t total = 0;
+  for (int64_t i = 0; i < E; i++) {
+    off[(size_t)i] = total;
+    if (n[(size_t)i] <= 1024 && m[(size_t)i] <= 4096) total += n[(size_t)i] + (asc ? 0 : m[(size_t)i]) + 2;
+  }
+  CK(d.small.grow(0, total, st));
+  CK(cudaMemcpyAsync(d.soff.p, off.data(), (size_t)E * 8, cudaMemcpyHostToDevice, st));
+  CK(cudaStreamSynchronize(st));
+  d.small_total = total;
+  const DiagArea a = d.small.view();
+  *out = SmallDiag{d.soff.as<int64_t>(), d.np.as<int32_t>(), a.kind, a.bv, a.dv, a.birth, a.death};
+  out->graph_ids = 1;
+  out->want_desc = asc ? 0 : 1;
   return TLC_OK;
 }
 
@@ -1024,13 +1140,17 @@ static int run_small(tlc_graph* g, const int32_t* d_targets, int64_t E, const tl
   int32_t *list_b = g->sm_list_b.as<int32_t>(), *list_c = g->sm_list_c.as<int32_t>();
   int32_t *list_big = g->sm_list_big.as<int32_t>(), *list_b2 = g->sm_list_b2.as<int32_t>();
   launch_ball_cache(g->gv, p, d_targets, E, vs, st);
+  SmallDiag dgs{};
+  const SmallDiag* diag = nullptr;
+  if (g->dg.on && (rc = small_diagram_area(g, p, d_targets, E, vs, &dgs))) return rc;
+  if (g->dg.on) diag = &dgs;
   if (ev0) cudaEventRecord(ev0, st);
   launch_small(g->gv, p, d_targets, E, vs, d_pi, d_pi32, d_status, list_b, list_c, list_big, counters,
-               nullptr, nullptr, nullptr, d_stats, g->sm_count, 1, st);
+               nullptr, nullptr, diag, d_stats, g->sm_count, 1, st);
   if (ev1) cudaEventRecord(ev1, st);
   // the rows class A deferred, routed by their exact sizes: class B, class C and the staged pipeline then run side by side
   launch_small(g->gv, p, d_targets, E, vs, d_pi, d_pi32, d_status, list_b, list_c, list_big, counters,
-               nullptr, nullptr, nullptr, d_stats, g->sm_count, 4, st, list_b2);
+               nullptr, nullptr, diag, d_stats, g->sm_count, 4, st, list_b2);
   CK(cudaEventRecord(g->ev_small_a, st));
   CK(cudaMemcpyAsync(g->sm_host.p, g->sm_dev.p, 32, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
@@ -1046,7 +1166,7 @@ static int run_small(tlc_graph* g, const int32_t* d_targets, int64_t E, const tl
     if (sb != st) CK(cudaStreamWaitEvent(sb, g->ev_small_a, 0));
     if (evb0) cudaEventRecord(evb0, sb);
     launch_small(g->gv, p, d_targets, E, vs, d_pi, d_pi32, d_status, list_b, list_c, list_big, counters,
-                 nullptr, nullptr, nullptr, d_stats, g->sm_count, 8, sb, list_b2);
+                 nullptr, nullptr, diag, d_stats, g->sm_count, 8, sb, list_b2);
     if (ev1b) cudaEventRecord(ev1b, sb);
     if (sb != st) CK(cudaEventRecord(g->ev_small_bc, sb));
   }
@@ -1054,7 +1174,7 @@ static int run_small(tlc_graph* g, const int32_t* d_targets, int64_t E, const tl
     if (sc != st) CK(cudaStreamWaitEvent(sc, g->ev_small_a, 0));
     if (evc0) cudaEventRecord(evc0, sc);
     launch_small(g->gv, p, d_targets, E, vs, d_pi, d_pi32, d_status, list_b, list_c, list_big, counters,
-                 nullptr, nullptr, nullptr, d_stats, g->sm_count, 16, sc, list_b2);
+                 nullptr, nullptr, diag, d_stats, g->sm_count, 16, sc, list_b2);
     if (ev2) cudaEventRecord(ev2, sc);
     if (sc != st) CK(cudaEventRecord(g->ev_small_c, sc));
   }
@@ -1397,6 +1517,117 @@ int tlc_small_diagrams(tlc_graph* g, const int32_t* targets, int64_t E, const tl
   CK(cudaGetLastError());
   if (pkind) for (int64_t i = 0; i < P; i++) pkind[i] = k8[(size_t)i];
   return TLC_OK;
+}
+
+}  // extern "C"
+
+// the checks of both diagram entry points, before any CUDA call
+static int check_diagram_args(tlc_graph* g, const int32_t* targets, int64_t E, const tlc_params* p, const tlc_diagrams* out) {
+  if (!g) return fail(TLC_E_INVALID, "graph is NULL");
+  if (!out || !out->poff) return fail(TLC_E_INVALID, "out and out->poff are required");
+  if (out->cap < 0) return fail(TLC_E_INVALID, "out->cap must be >= 0");
+  if (E < 0 || E >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "E must be in [0, 2^31)");
+  if (E > 0 && !targets) return fail(TLC_E_INVALID, "targets is NULL");
+  return check_params(p);
+}
+
+// the whole path over device-resident targets with pair collection; poff[0..E] (device) receives the final offsets,
+// *total their sum.  The pairs stay in the staging until gather_diagrams.
+static int run_diagrams(tlc_graph* g, const int32_t* d_targets, int64_t E, const tlc_params* p, double* d_pi,
+                        uint8_t* d_status, int64_t* d_poff, int64_t* total) {
+  DiagCollect& d = g->dg;
+  cudaStream_t st = g->stream;
+  CK(d.np.reserve((size_t)E * 4));
+  CK(d.soff.reserve((size_t)E * 8));
+  CK(cudaMemsetAsync(d.np.p, 0, (size_t)E * 4, st));  // targets no stage finishes have no pairs
+  d.small_total = 0;
+  d.staged_used = 0;
+  d.on = true;
+  const int rc = run_pipeline(g, d_targets, E, p, d_pi, nullptr, d_status, nullptr, nullptr);
+  d.on = false;
+  if (rc) return rc;
+  launch_scan_counts(d.np.as<int32_t>(), E, d_poff, st);
+  CK(cudaMemcpyAsync(total, d_poff + E, 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+  return TLC_OK;
+}
+
+static void gather_diagrams(tlc_graph* g, int64_t E, const int64_t* d_poff, const DiagArea& out) {
+  const DiagCollect& d = g->dg;
+  launch_gather_pairs(d.np.as<int32_t>(), d.soff.as<int64_t>(), d_poff, E, d.small.view(), d.staged.view(), d.small_total,
+                      out, g->sm_count, g->stream);
+}
+
+static int capacity_error(int64_t total, int64_t cap) {
+  return fail(TLC_E_CAPACITY, "the diagrams hold " + std::to_string(total) + " pairs, out->cap is " + std::to_string(cap));
+}
+
+extern "C" {
+
+int tlc_vicinity_diagrams_dev(tlc_graph* g, const int32_t* dev_targets, int64_t E, const tlc_params* p, tlc_diagrams* out,
+                              double* dev_out_pi, uint8_t* dev_out_status, int64_t* total_pairs) {
+  int rc = check_diagram_args(g, dev_targets, E, p, out);
+  if (rc) return rc;
+  CK(cudaSetDevice(g->device));
+  cudaStream_t st = g->stream;
+  int64_t total = 0;
+  if (E == 0) {
+    CK(cudaMemsetAsync(out->poff, 0, 8, st));
+    CK(cudaStreamSynchronize(st));
+  } else {
+    double* d_pi = dev_out_pi;
+    if (!d_pi) {  // the image rows are computed anyway: the graph's grow-only staging takes them
+      if ((rc = ensure_io_buffers(g, E, p->resolution * p->resolution))) return rc;
+      d_pi = g->io_pi.as<double>();
+    }
+    if ((rc = run_diagrams(g, dev_targets, E, p, d_pi, dev_out_status, out->poff, &total))) return rc;
+    if (out->npairs) CK(cudaMemcpyAsync(out->npairs, g->dg.np.p, (size_t)E * 4, cudaMemcpyDeviceToDevice, st));
+    if (total <= out->cap) gather_diagrams(g, E, out->poff, DiagArea{out->kind, out->bv, out->dv, out->birth, out->death});
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+  }
+  if (total_pairs) *total_pairs = total;
+  return total > out->cap ? capacity_error(total, out->cap) : TLC_OK;
+}
+
+int tlc_vicinity_diagrams(tlc_graph* g, const int32_t* targets, int64_t E, const tlc_params* p, tlc_diagrams* out,
+                          double* out_pi, uint8_t* out_status, int64_t* total_pairs) {
+  int rc = check_diagram_args(g, targets, E, p, out);
+  if (rc) return rc;
+  CK(cudaSetDevice(g->device));
+  cudaStream_t st = g->stream;
+  int64_t total = 0;
+  out->poff[0] = 0;
+  if (E > 0) {
+    const int r2 = p->resolution * p->resolution;
+    if ((rc = ensure_io_buffers(g, E, r2))) return rc;  // grow-only device staging shared with tlc_vicinity_pi
+    int32_t* d_t = g->io_t.as<int32_t>();
+    double* d_pi = g->io_pi.as<double>();
+    uint8_t* d_st = g->io_st.as<uint8_t>();
+    DiagCollect& d = g->dg;
+    CK(d.poff.reserve((size_t)(E + 1) * 8));
+    CK(cudaMemcpyAsync(d_t, targets, (size_t)E * 8, cudaMemcpyHostToDevice, st));
+    if ((rc = run_diagrams(g, d_t, E, p, d_pi, d_st, d.poff.as<int64_t>(), &total))) return rc;
+    CK(cudaMemcpyAsync(out->poff, d.poff.p, (size_t)(E + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (out->npairs) CK(cudaMemcpyAsync(out->npairs, d.np.p, (size_t)E * 4, cudaMemcpyDeviceToHost, st));
+    if (out_pi) CK(cudaMemcpyAsync(out_pi, d_pi, (size_t)E * r2 * 8, cudaMemcpyDeviceToHost, st));
+    if (out_status) CK(cudaMemcpyAsync(out_status, d_st, (size_t)E, cudaMemcpyDeviceToHost, st));
+    if (total <= out->cap && total > 0) {
+      CK(d.out.grow(0, total, st));
+      const DiagArea a = d.out.view();
+      gather_diagrams(g, E, d.poff.as<int64_t>(), a);
+      if (out->kind) CK(cudaMemcpyAsync(out->kind, a.kind, (size_t)total, cudaMemcpyDeviceToHost, st));
+      if (out->bv) CK(cudaMemcpyAsync(out->bv, a.bv, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
+      if (out->dv) CK(cudaMemcpyAsync(out->dv, a.dv, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
+      if (out->birth) CK(cudaMemcpyAsync(out->birth, a.birth, (size_t)total * 8, cudaMemcpyDeviceToHost, st));
+      if (out->death) CK(cudaMemcpyAsync(out->death, a.death, (size_t)total * 8, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+  }
+  if (total_pairs) *total_pairs = total;
+  return total > out->cap ? capacity_error(total, out->cap) : TLC_OK;
 }
 
 int tlc_ollivier_ricci(int device, int32_t N, int64_t nnz, const int32_t* rowptr, const int32_t* col, double alpha,

@@ -256,6 +256,8 @@ struct SmallDiag {  // optional diagram output: pairs of row t at poff[t] (capac
   uint8_t* kind;
   int32_t *bv, *dv;
   double *birth, *death;
+  int graph_ids = 0;  // 1: birth / death vertices as graph ids (default: local ids)
+  int want_desc = 1;  // 0: ascending sweep only (PD_up and [min,max])
 };
 struct SmallStats {  // device accumulators of one call
   unsigned long long handled[3];  // rows finished by class A / B / C (any status)
@@ -268,6 +270,26 @@ void launch_small(const GraphView& g, const Params& p, const int32_t* targets, i
                   int phases, cudaStream_t st, int32_t* list_b2 = nullptr);
 // rows of a sub-list: sub[i] = targets[list[i]], idx[i] = list[i]
 void launch_gather_targets(const int32_t* targets, const int32_t* list, int64_t k, int32_t* sub, int64_t* idx, cudaStream_t st);
+
+// kernel 7 (k7_diagrams.cu): the diagrams of a batch call.  A pair array set (structure of arrays, graph vertex ids).
+struct DiagArea {
+  uint8_t* kind;
+  int32_t *bv, *dv;
+  double *birth, *death;
+};
+// pairs a target's diagram holds: those of the statuses kernel S and the staged pipeline report pairs for
+__host__ __device__ inline int diag_pairs(uint8_t status, int32_t np) {
+  return (status <= TLC_ST_TRIVIAL || status == TLC_ST_NO_TREE_EDGES) && np > 0 ? np : 0;
+}
+// the chunk's pairs into `area` at dst[t] - area_base, graph ids; np_out / soff_out[rows[t]] = count / dst[t] (rows[t] < 0: skipped)
+void launch_export_pairs(const ChunkView& c, const int64_t* dst, const int64_t* rows, const DiagArea& area,
+                         int64_t area_base, int32_t* np_out, int64_t* soff_out, int sm_count, cudaStream_t st);
+// poff[0..E] = exclusive scan of np[0..E)
+void launch_scan_counts(const int32_t* np, int64_t E, int64_t* poff, cudaStream_t st);
+// out[poff[t] ..] = segment t of the staging (offsets soff[t] < split_at in a, the others in b at soff[t] - split_at);
+// NULL arrays of `out` are skipped
+void launch_gather_pairs(const int32_t* np, const int64_t* soff, const int64_t* poff, int64_t E, const DiagArea& a,
+                         const DiagArea& b, int64_t split_at, const DiagArea& out, int sm_count, cudaStream_t st);
 
 // multi-GPU exchange by peer stores (k5_gather.cu): the tables of all ranks, this rank's own included
 constexpr int PEER_MAX = 16;

@@ -218,6 +218,23 @@ class graph2pi():
             tg, hop=hop, descriptor=desc, resolution=resolution, flags=self._flags(True, extended_flag),
             out=self.pi_sg)
 
+    def get_pdgm_for_all_edges(self, total_edges, cores, hop=2, norm=True, extended_flag=False, descriptor='min'):
+        """The diagram counterpart of get_pimg_for_all_edges: self.pd_sg is a list with one float64 [K, 2] (birth,
+        death) array per target -- np.array(PD0 + PD1) of riccidist2dgm.py:323-328, the array the reference hands to
+        the imager -- empty for targets whose image the reference zeroes; self.pd_status holds the statuses."""
+        self.t1 = time.time()
+        E = len(total_edges)
+        self.pd_sg = [np.zeros((0, 2)) for _ in range(E)]
+        self.pd_status = np.zeros(E, np.uint8)
+        if E == 0:
+            return
+        desc = descriptor if descriptor in _DESCRIPTORS else -1
+        d = self._graph.vicinity_diagrams(self._map_targets(total_edges), hop=hop, descriptor=desc,
+                                          flags=self._flags(True, extended_flag))
+        bd = np.stack([d["birth"], d["death"]], axis=1)
+        self.pd_sg = [bd[d["poff"][i]:d["poff"][i + 1]] for i in range(E)]
+        self.pd_status = d["status"]
+
     def multi_wrapper_all_edges(self, args):
         return self.get_pimg_for_one_edge(*args)
 

@@ -19,6 +19,7 @@ F_NO_SMALL = 4096
 F_NO_TABLE = 8192
 F_FILT_HKS = 16384
 ST_NOT_SMALL = 255
+E_INVALID, E_CUDA, E_NOMEM, E_NODEVICE, E_CAPACITY = -1, -2, -3, -4, -5
 K_UP, K_ESS, K_DOWN, K_ESS_REV, K_ONE = 0, 1, 2, 3, 4
 ST_OK, ST_TRIVIAL, ST_EMPTY, ST_DISCONNECTED, ST_DEGENERATE, ST_UNKNOWN_NODE, ST_BAD_DESCRIPTOR, ST_NO_TREE_EDGES = range(8)
 ST_NAMES = ["OK", "TRIVIAL", "EMPTY", "DISCONNECTED", "DEGENERATE", "UNKNOWN_NODE", "BAD_DESCRIPTOR", "NO_TREE_EDGES"]
@@ -28,7 +29,8 @@ EXPORTS = ["tlc_graph_create", "tlc_graph_destroy", "tlc_vicinity_pi", "tlc_vici
            "tlc_launch_count", "tlc_last_stage_ms", "tlc_last_algorithmic_bytes", "tlc_graph_set_stream",
            "tlc_last_counts", "tlc_last_direct", "tlc_pi_gather", "tlc_last_small", "tlc_small_diagrams",
            "tlc_table_create", "tlc_table_attach", "tlc_vicinity_pi_exchange", "tlc_last_table",
-           "tlc_ollivier_ricci", "tlc_graph_set_hks_time", "tlc_table_build_ms"]
+           "tlc_ollivier_ricci", "tlc_graph_set_hks_time", "tlc_table_build_ms", "tlc_vicinity_diagrams",
+           "tlc_vicinity_diagrams_dev"]
 
 
 class Params(C.Structure):
@@ -48,6 +50,12 @@ class Detail(C.Structure):
                 ("pbirth", C.c_void_p), ("pdeath", C.c_void_p),
                 ("pos", C.c_void_p), ("neg", C.c_void_p),
                 ("pi", C.c_void_p), ("status", C.c_void_p), ("pi_up", C.c_void_p), ("pi_one", C.c_void_p)]
+
+
+class Diagrams(C.Structure):
+    """tlc_diagrams: the pair arrays of tlc_vicinity_diagrams(_dev), host or device addresses"""
+    _fields_ = [("cap", C.c_int64), ("poff", C.c_void_p), ("npairs", C.c_void_p), ("kind", C.c_void_p),
+                ("bv", C.c_void_p), ("dv", C.c_void_p), ("birth", C.c_void_p), ("death", C.c_void_p)]
 
 
 class TlcError(RuntimeError):
@@ -117,6 +125,9 @@ def lib():
     L.tlc_vicinity_pi_exchange.argtypes = [vp, vp, vp, i64, C.POINTER(Params), C.POINTER(i64)]
     L.tlc_small_diagrams.restype = C.c_int
     L.tlc_small_diagrams.argtypes = [vp, vp, i64, C.POINTER(Params), vp] + [vp] * 10
+    for name in ("tlc_vicinity_diagrams", "tlc_vicinity_diagrams_dev"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = [vp, vp, i64, C.POINTER(Params), C.POINTER(Diagrams), vp, vp, C.POINTER(i64)]
     _lib = L
     return L
 

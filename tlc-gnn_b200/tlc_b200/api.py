@@ -181,6 +181,80 @@ class VicinityGraph:
                             pdv=pdv[a:b], pbirth=pbirth[a:b], pdeath=pdeath[a:b]))
         return out
 
+    # ---- persistence diagrams of a batch (include/tlc_b200.h: tlc_vicinity_diagrams*) ----
+    _diagram_cap = 0  # grow-only guess of the pair arrays' capacity
+
+    def _diagrams(self, fn, targets_ptr, E, p, alloc, pi_ptr, st_ptr, cap):
+        """one diagram call with the capacity guess (or `cap` pairs), once more with the exact total on TLC_E_CAPACITY;
+        alloc(cap) -> (arrays dict, Diagrams struct)"""
+        total = C.c_int64(0)
+        cap = max(self._diagram_cap, 8 * E) if cap is None else int(cap)
+        for attempt in range(2):
+            arrs, d = alloc(cap)
+            rc = fn(self._h, targets_ptr, E, C.byref(p), C.byref(d), pi_ptr, st_ptr, C.byref(total))
+            if rc == L.E_CAPACITY and attempt == 0:
+                cap = int(total.value)
+                continue
+            L.check(rc)
+            break
+        self._diagram_cap = max(self._diagram_cap, cap)
+        return arrs, int(total.value)
+
+    def vicinity_diagrams(self, targets, hop=2, mode=L.MODE_EDGE, descriptor="sum", resolution=5, flags=L.F_NORM,
+                          img_mask=None, cap=None):
+        """the persistence diagrams of a batch, host buffers: dict of numpy arrays poff int64[E+1] (target t's pairs are
+        [poff[t], poff[t+1])), kind uint8, bv / dv int32 (graph ids), birth / death float64, status uint8[E] and the image
+        rows pi float64[E, res^2].  cap: capacity of the first attempt in pairs (default: a grow-only guess); a call that
+        needs more is repeated once with the exact total"""
+        t = np.ascontiguousarray(targets, dtype=np.int32).reshape(-1, 2)
+        E = t.shape[0]
+        p = make_params(hop, mode, descriptor, resolution, flags, img_mask)
+        pi = np.zeros((E, int(resolution) * int(resolution)))
+        status = np.zeros(E, np.uint8)
+        poff = np.zeros(E + 1, np.int64)
+
+        def alloc(cap):
+            a = dict(poff=poff, kind=np.zeros(cap, np.uint8), bv=np.zeros(cap, np.int32), dv=np.zeros(cap, np.int32),
+                     birth=np.zeros(cap), death=np.zeros(cap))
+            d = L.Diagrams(cap, poff.ctypes.data, None, *(a[k].ctypes.data for k in ("kind", "bv", "dv", "birth", "death")))
+            return a, d
+
+        a, total = self._diagrams(L.lib().tlc_vicinity_diagrams, t.ctypes.data, E, p, alloc, pi.ctypes.data,
+                                  status.ctypes.data, cap)
+        out = {k: (v if k == "poff" else v[:total]) for k, v in a.items()}
+        out.update(status=status, pi=pi)
+        return out
+
+    def vicinity_diagrams_dev(self, targets_dev, hop=2, mode=L.MODE_EDGE, descriptor="sum", resolution=5, flags=L.F_NORM,
+                              img_mask=None, want_pi=False, cap=None):
+        """the persistence diagrams of a batch, device buffers: targets_dev int32[E, 2] (torch, this graph's device) ->
+        dict of CUDA tensors poff int64[E+1], kind uint8, bv / dv int32 (graph ids), birth / death float64, status uint8[E]
+        and, with want_pi, the image rows pi float64[E, res^2] (else None); cap as in vicinity_diagrams"""
+        import torch
+        E = int(targets_dev.shape[0])
+        dev = torch.device("cuda", self.device)
+        tp = _dev_ptr(targets_dev, "int32", (E, 2), self.device, "targets_dev") if E else None
+        p = make_params(hop, mode, descriptor, resolution, flags, img_mask)
+        pi = torch.zeros((E, int(resolution) * int(resolution)), dtype=torch.float64, device=dev) if want_pi else None
+        status = torch.zeros(E, dtype=torch.uint8, device=dev)
+        poff = torch.zeros(E + 1, dtype=torch.int64, device=dev)
+        torch.cuda.synchronize(dev)  # (the library works on its own stream)
+
+        def alloc(cap):
+            a = dict(poff=poff, kind=torch.empty(cap, dtype=torch.uint8, device=dev),
+                     bv=torch.empty(cap, dtype=torch.int32, device=dev), dv=torch.empty(cap, dtype=torch.int32, device=dev),
+                     birth=torch.empty(cap, dtype=torch.float64, device=dev),
+                     death=torch.empty(cap, dtype=torch.float64, device=dev))
+            torch.cuda.synchronize(dev)
+            d = L.Diagrams(cap, poff.data_ptr(), None, *(a[k].data_ptr() for k in ("kind", "bv", "dv", "birth", "death")))
+            return a, d
+
+        a, total = self._diagrams(L.lib().tlc_vicinity_diagrams_dev, tp, E, p, alloc,
+                                  pi.data_ptr() if pi is not None else None, status.data_ptr(), cap)
+        out = {k: (v if k == "poff" else v[:total]) for k, v in a.items()}
+        out.update(status=status, pi=pi)
+        return out
+
     # ---- multi-GPU exchange by peer stores (include/tlc_b200.h: tlc_table_*) ----
     def table_create(self, rows, resolution=5):
         """this rank's exchange table float32[rows][res^2 + 1]: -> (device address of row 0, 64-byte CUDA IPC handle)"""
