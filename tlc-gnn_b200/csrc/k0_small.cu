@@ -30,28 +30,7 @@ namespace tlc {
 namespace {
 
 constexpr unsigned FULLM = 0xffffffffu;
-constexpr unsigned long long S_INF = 0x7ff0000000000000ull;
 constexpr int PBUF = 32;  // pairs buffered before the team rasterises them
-
-struct PySumS {  // CPython's float sum(): first item exact, then Neumaier (3.12+) or plain adds   SURVEY.md F5
-  double s, c;
-  int k;
-};
-__device__ __forceinline__ void pys_add(PySumS& p, double x, bool plain) {
-  if (p.k == 0) { p.s = x; p.k = 1; return; }
-  if (plain) { p.s = __dadd_rn(p.s, x); return; }
-  const double t = __dadd_rn(p.s, x);
-  if (fabs(p.s) >= fabs(x)) p.c = __dadd_rn(p.c, __dadd_rn(__dadd_rn(p.s, -t), x));
-  else p.c = __dadd_rn(p.c, __dadd_rn(__dadd_rn(x, -t), p.s));
-  p.s = t;
-}
-__device__ __forceinline__ double pys_get(const PySumS& p, bool plain) {
-  if (p.k == 0) return 0.0;
-  if (!plain && p.c != 0.0 && isfinite(p.c)) return __dadd_rn(p.s, p.c);
-  return p.s;
-}
-
-__device__ __forceinline__ double s_norm_cdf(double x) { return erfc(-x / 1.4142135623730951) * 0.5; }  // PersistenceImager.pyx:60
 
 // ---- team primitives: NT == 32 -> a warp (several teams per CTA), NT > 32 -> the whole CTA ----
 template <int NT>
@@ -194,16 +173,9 @@ __device__ __forceinline__ void flush_pairs(const Team<NT>& tm, const double* pb
     if (act) {
       const double birth = pb[2 * k], death = pb[2 * k + 1];
       const double pers = death - birth;  // skew :366
-      const double w = pers < 0.0 ? 0.0 : (pers > 1.0 ? 1.0 : pers);  // linear_ramp :22-28
+      const double w = ramp_weight(pers);
       double gb[5], gp[5];
-      double pbv = s_norm_cdf(0.0 - birth), ppv = s_norm_cdf(0.0 - pers);
-#pragma unroll
-      for (int i = 1; i <= 5; i++) {
-        const double pt = i * step;
-        const double cb = s_norm_cdf(pt - birth), cp = s_norm_cdf(pt - pers);
-        gb[i - 1] = cb - pbv; gp[i - 1] = cp - ppv;
-        pbv = cb; ppv = cp;
-      }
+      cdf_diffs(5, step, birth, pers, gb, gp);
 #pragma unroll
       for (int i = 0; i < 5; i++) {
         const double wb = w * gb[i];
@@ -222,17 +194,6 @@ __device__ __forceinline__ void flush_pairs(const Team<NT>& tm, const double* pb
     }
   }
   tm.sync();
-}
-
-template <typename LID>
-__device__ __forceinline__ int s_find(LID* p, int x) {  // path halving  accelerated_PD.py:53-58
-  for (;;) {
-    const int px = (int)p[x];
-    if (px == x) return x;
-    const int gp = (int)p[px];
-    p[x] = (LID)gp;
-    x = gp;
-  }
 }
 
 template <int NT, int NC, int AC>
@@ -299,7 +260,7 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
     const int64_t dpo = a.poff ? a.poff[row] : 0;
     bool deferred = false;
 
-    // dict_node[u] KeyError -> zeros (riccidist2dgm.py:353); the reference graph has no isolated nodes
+    // unknown_target, written out: calling it changes this kernel's register allocation
     bool bad = u < 0 || u >= g.N || (!node_mode && (v < 0 || v >= g.N));
     if (!bad) bad = g.rowptr[u + 1] == g.rowptr[u] || (!node_mode && g.rowptr[v + 1] == g.rowptr[v]);
     if (bad) status = TLC_ST_UNKNOWN_NODE;
@@ -430,21 +391,21 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
     if (status == TLC_ST_OK) {
       // ---------------- 3. filtration: build_fv(weight_graph=True, norm)   riccidist2dgm.py:20-61 ----------------
       if (!roots_in) {
-        // nx.NodeNotFound for every vertex -> dist = 100   :31-32,36-37
-        for (int x = tid; x < n; x += NT) { d1[x] = (unsigned long long)__double_as_longlong(100.0); d2[x] = d1[x]; }
+        // nx.NodeNotFound for every vertex
+        for (int x = tid; x < n; x += NT) { d1[x] = (unsigned long long)__double_as_longlong(NO_PATH_DIST); d2[x] = d1[x]; }
       } else {
         const bool two = !node_mode && lu != lv;
         for (int rr = 0; rr < (two ? 2 : 1); rr++) {
           const int root = rr == 0 ? lu : lv;
           unsigned long long* dist = rr == 0 ? d1 : d2;
-          for (int x = tid; x < n; x += NT) { dist[x] = x == root ? 0ull : S_INF; tpe[x] = 0x7fffffff; }
+          for (int x = tid; x < n; x += NT) { dist[x] = x == root ? 0ull : INF_BITS; tpe[x] = 0x7fffffff; }
           tm.sync();
           // least fixpoint of d[y] = min_x fl(d[x] + w(x, y)): relaxation rounds over all directed entries
           for (int round = 0; round <= n; round++) {
             bool ch = false;
             for (int e = tid; e < A2; e += NT) {
               const unsigned long long dxb = dist[esrc[e]];
-              if (dxb == S_INF) continue;
+              if (dxb == INF_BITS) continue;
               const unsigned long long tb = (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dxb), aw[e]));
               const int y = (int)anb[e];
               if (tb < dist[y]) { atomicMin(&dist[y], tb); ch = true; }
@@ -456,7 +417,7 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
           for (int e = tid; e < A2; e += NT) {
             const int x = (int)esrc[e];
             const unsigned long long dxb = dist[x], dyb = dist[anb[e]];
-            if (x == root || dxb == S_INF || dyb == S_INF) continue;
+            if (x == root || dxb == INF_BITS || dyb == INF_BITS) continue;
             if ((unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dyb), aw[e])) == dxb) atomicMin(&tpe[x], e);
           }
           tm.sync();
@@ -468,12 +429,12 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
             double res = 0.0;
             if (x < n) {
               if (x == root) res = 0.0;
-              else if (dist[x] == S_INF) res = 100.0;  // nx.NetworkXNoPath -> 100 (disconnected vicinity: status 3 from the sweep)
+              else if (dist[x] == INF_BITS) res = NO_PATH_DIST;  // nx.NetworkXNoPath (disconnected vicinity: status 3 from the sweep)
               else {
-                PySumS ps{0.0, 0.0, 0};
+                PySum ps{0.0, 0.0, 0};
                 int y = x, guard = 0;
-                while (y != root && guard++ <= n) { const int e = tpe[y]; pys_add(ps, aw[e], plain); y = (int)anb[e]; }
-                res = pys_get(ps, plain);
+                while (y != root && guard++ <= n) { const int e = tpe[y]; pysum_add(ps, aw[e], plain); y = (int)anb[e]; }
+                res = pysum_get(ps, plain);
               }
             }
             res_x[j] = res;
@@ -488,19 +449,18 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
         }
         if (!two) for (int x = tid; x < n; x += NT) d2[x] = d1[x];
         tm.sync();
-        // `if x in [root_1, root_2]`: all three attributes 0   :22-25
-        if (tid == 0) { d1[lu] = 0ull; d2[lu] = 0ull; d1[lv] = 0ull; d2[lv] = 0ull; }
+        if (tid == 0) zero_roots(d1, d2, lu, lv);
         tm.sync();
       }
-      // descriptors + normalisation   :47-56 ; data_utils_NC.py:52-54
+      // descriptors + normalisation
       double mx = -1.0, sm = -1.0;
       for (int x = tid; x < n; x += NT) {
         const double da = __longlong_as_double((long long)d1[x]), db = __longlong_as_double((long long)d2[x]);
-        mx = fmax(mx, fmax(da, db));
-        sm = fmax(sm, node_mode ? da : __dadd_rn(da, db));
+        mx = fmax(mx, fv_descriptor(TLC_DESC_MAX, node_mode, da, db));
+        sm = fmax(sm, fv_descriptor(TLC_DESC_SUM, node_mode, da, db));
       }
       double smax = tm.maxd(mx), ssum = tm.maxd(sm);
-      if (norm) {
+      if (norm) {  // fv_normalisers, written out for the same reason
         if (p.flags & TLC_F_NORM_EPS) { smax = __dadd_rn(smax, 1e-10); ssum = __dadd_rn(ssum, 1e-10); }
         else if (smax == 0.0 || ssum == 0.0) {
           // ZeroDivisionError -> zeros (:54-56,356-357); every vertex is a root here, so n <= 2 and the connectivity
@@ -511,12 +471,7 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
       if (status == TLC_ST_OK) {
         for (int x = tid; x < n; x += NT) {
           const double da = __longlong_as_double((long long)d1[x]), db = __longlong_as_double((long long)d2[x]);
-          double f;
-          if (p.descriptor == TLC_DESC_MIN) f = fmin(da, db);
-          else if (p.descriptor == TLC_DESC_MAX) f = fmax(da, db);
-          else f = node_mode ? da : __dadd_rn(da, db);
-          if (norm) f = __ddiv_rn(f, p.descriptor == TLC_DESC_SUM ? ssum : smax);
-          fv[x] = f;
+          fv[x] = fv_value(p.descriptor, node_mode, norm, smax, ssum, da, db);
         }
       }
       tm.sync();
@@ -587,7 +542,7 @@ __global__ void __launch_bounds__(NT == 32 ? 128 : NT) small_kernel(SmallArgs a)
             const int k = k0 + lane;
             const bool valid = k < m;
             int e = 0, ea = 0, eb = 0, ra = 0, rb = 0;
-            if (valid) { e = sidx[k]; ea = elo[e]; eb = ehi[e]; ra = s_find(par, ea); rb = s_find(par, eb); }
+            if (valid) { e = sidx[k]; ea = elo[e]; eb = ehi[e]; ra = uf_find(par, ea); rb = uf_find(par, eb); }
             __syncwarp();
             unsigned cm = __ballot_sync(FULLM, valid && ra != rb);
             unsigned negm = 0;

@@ -34,7 +34,6 @@ struct K1Shared {
   unsigned long long xacc;  // ... and number of rowptr pairs read (X)
 };
 
-__device__ __forceinline__ bool test_bit(const uint32_t* bm, int32_t y) { return (bm[y >> 5] >> (y & 31)) & 1u; }
 __device__ __forceinline__ bool set_bit(uint32_t* bm, int32_t y) {  // returns true if newly set
   const uint32_t bit = 1u << (y & 31);
   if (bm[y >> 5] & bit) return false;
@@ -195,9 +194,7 @@ vicinity_light_kernel(GraphView g, Params p, const int32_t* __restrict__ targets
   const bool node_mode = p.mode == TLC_MODE_NODE;
   for (int64_t t = warp; t < E; t += nwarps) {
     const int32_t u = targets[2 * t], v = targets[2 * t + 1];
-    bool bad = u < 0 || u >= g.N || (!node_mode && (v < 0 || v >= g.N));
-    if (!bad) bad = g.rowptr[u + 1] == g.rowptr[u] || (!node_mode && g.rowptr[v + 1] == g.rowptr[v]);
-    if (bad) {
+    if (unknown_target(g, u, v, node_mode)) {
       if (lane == 0) { out_n[t] = 0; out_m[t] = 0; out_ds[t] = 0; out_status[t] = TLC_ST_UNKNOWN_NODE; if (out_bytes) out_bytes[t] = 0.0; }
       continue;
     }
@@ -253,10 +250,7 @@ vicinity_kernel(GraphView g, Params p, const int32_t* __restrict__ targets, int6
     const int64_t ti = FILL ? c.tidx[t] : t;
     const int32_t u = targets[2 * ti], v = targets[2 * ti + 1];
     const bool node_mode = p.mode == TLC_MODE_NODE;
-    // dict_node[u] KeyError (riccidist2dgm.py:353); the reference graph has no isolated nodes
-    bool bad = u < 0 || u >= g.N || (!node_mode && (v < 0 || v >= g.N));
-    if (!bad) bad = g.rowptr[u + 1] == g.rowptr[u] || (!node_mode && g.rowptr[v + 1] == g.rowptr[v]);
-    if (bad) {
+    if (unknown_target(g, u, v, node_mode)) {
       if (tid == 0) {
         if (!FILL) { out_n[t] = 0; out_m[t] = 0; out_ds[t] = 0; out_status[t] = TLC_ST_UNKNOWN_NODE; }
         else { c.tn[t] = 0; c.tm[t] = 0; c.tnp[t] = 0; c.tnpos[t] = 0; c.tnneg[t] = 0; c.tlu[t] = -1; c.tlv[t] = -1;

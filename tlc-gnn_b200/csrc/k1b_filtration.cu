@@ -35,26 +35,6 @@
 namespace tlc {
 namespace {
 
-constexpr unsigned long long INF_BITS = 0x7ff0000000000000ull;
-
-struct PySum {  // CPython's float sum(): first item exact, then Neumaier (3.12+) or plain adds
-  double s, c;
-  int k;
-};
-__device__ __forceinline__ void pysum_add(PySum& p, double x, bool plain) {
-  if (p.k == 0) { p.s = x; p.k = 1; return; }
-  if (plain) { p.s = __dadd_rn(p.s, x); return; }
-  const double t = __dadd_rn(p.s, x);
-  if (fabs(p.s) >= fabs(x)) p.c = __dadd_rn(p.c, __dadd_rn(__dadd_rn(p.s, -t), x));
-  else p.c = __dadd_rn(p.c, __dadd_rn(__dadd_rn(x, -t), p.s));
-  p.s = t;
-}
-__device__ __forceinline__ double pysum_get(const PySum& p, bool plain) {
-  if (p.k == 0) return 0.0;
-  if (!plain && p.c != 0.0 && isfinite(p.c)) return __dadd_rn(p.s, p.c);
-  return p.s;
-}
-
 #ifndef FILT_QCAP
 #define FILT_QCAP 1024
 #endif
@@ -86,30 +66,6 @@ struct FiltShared {
   unsigned long long nmin[2];
 };
 
-// exclusive scan of data[0..cnt) in shared memory, two barriers; returns the total.  All threads call.
-__device__ inline int block_scan_shfl(int32_t* data, int cnt, int32_t* wsum) {
-  const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, wid = tid >> 5, nw = (nt + 31) >> 5;
-  const int per = (cnt + nt - 1) / nt;
-  const int lo = min(tid * per, cnt), hi = min(lo + per, cnt);
-  int s = 0;
-  for (int i = lo; i < hi; i++) s += data[i];
-  int inc = s;
-  for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
-  if (lane == 31) wsum[wid] = inc;
-  __syncthreads();
-  if (wid == 0) {
-    const int wv = lane < nw ? wsum[lane] : 0;
-    int winc = wv;
-    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, winc, o); if (lane >= o) winc += v; }
-    if (lane < nw) wsum[lane] = winc - wv;
-    if (lane == 31) wsum[32] = winc;
-  }
-  __syncthreads();
-  int run = wsum[wid] + inc - s;
-  for (int i = lo; i < hi; i++) { const int v = data[i]; data[i] = run; run += v; }
-  return wsum[32];
-}
-
 struct DirectArgs {
   GraphView g;
   const uint32_t* ball_cache;  // [N][W] closed k-hop balls (kernel 1's ball cache)
@@ -135,25 +91,12 @@ __global__ void __launch_bounds__(1024) filtration_kernel(Params p, ChunkView c,
     const int64_t ti = c.tidx[t];
     const int32_t u = c.tgt[2 * ti], v = c.tgt[2 * ti + 1];
     const GraphView& g = da.g;
-    bool bad = u < 0 || u >= g.N || (!node_mode && (v < 0 || v >= g.N));  // dict_node KeyError   :353
-    if (!bad) bad = g.rowptr[u + 1] == g.rowptr[u] || (!node_mode && g.rowptr[v + 1] == g.rowptr[v]);
-    if (bad) {
+    if (unknown_target(g, u, v, node_mode)) {
       if (tid == 0) { c.tn[t] = 0; c.tnp[t] = 0; c.tnpos[t] = 0; c.tnneg[t] = 0; c.tlu[t] = -1; c.tlv[t] = -1;
                       c.tstatus[t] = TLC_ST_UNKNOWN_NODE; }
       return;
     }
-    const uint32_t* __restrict__ bu = da.ball_cache + (size_t)u * W;
-    const uint32_t* __restrict__ bv = da.ball_cache + (size_t)v * W;
-    for (int w = tid; w < W; w += nt) {
-      const uint32_t x = node_mode ? bu[w] : (bu[w] & bv[w]);
-      bm[w] = x;
-      bm[W + w] = __popc(x);
-    }
-    __syncthreads();
-    n = block_scan_shfl(reinterpret_cast<int32_t*>(bm + W), W, sh.wsum);
-    __syncthreads();
-    uint32_t* gb = c.dbm + (size_t)t * 2 * W;  // kernels 2v / 3v map graph ids through it
-    for (int w = tid; w < 2 * W; w += nt) gb[w] = bm[w];
+    n = graph_row_bitmap(c, t, da.ball_cache, W, u, v, node_mode, bm, sh.wsum);
     for (int w = wid; w < W; w += nw) {  // a warp per bitmap word: vertex list, graph rows, settling margins
       const uint32_t bits = bm[w];
       if (!((bits >> lane) & 1u)) continue;
@@ -216,8 +159,8 @@ __global__ void __launch_bounds__(1024) filtration_kernel(Params p, ChunkView c,
   const uint16_t* slid = reinterpret_cast<const uint16_t*>(bm + 2 * W);
   int mcnt = 0;
   if (!roots_in) {
-    // nx.NodeNotFound for every vertex -> dist = 100   riccidist2dgm.py:31-32,36-37
-    for (int x = tid; x < n; x += nt) { d1[x] = 100.0; d2[x] = 100.0; c.neg[vo + x] = -1; c.vcls[vo + x] = -1; }
+    // nx.NodeNotFound for every vertex
+    for (int x = tid; x < n; x += nt) { d1[x] = NO_PATH_DIST; d2[x] = NO_PATH_DIST; c.neg[vo + x] = -1; c.vcls[vo + x] = -1; }
     if (count_m) {
       for (int x = wid; x < n; x += nw) {
         const int a = astart[x], dg = adeg[x];
@@ -291,7 +234,7 @@ __global__ void __launch_bounds__(1024) filtration_kernel(Params p, ChunkView c,
           }
           lmin = d < lmin ? d : lmin;  // still tentative after this phase
         }
-        for (int o = 16; o; o >>= 1) { const unsigned long long v = __shfl_xor_sync(0xffffffffu, lmin, o); lmin = v < lmin ? v : lmin; }
+        lmin = warp_min_u64(lmin);
         if (lane == 0 && lmin != INF_BITS) atomicMin(&sh.nmin[cur ^ 1], lmin);
         __syncthreads();
         const int qn = min(sh.qn[cur], QCAP);
@@ -389,7 +332,7 @@ __global__ void __launch_bounds__(1024) filtration_kernel(Params p, ChunkView c,
             }
           }
         }
-        for (int o = 16; o; o >>= 1) { const unsigned long long v = __shfl_xor_sync(0xffffffffu, umin, o); umin = v < umin ? v : umin; }
+        umin = warp_min_u64(umin);
         if (lane == 0 && umin != INF_BITS) atomicMin(&sh.nmin[cur ^ 1], umin);
         __syncthreads();
         for (int i = tid; i < qn; i += nt) {
@@ -414,7 +357,7 @@ __global__ void __launch_bounds__(1024) filtration_kernel(Params p, ChunkView c,
       for (int x = tid; x < n; x += nt) {
         double res;
         if (x == root) res = 0.0;
-        else if (state[x] != DONE) res = 100.0;  // nx.NetworkXNoPath -> 100 (disconnected vicinity; status 3 later)
+        else if (state[x] != DONE) res = NO_PATH_DIST;  // nx.NetworkXNoPath (disconnected vicinity; status 3 later)
         else {
           PySum ps{0.0, 0.0, 0};
           int y = x, guard = 0;
@@ -430,8 +373,7 @@ __global__ void __launch_bounds__(1024) filtration_kernel(Params p, ChunkView c,
     }
     if (!two) for (int x = tid; x < n; x += nt) d2[x] = d1[x];
     __syncthreads();
-    // `if x in [root_1, root_2]`: all three attributes 0   riccidist2dgm.py:22-25
-    if (tid == 0) { d1[lu] = 0.0; d2[lu] = 0.0; d1[lv] = 0.0; d2[lv] = 0.0; }
+    if (tid == 0) zero_roots(d1, d2, lu, lv);
   }
   __syncthreads();
 
@@ -443,28 +385,17 @@ __global__ void __launch_bounds__(1024) filtration_kernel(Params p, ChunkView c,
   double mx = -1.0, sm = -1.0;
   for (int x = tid; x < n; x += nt) {
     const double a = d1[x], b = d2[x];
-    mx = fmax(mx, fmax(a, b));
-    sm = fmax(sm, node_mode ? a : __dadd_rn(a, b));
+    mx = fmax(mx, fv_descriptor(TLC_DESC_MAX, node_mode, a, b));
+    sm = fmax(sm, fv_descriptor(TLC_DESC_SUM, node_mode, a, b));
   }
   double smax = block_reduce_max(mx, sh.redd);
   double ssum = block_reduce_max(sm, sh.redd);
   const bool norm = (p.flags & TLC_F_NORM) != 0;
-  if (norm) {
-    if (p.flags & TLC_F_NORM_EPS) { smax = __dadd_rn(smax, 1e-10); ssum = __dadd_rn(ssum, 1e-10); }
-    else if (smax == 0.0 || ssum == 0.0) {  // ZeroDivisionError -> zeros   riccidist2dgm.py:54-56,356-357
-      if (tid == 0) c.tstatus[t] = TLC_ST_DEGENERATE;
-      return;
-    }
+  if (norm && !fv_normalisers(p.flags, smax, ssum)) {
+    if (tid == 0) c.tstatus[t] = TLC_ST_DEGENERATE;
+    return;
   }
-  for (int x = tid; x < n; x += nt) {
-    const double a = d1[x], b = d2[x];
-    double f;
-    if (p.descriptor == TLC_DESC_MIN) f = fmin(a, b);
-    else if (p.descriptor == TLC_DESC_MAX) f = fmax(a, b);
-    else f = node_mode ? a : __dadd_rn(a, b);
-    if (norm) f = __ddiv_rn(f, p.descriptor == TLC_DESC_SUM ? ssum : smax);
-    fval[x] = f;
-  }
+  for (int x = tid; x < n; x += nt) fval[x] = fv_value(p.descriptor, node_mode, norm, smax, ssum, d1[x], d2[x]);
 }
 
 }  // namespace

@@ -31,55 +31,6 @@
 namespace tlc {
 namespace {
 
-constexpr unsigned long long T_INF = 0x7ff0000000000000ull;
-
-struct PySumT {  // CPython's float sum(): first item exact, then Neumaier (3.12+) or plain adds
-  double s, c;
-  int k;
-};
-__device__ __forceinline__ void pyt_add(PySumT& p, double x, bool plain) {
-  if (p.k == 0) { p.s = x; p.k = 1; return; }
-  if (plain) { p.s = __dadd_rn(p.s, x); return; }
-  const double t = __dadd_rn(p.s, x);
-  if (fabs(p.s) >= fabs(x)) p.c = __dadd_rn(p.c, __dadd_rn(__dadd_rn(p.s, -t), x));
-  else p.c = __dadd_rn(p.c, __dadd_rn(__dadd_rn(x, -t), p.s));
-  p.s = t;
-}
-__device__ __forceinline__ double pyt_get(const PySumT& p, bool plain) {
-  if (p.k == 0) return 0.0;
-  if (!plain && p.c != 0.0 && isfinite(p.c)) return __dadd_rn(p.s, p.c);
-  return p.s;
-}
-
-__device__ __forceinline__ unsigned long long shfl_min_u64(unsigned long long v) {
-#pragma unroll
-  for (int o = 16; o; o >>= 1) { const unsigned long long u = __shfl_xor_sync(0xffffffffu, v, o); v = u < v ? u : v; }
-  return v;
-}
-
-__device__ inline int scan_words(int32_t* data, int cnt, int32_t* wsum) {  // exclusive scan in shared memory, returns the total
-  const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, wid = tid >> 5, nw = (nt + 31) >> 5;
-  const int per = (cnt + nt - 1) / nt;
-  const int lo = min(tid * per, cnt), hi = min(lo + per, cnt);
-  int s = 0;
-  for (int i = lo; i < hi; i++) s += data[i];
-  int inc = s;
-  for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
-  if (lane == 31) wsum[wid] = inc;
-  __syncthreads();
-  if (wid == 0) {
-    const int wv = lane < nw ? wsum[lane] : 0;
-    int winc = wv;
-    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, winc, o); if (lane >= o) winc += v; }
-    if (lane < nw) wsum[lane] = winc - wv;
-    if (lane == 31) wsum[32] = winc;
-  }
-  __syncthreads();
-  int run = wsum[wid] + inc - s;
-  for (int i = lo; i < hi; i++) { const int v = data[i]; data[i] = run; run += v; }
-  return wsum[32];
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
 // table build: one CTA per root, whole graph, distances + parents in shared memory
 // ---------------------------------------------------------------------------------------------------------------------
@@ -122,21 +73,21 @@ __global__ void __launch_bounds__(1024) sssp_build_kernel(GraphView g, SsspTable
   for (int idx = blockIdx.x; idx < cnt; idx += gridDim.x) {
     const int32_t root = tb.list[idx];
     __syncthreads();
-    for (int x = tid; x < N; x += nt) { dist[x] = T_INF; state[x] = 0; par[x] = -1; }
+    for (int x = tid; x < N; x += nt) { dist[x] = INF_BITS; state[x] = 0; par[x] = -1; }
     __syncthreads();
     if (tid == 0) { dist[root] = 0ull; state[root] = 1; }
     __syncthreads();
     for (int phase = 0; phase < 2 * N + 2; phase++) {
       // smallest tentative distance
-      if (tid == 0) { sh.dmin = T_INF; sh.qn = 0; sh.qhead = 0; }
+      if (tid == 0) { sh.dmin = INF_BITS; sh.qn = 0; sh.qhead = 0; }
       __syncthreads();
-      unsigned long long lm = T_INF;
+      unsigned long long lm = INF_BITS;
       for (int x = tid; x < N; x += nt) if (state[x] == 1) { const unsigned long long d = dist[x]; lm = d < lm ? d : lm; }
-      lm = shfl_min_u64(lm);
-      if (lane == 0 && lm != T_INF) atomicMin(&sh.dmin, lm);
+      lm = warp_min_u64(lm);
+      if (lane == 0 && lm != INF_BITS) atomicMin(&sh.dmin, lm);
       __syncthreads();
       const unsigned long long dminb = sh.dmin;
-      if (dminb == T_INF) break;
+      if (dminb == INF_BITS) break;
       const double dmin = __longlong_as_double((long long)dminb);
       // settle every tentative x with d[x] <= fl(dmin + minw[x])   (Crauser et al.'s IN criterion, exact by monotonicity of fl)
       for (int x = tid; x < N; x += nt) {
@@ -169,7 +120,7 @@ __global__ void __launch_bounds__(1024) sssp_build_kernel(GraphView g, SsspTable
     // tree rule: parent[x] = smallest id y with fl(d[y] + w) == d[x] (rows ascend: the first matching position)
     for (int x = wid; x < N; x += nw) {
       const unsigned long long dxb = dist[x];
-      if (x == root || dxb == T_INF) continue;
+      if (x == root || dxb == INF_BITS) continue;
       const int a = g.rowptr[x], b = g.rowptr[x + 1];
       for (int e0 = a; e0 < b; e0 += 32) {
         const int e = e0 + lane;
@@ -180,7 +131,7 @@ __global__ void __launch_bounds__(1024) sssp_build_kernel(GraphView g, SsspTable
           y = g.col[e];
           w = __dadd_rn(g.kappa[e], 1.0);
           const unsigned long long dyb = dist[y];
-          hit = dyb != T_INF && (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dyb), w)) == dxb;
+          hit = dyb != INF_BITS && (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dyb), w)) == dxb;
         }
         const unsigned bal = __ballot_sync(0xffffffffu, hit);
         if (bal) {
@@ -203,12 +154,12 @@ __global__ void __launch_bounds__(1024) sssp_build_kernel(GraphView g, SsspTable
       Wrow[x] = par[x] >= 0 ? pw[x] : 0.0;
       double res;
       if (x == root) res = 0.0;
-      else if (dxb == T_INF || par[x] < 0) res = 100.0;
+      else if (dxb == INF_BITS || par[x] < 0) res = NO_PATH_DIST;
       else {
-        PySumT ps{0.0, 0.0, 0};
+        PySum ps{0.0, 0.0, 0};
         int y = x, guard = 0;
-        while (y != root && guard++ <= N) { pyt_add(ps, pw[y], plain != 0); y = par[y]; }
-        res = pyt_get(ps, plain != 0);
+        while (y != root && guard++ <= N) { pysum_add(ps, pw[y], plain != 0); y = par[y]; }
+        res = pysum_get(ps, plain != 0);
       }
       Qrow[x] = res;
     }
@@ -259,25 +210,12 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
   // ---- 0. the vicinity (as kernel 1b's graph-row prologue): nodes = set(nodes_u) & set(nodes_v), local ids = ranks   :311-316
   const int64_t ti = c.tidx[t];
   const int32_t u = c.tgt[2 * ti], v = c.tgt[2 * ti + 1];
-  bool bad = u < 0 || u >= N || (!node_mode && (v < 0 || v >= N));  // dict_node KeyError   :353
-  if (!bad) bad = g.rowptr[u + 1] == g.rowptr[u] || (!node_mode && g.rowptr[v + 1] == g.rowptr[v]);
-  if (bad) {
+  if (unknown_target(g, u, v, node_mode)) {
     if (tid == 0) { c.tn[t] = 0; c.tnp[t] = 0; c.tnpos[t] = 0; c.tnneg[t] = 0; c.tlu[t] = -1; c.tlv[t] = -1;
                     c.tstatus[t] = TLC_ST_UNKNOWN_NODE; }
     return;
   }
-  const uint32_t* __restrict__ bu = ball_cache + (size_t)u * W;
-  const uint32_t* __restrict__ bv = ball_cache + (size_t)v * W;
-  for (int w = tid; w < W; w += nt) {
-    const uint32_t x = node_mode ? bu[w] : (bu[w] & bv[w]);
-    bm[w] = x;
-    bm[W + w] = __popc(x);
-  }
-  __syncthreads();
-  const int n = scan_words(reinterpret_cast<int32_t*>(bm + W), W, sh.wsum);
-  __syncthreads();
-  uint32_t* gb = c.dbm + (size_t)t * 2 * W;  // kernels 2v / 3v map graph ids through it
-  for (int w = tid; w < 2 * W; w += nt) gb[w] = bm[w];
+  const int n = graph_row_bitmap(c, t, ball_cache, W, u, v, node_mode, bm, sh.wsum);
   {
     uint32_t* l32 = reinterpret_cast<uint32_t*>(lid);
     for (int i = tid; i < (N + 1) / 2; i += nt) l32[i] = 0xffffffffu;
@@ -327,8 +265,8 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
   constexpr uint8_t UNKNOWN = 0, VALID = 1, INVALID = 2, UNREACH = 3;
 
   if (!roots_in) {
-    // nx.NodeNotFound for every vertex -> dist = 100   riccidist2dgm.py:31-32,36-37
-    for (int x = tid; x < n; x += nt) { d1[x] = 100.0; d2[x] = 100.0; hint[x] = -1; hint0[x] = -1; }
+    // nx.NodeNotFound for every vertex
+    for (int x = tid; x < n; x += nt) { d1[x] = NO_PATH_DIST; d2[x] = NO_PATH_DIST; hint[x] = -1; hint0[x] = -1; }
   } else {
     for (int r = 0; r < (two ? 2 : 1); r++) {
       const int root = r == 0 ? lu : lv;
@@ -382,7 +320,7 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
         if (iv) {
           const int32_t gx = vert[x];
           inv[base + __popc(bal & lanemask_lt())] = x;
-          dist[x] = T_INF; bpos[x] = 0x7fffffff;
+          dist[x] = INF_BITS; bpos[x] = 0x7fffffff;
           atomicAdd(&sh.dinv, g.rowptr[gx + 1] - g.rowptr[gx]);
         }
       }
@@ -452,7 +390,7 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
             int trips = (b - a + 31) >> 5;  // the longest of the warp's four chunks: the votes below are warp-wide
             trips = max(trips, __shfl_xor_sync(0xffffffffu, trips, 8));
             trips = max(trips, __shfl_xor_sync(0xffffffffu, trips, 16));
-            unsigned long long best = T_INF;
+            unsigned long long best = INF_BITS;
             for (int t5 = 0; t5 < trips; t5++) {
               const int e0 = a + l8 + 32 * t5;
               uint4 rc[4];
@@ -476,12 +414,12 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
                 const unsigned long long dyb = dist[ly];
                 if (!first && cls[ly] == INVALID) {  // a reread chunk also pushes: the pairs it would have listed go both ways
                   const unsigned long long dxb = dist[x];
-                  if (dxb != T_INF) {
+                  if (dxb != INF_BITS) {
                     const unsigned long long c2 = (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dxb), w));
                     if (c2 < dyb && c2 < atomicMin(&dist[ly], c2)) ch = 1;
                   }
                 }
-                if (dyb == T_INF) continue;
+                if (dyb == INF_BITS) continue;
                 const unsigned long long cand = (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dyb), w));
                 best = cand < best ? cand : best;
               }
@@ -530,11 +468,11 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
           if (epr[i] == 0xffffffffu) continue;
           const int x = (int)(epr[i] >> 16), ly = (int)(epr[i] & 0xffffu);
           const unsigned long long dyb = dist[ly], dxb = dist[x];
-          if (dyb != T_INF) {
+          if (dyb != INF_BITS) {
             const unsigned long long cand = (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dyb), ewt[i]));
             if (cand < dxb && cand < atomicMin(&dist[x], cand)) ch = 1;
           }
-          if (dxb != T_INF) {
+          if (dxb != INF_BITS) {
             const unsigned long long c2 = (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dxb), ewt[i]));
             if (c2 < dyb && c2 < atomicMin(&dist[ly], c2)) ch = 1;
           }
@@ -544,14 +482,14 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
           ia_get(wid * capw + k, pr, pos);
           const int x = (int)(pr >> 16), ly = (int)(pr & 0xffffu);
           const unsigned long long dyb = dist[ly], dxb = dist[x];
-          if (dyb == T_INF && dxb == T_INF) continue;
+          if (dyb == INF_BITS && dxb == INF_BITS) continue;
           const uint4 rc = __ldg(g.rec + pos);
           const double w = __hiloint2double((int)rc.w, (int)rc.z);
-          if (dyb != T_INF) {
+          if (dyb != INF_BITS) {
             const unsigned long long cand = (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dyb), w));
             if (cand < dxb && cand < atomicMin(&dist[x], cand)) ch = 1;
           }
-          if (dxb != T_INF) {
+          if (dxb != INF_BITS) {
             const unsigned long long c2 = (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dxb), w));
             if (c2 < dyb && c2 < atomicMin(&dist[ly], c2)) ch = 1;
           }
@@ -572,8 +510,8 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
         for (int j = 0; j < 8; j++) {
         const int x = __shfl_sync(gm, mx, j, 8), a = __shfl_sync(gm, ma, j, 8);
         int b = __shfl_sync(gm, mb, j, 8);
-        const unsigned long long dxb = b > a ? dist[x] : T_INF;
-        if (dxb == T_INF) b = a;
+        const unsigned long long dxb = b > a ? dist[x] : INF_BITS;
+        if (dxb == INF_BITS) b = a;
         int hit = 0x7fffffff;
         for (int e0 = a; e0 < b; e0 += 32) {   // (uniform over the group: the exit test below is a group vote)
           uint4 rc[4];
@@ -585,7 +523,7 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
             const uint16_t ly = lid[rc[q].x];
             if (ly == 0xffff) continue;
             const unsigned long long dyb = dist[ly];
-            if (dyb != T_INF && (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dyb), __hiloint2double((int)rc[q].w, (int)rc[q].z))) == dxb)
+            if (dyb != INF_BITS && (unsigned long long)__double_as_longlong(__dadd_rn(__longlong_as_double((long long)dyb), __hiloint2double((int)rc[q].w, (int)rc[q].z))) == dxb)
               hit = e0 + l8 + 8 * q;
           }
           if (__ballot_sync(gm, hit != 0x7fffffff)) break;   // (the group's own vote: groups leave at different times)
@@ -606,7 +544,7 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
           if (cls[x] == VALID) wb = (unsigned long long)__double_as_longlong(Wrow[vert[x]]);
           else {
             const int pos = bpos[x];
-            if (dist[x] != T_INF && pos != 0x7fffffff) {
+            if (dist[x] != INF_BITS && pos != 0x7fffffff) {
               const uint4 rc = __ldg(g.rec + pos);
               parl[x] = lid[rc.x];
               wb = ((unsigned long long)rc.w << 32) | rc.z;
@@ -623,17 +561,17 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
         const uint8_t cl = cls[x];
         if (x == root) res = 0.0;
         else if (cl == VALID) { res = Qrow[vert[x]]; hnt[x] = (int32_t)parl[x]; }
-        else if (cl == UNREACH) res = 100.0;  // nx.NetworkXNoPath -> 100 (disconnected vicinity; status 3 later)
+        else if (cl == UNREACH) res = NO_PATH_DIST;  // nx.NetworkXNoPath (disconnected vicinity; status 3 later)
         else {
           hnt[x] = (int32_t)parl[x];
-          PySumT ps{0.0, 0.0, 0};
+          PySum ps{0.0, 0.0, 0};
           int y = x, guard = 0;
           while (y != root && guard++ <= n) {
             const int py = (int)parl[y];
-            pyt_add(ps, __longlong_as_double((long long)dist[y]), plain);
+            pysum_add(ps, __longlong_as_double((long long)dist[y]), plain);
             y = py;
           }
-          res = pyt_get(ps, plain);
+          res = pysum_get(ps, plain);
         }
         out[x] = res;
       }
@@ -642,8 +580,7 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
     }
     if (!two) for (int x = tid; x < n; x += nt) d2[x] = d1[x];
     __syncthreads();
-    // `if x in [root_1, root_2]`: all three attributes 0   riccidist2dgm.py:22-25
-    if (tid == 0) { d1[lu] = 0.0; d2[lu] = 0.0; d1[lv] = 0.0; d2[lv] = 0.0; }
+    if (tid == 0) zero_roots(d1, d2, lu, lv);
   }
   __syncthreads();
 
@@ -651,28 +588,17 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
   double mx = -1.0, sm = -1.0;
   for (int x = tid; x < n; x += nt) {
     const double a = d1[x], b = d2[x];
-    mx = fmax(mx, fmax(a, b));
-    sm = fmax(sm, node_mode ? a : __dadd_rn(a, b));
+    mx = fmax(mx, fv_descriptor(TLC_DESC_MAX, node_mode, a, b));
+    sm = fmax(sm, fv_descriptor(TLC_DESC_SUM, node_mode, a, b));
   }
   double smax = block_reduce_max(mx, sh.redd);
   double ssum = block_reduce_max(sm, sh.redd);
   const bool norm = (p.flags & TLC_F_NORM) != 0;
-  if (norm) {
-    if (p.flags & TLC_F_NORM_EPS) { smax = __dadd_rn(smax, 1e-10); ssum = __dadd_rn(ssum, 1e-10); }
-    else if (smax == 0.0 || ssum == 0.0) {  // ZeroDivisionError -> zeros   riccidist2dgm.py:54-56,356-357
-      if (tid == 0) c.tstatus[t] = TLC_ST_DEGENERATE;
-      return;
-    }
+  if (norm && !fv_normalisers(p.flags, smax, ssum)) {
+    if (tid == 0) c.tstatus[t] = TLC_ST_DEGENERATE;
+    return;
   }
-  for (int x = tid; x < n; x += nt) {
-    const double a = d1[x], b = d2[x];
-    double f;
-    if (p.descriptor == TLC_DESC_MIN) f = fmin(a, b);
-    else if (p.descriptor == TLC_DESC_MAX) f = fmax(a, b);
-    else f = node_mode ? a : __dadd_rn(a, b);
-    if (norm) f = __ddiv_rn(f, p.descriptor == TLC_DESC_SUM ? ssum : smax);
-    fval[x] = f;
-  }
+  for (int x = tid; x < n; x += nt) fval[x] = fv_value(p.descriptor, node_mode, norm, smax, ssum, d1[x], d2[x]);
   TPROF(10);
 }
 

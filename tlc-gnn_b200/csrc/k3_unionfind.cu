@@ -20,16 +20,6 @@
 namespace tlc {
 namespace {
 
-__device__ __forceinline__ int uf_find(int32_t* p, int x) {  // path halving  accelerated_PD.py:53-58
-  for (;;) {
-    const int px = p[x];
-    if (px == x) return x;
-    const int gp = p[px];
-    p[x] = gp;
-    x = gp;
-  }
-}
-
 struct UfShared {
   int32_t cl_k[1024], cl_a[1024], cl_b[1024];
   int32_t wcnt[33];

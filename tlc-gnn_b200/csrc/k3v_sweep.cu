@@ -35,17 +35,6 @@ struct RepBuf {
   int32_t perm[REP_CAP];
 };
 
-template <typename PT>
-__device__ __forceinline__ int find_root(PT* p, int x) {  // path halving  accelerated_PD.py:53-58
-  for (;;) {
-    const int px = (int)p[x];
-    if (px == x) return x;
-    const int gp = (int)p[px];
-    p[x] = (PT)gp;
-    x = gp;
-  }
-}
-
 __device__ __forceinline__ bool rep_less(unsigned long long ka, int la, int ha, unsigned long long kb, int lb, int hb) {
   if (ka != kb) return ka < kb;
   if (la != lb) return la < lb;  // canonical edge index order == lexicographic (lo, hi)
@@ -136,7 +125,7 @@ __global__ void __launch_bounds__(SWEEP_WARPS * 32) sweep_kernel(Params p, Chunk
         const bool triv = lane >= nbk || ((cur_first >> 30) & 3) == 1;  // bit 30 set, bit 31 clear
         if (__all_sync(FULL, triv)) {
           const int ge = (nbk < 32 ? __shfl_sync(FULL, cur_first, nbk) : __shfl_sync(FULL, nxt_first, 0)) & 0x3fffffff;
-          const int R = find_root(parent, 0);
+          const int R = uf_find(parent, 0);
           __syncwarp();
           for (int x = s + lane; x < ge; x += 32) parent[x] = (PT)R;
           __syncwarp();
@@ -162,7 +151,7 @@ __global__ void __launch_bounds__(SWEEP_WARPS * 32) sweep_kernel(Params p, Chunk
       bool ok = true;
       if (ncomp == 1) {
         // the processed prefix is ONE component: every earlier-block neighbour is in it, no row needs reading
-        R = find_root(parent, 0);
+        R = uf_find(parent, 0);
       } else {
         nrowcheck++;
         // several components below: all earlier-block neighbours of the block must share one root
@@ -174,7 +163,7 @@ __global__ void __launch_bounds__(SWEEP_WARPS * 32) sweep_kernel(Params p, Chunk
             const int ly = j < dg ? nbr(a + j) : -1;
             const int ry = ly >= 0 ? vrank[ly] : e;  // e: "not in an earlier block", ignored
             const bool out = ry < s;
-            const int rt = out ? find_root(parent, ry) : -1;
+            const int rt = out ? uf_find(parent, ry) : -1;
             const unsigned bo = __ballot_sync(FULL, out);
             if (bo) {
               if (R < 0) R = __shfl_sync(FULL, rt, __ffs(bo) - 1);
@@ -234,7 +223,7 @@ __global__ void __launch_bounds__(SWEEP_WARPS * 32) sweep_kernel(Params p, Chunk
             }
           }
           if (valid) {
-            ry = find_root(parent, y);  // no union has happened in this block yet: component at block start
+            ry = uf_find(parent, y);  // no union has happened in this block yet: component at block start
             K = f64_to_ordered(key_asc(fx, fval[ly]));
             lo = min(lx, ly); hi = max(lx, ly);
           }
@@ -279,7 +268,7 @@ __global__ void __launch_bounds__(SWEEP_WARPS * 32) sweep_kernel(Params p, Chunk
         __syncwarp();
         // the reference's union step for edge [a, b], a < b (local ids); lane 0 only
         auto apply_edge = [&](int a, int bb) {
-          const int A = find_root(parent, vrank[a]), B = find_root(parent, vrank[bb]);
+          const int A = uf_find(parent, vrank[a]), B = uf_find(parent, vrank[bb]);
           if (A == B) return;
           const int la = vord[A], lb = vord[B];  // local ids of the two roots
           const double fA = fval[la], fB = fval[lb];

@@ -15,28 +15,13 @@
 namespace tlc {
 namespace {
 
-__device__ __forceinline__ double norm_cdf(double x) {  // erfc(-x / sqrt(2)) / 2   PersistenceImager.pyx:60
-  return erfc(-x / 1.4142135623730951) * 0.5;
-}
-
-__device__ __forceinline__ double ramp_weight(double pers) {  // linear_ramp defaults  :22-28
-  return pers < 0.0 ? 0.0 : (pers > 1.0 ? 1.0 : pers);
-}
-
 template <int RES>
 __device__ __forceinline__ void splat_point(double birth, double death, double step, double* acc) {
   const double pers = death - birth;  // skew :366
   const double w = ramp_weight(pers);
   if (w == 0.0) return;
   double gb[RES > 0 ? RES : 1], gp[RES > 0 ? RES : 1];
-  double pb = norm_cdf(0.0 - birth), pp = norm_cdf(0.0 - pers);
-#pragma unroll
-  for (int i = 1; i <= RES; i++) {
-    const double pt = i * step;
-    const double cb = norm_cdf(pt - birth), cp = norm_cdf(pt - pers);
-    gb[i - 1] = cb - pb; gp[i - 1] = cp - pp;
-    pb = cb; pp = cp;
-  }
+  cdf_diffs(RES, step, birth, pers, gb, gp);
 #pragma unroll
   for (int i = 0; i < RES; i++) {
     const double wb = w * gb[i];
@@ -51,13 +36,7 @@ __device__ void splat_point_generic(int res, double birth, double death, double 
   const double w = ramp_weight(pers);
   if (w == 0.0) return;
   double gb[16], gp[16];
-  double pb = norm_cdf(0.0 - birth), pp = norm_cdf(0.0 - pers);
-  for (int i = 1; i <= res; i++) {
-    const double pt = i * step;
-    const double cb = norm_cdf(pt - birth), cp = norm_cdf(pt - pers);
-    gb[i - 1] = cb - pb; gp[i - 1] = cp - pp;
-    pb = cb; pp = cp;
-  }
+  cdf_diffs(res, step, birth, pers, gb, gp);
   for (int i = 0; i < res; i++)
     for (int j = 0; j < res; j++) atomicAdd(&simg[i * res + j], w * gb[i] * gp[j]);
 }

@@ -47,8 +47,6 @@ struct RicciArgs {
   int32_t* iters;          // [nnz] or nullptr: Sinkhorn iterations spent
 };
 
-__device__ __forceinline__ bool bit_of(const uint32_t* bm, int y) { return (bm[y >> 5] >> (y & 31)) & 1u; }
-
 __device__ inline double block_sum(double v, double* red) {
   for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   const int w = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
@@ -105,7 +103,7 @@ __global__ void __launch_bounds__(256) ricci_kernel(RicciArgs a) {
       const uint32_t* b2 = a.ball2 + (size_t)an * a.W;
       for (int j = lane; j < nb; j += 32) {
         const int bn = sv[j];
-        codes[(size_t)i * nb + j] = bn == an ? 0 : (bit_of(b1, bn) ? 1 : (bit_of(b2, bn) ? 2 : 3));
+        codes[(size_t)i * nb + j] = bn == an ? 0 : (test_bit(b1, bn) ? 1 : (test_bit(b2, bn) ? 2 : 3));
       }
     }
     __syncthreads();

@@ -87,6 +87,17 @@ __device__ __forceinline__ unsigned lanemask_lt() {
   return m;
 }
 
+// bit pattern of +inf: the distance of a vertex no relaxation has reached (distances are compared as u64 bit patterns)
+constexpr unsigned long long INF_BITS = 0x7ff0000000000000ull;
+
+__device__ __forceinline__ bool test_bit(const uint32_t* bm, int32_t y) { return (bm[y >> 5] >> (y & 31)) & 1u; }
+
+__device__ __forceinline__ unsigned long long warp_min_u64(unsigned long long v) {
+#pragma unroll
+  for (int o = 16; o; o >>= 1) { const unsigned long long u = __shfl_xor_sync(0xffffffffu, v, o); v = u < v ? u : v; }
+  return v;
+}
+
 // graph-row route: local id of graph node g in the vicinity whose bitmap / word prefix is bm[0..W) / bm[W..2W), -1 if absent
 __device__ __forceinline__ int bitmap_rank(const uint32_t* bm, int W, int g) {
   const uint32_t word = bm[g >> 5];
@@ -150,6 +161,30 @@ __device__ inline int block_exclusive_scan(int32_t* data, int n, int32_t* sh) {
   return total;
 }
 
+// exclusive scan of data[0..cnt) in shared memory, two barriers; returns the total.  `wsum` needs 33 ints.  All threads call.
+__device__ inline int block_scan_shfl(int32_t* data, int cnt, int32_t* wsum) {
+  const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, wid = tid >> 5, nw = (nt + 31) >> 5;
+  const int per = (cnt + nt - 1) / nt;
+  const int lo = min(tid * per, cnt), hi = min(lo + per, cnt);
+  int s = 0;
+  for (int i = lo; i < hi; i++) s += data[i];
+  int inc = s;
+  for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
+  if (lane == 31) wsum[wid] = inc;
+  __syncthreads();
+  if (wid == 0) {
+    const int wv = lane < nw ? wsum[lane] : 0;
+    int winc = wv;
+    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, winc, o); if (lane >= o) winc += v; }
+    if (lane < nw) wsum[lane] = winc - wv;
+    if (lane == 31) wsum[32] = winc;
+  }
+  __syncthreads();
+  int run = wsum[wid] + inc - s;
+  for (int i = lo; i < hi; i++) { const int v = data[i]; data[i] = run; run += v; }
+  return wsum[32];
+}
+
 __device__ inline int block_reduce_sum(int v, int32_t* sh) {
   for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   const int w = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
@@ -172,6 +207,115 @@ __device__ inline double block_reduce_max(double v, double* sh) {
   for (int i = 1; i < nw; i++) t = fmax(t, sh[i]);
   __syncthreads();
   return t;
+}
+
+// ---------------------------------------------------------------------------------------------
+// the reference's arithmetic, one definition for every kernel (the parity tests pin each IEEE operation order)
+// ---------------------------------------------------------------------------------------------
+// dict_node[u] KeyError (riccidist2dgm.py:353): an endpoint outside the graph; the reference graph has no isolated nodes
+__device__ __forceinline__ bool unknown_target(const GraphView& g, int32_t u, int32_t v, bool node_mode) {
+  bool bad = u < 0 || u >= g.N || (!node_mode && (v < 0 || v >= g.N));
+  if (!bad) bad = g.rowptr[u + 1] == g.rowptr[u] || (!node_mode && g.rowptr[v + 1] == g.rowptr[v]);
+  return bad;
+}
+
+// kernels 1b / 1t, graph-row route: the vicinity bitmap of target t from its cached balls into bm[0..W) and its word-prefix
+// ranks into bm[W..2W) (both in shared memory), copied to c.dbm for kernels 2v / 3v; returns n.  The whole CTA calls.
+// nodes = set(nodes_u) & set(nodes_v), canonical local ids = ranks   riccidist2dgm.py:311-316
+__device__ __forceinline__ int graph_row_bitmap(const ChunkView& c, int t, const uint32_t* ball_cache, int W, int32_t u,
+                                                int32_t v, bool node_mode, uint32_t* bm, int32_t* wsum) {
+  const int tid = threadIdx.x, nt = blockDim.x;
+  const uint32_t* __restrict__ bu = ball_cache + (size_t)u * W;
+  const uint32_t* __restrict__ bv = ball_cache + (size_t)v * W;
+  for (int w = tid; w < W; w += nt) {
+    const uint32_t x = node_mode ? bu[w] : (bu[w] & bv[w]);
+    bm[w] = x;
+    bm[W + w] = __popc(x);
+  }
+  __syncthreads();
+  const int n = block_scan_shfl(reinterpret_cast<int32_t*>(bm + W), W, wsum);
+  __syncthreads();
+  uint32_t* gb = c.dbm + (size_t)t * 2 * W;
+  for (int w = tid; w < 2 * W; w += nt) gb[w] = bm[w];
+  return n;
+}
+
+// nx.NodeNotFound (a root outside the vicinity) / nx.NetworkXNoPath -> dist = 100   riccidist2dgm.py:31-32,36-37
+constexpr double NO_PATH_DIST = 100.0;
+
+// `if x in [root_1, root_2]`: all three attributes 0   riccidist2dgm.py:22-25
+template <typename T>
+__device__ __forceinline__ void zero_roots(T* d1, T* d2, int lu, int lv) {
+  d1[lu] = T(0); d2[lu] = T(0); d1[lv] = T(0); d2[lv] = T(0);
+}
+
+struct PySum {  // CPython's float sum(): first item exact, then Neumaier (3.12+) or plain adds   SURVEY.md F5
+  double s, c;
+  int k;
+};
+__device__ __forceinline__ void pysum_add(PySum& p, double x, bool plain) {
+  if (p.k == 0) { p.s = x; p.k = 1; return; }
+  if (plain) { p.s = __dadd_rn(p.s, x); return; }
+  const double t = __dadd_rn(p.s, x);
+  if (fabs(p.s) >= fabs(x)) p.c = __dadd_rn(p.c, __dadd_rn(__dadd_rn(p.s, -t), x));
+  else p.c = __dadd_rn(p.c, __dadd_rn(__dadd_rn(x, -t), p.s));
+  p.s = t;
+}
+__device__ __forceinline__ double pysum_get(const PySum& p, bool plain) {
+  if (p.k == 0) return 0.0;
+  if (!plain && p.c != 0.0 && isfinite(p.c)) return __dadd_rn(p.s, p.c);
+  return p.s;
+}
+
+// build_fv's descriptor of one vertex from its distances a, b to the two roots   riccidist2dgm.py:47-53 ; data_utils_NC.py:52-54
+__device__ __forceinline__ double fv_descriptor(int descriptor, bool node_mode, double a, double b) {
+  if (descriptor == TLC_DESC_MIN) return fmin(a, b);
+  if (descriptor == TLC_DESC_MAX) return fmax(a, b);
+  return node_mode ? a : __dadd_rn(a, b);
+}
+// build_fv's normalisers (:54-56): smax / ssum, the vicinity's largest MAX / SUM descriptor, + 1e-10 with TLC_F_NORM_EPS.
+// Without it a zero normaliser raises ZeroDivisionError (the target gets zeros, :356-357): returns false.
+__device__ __forceinline__ bool fv_normalisers(uint32_t flags, double& smax, double& ssum) {
+  if (flags & TLC_F_NORM_EPS) { smax = __dadd_rn(smax, 1e-10); ssum = __dadd_rn(ssum, 1e-10); return true; }
+  return !(smax == 0.0 || ssum == 0.0);
+}
+__device__ __forceinline__ double fv_value(int descriptor, bool node_mode, bool norm, double smax, double ssum, double a,
+                                           double b) {
+  double f = fv_descriptor(descriptor, node_mode, a, b);
+  if (norm) f = __ddiv_rn(f, descriptor == TLC_DESC_SUM ? ssum : smax);
+  return f;
+}
+
+// find with path halving   accelerated_PD.py:53-58
+template <typename PT>
+__device__ __forceinline__ int uf_find(PT* p, int x) {
+  for (;;) {
+    const int px = (int)p[x];
+    if (px == x) return x;
+    const int gp = (int)p[px];
+    p[x] = (PT)gp;
+    x = gp;
+  }
+}
+
+// the persistence image's per-point factors: PersistenceImager.transform (PersistenceImager.pyx:352-388), isotropic
+// sigma = 1, skew (persistence = death - birth, :366)
+__device__ __forceinline__ double norm_cdf(double x) {  // erfc(-x / sqrt(2)) / 2   :60
+  return erfc(-x / 1.4142135623730951) * 0.5;
+}
+__device__ __forceinline__ double ramp_weight(double pers) {  // linear_ramp defaults  :22-28
+  return pers < 0.0 ? 0.0 : (pers > 1.0 ? 1.0 : pers);
+}
+// the point's CDF differences over the pixels of both axes, mesh i * step (i = 0 .. res)   :302-314,385-388
+__device__ __forceinline__ void cdf_diffs(int res, double step, double birth, double pers, double* gb, double* gp) {
+  double pb = norm_cdf(0.0 - birth), pp = norm_cdf(0.0 - pers);
+#pragma unroll
+  for (int i = 1; i <= res; i++) {
+    const double pt = i * step;
+    const double cb = norm_cdf(pt - birth), cp = norm_cdf(pt - pers);
+    gb[i - 1] = cb - pb; gp[i - 1] = cp - pp;
+    pb = cb; pp = cp;
+  }
 }
 
 // ---------------------------------------------------------------------------------------------
