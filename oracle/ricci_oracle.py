@@ -11,8 +11,9 @@ pinned in its requirements.txt, and neither is installed here (no network): `Gra
 POT 0.8 ot/bregman.py sinkhorn_knopp) for the reference's call -- an unweighted nx.Graph, so every edge weight is 1:
 
   * mass distribution of a node x (`_get_single_node_neighbors_distributions`): neighbour weights base ** (-w ** exp_power)
-    = e ** -1 each, normalised -> (1 - alpha) / deg(x) on every neighbour, alpha on x itself; only the nbr_topk = 3000
-    neighbours with the largest (weight, id) are kept (a heap of that size);
+    = e ** -1 each, normalised by their python sum() -> (1 - alpha) * e^-1 / (e^-1 added k times) on each of the k
+    kept neighbours, alpha on x itself; only the nbr_topk = 3000 neighbours with the largest (weight, id) are kept (a
+    heap of that size);
   * cost matrix d = all-pairs shortest path lengths between the two supports (`_apsp[np.ix_(src, tgt)]`): hop counts,
     0..3 for the supports of an edge;
   * m = ot.sinkhorn2(x, y, d, 1e-1, method='sinkhorn'): K = exp(d / -reg); u = 1/dim_a, v = 1/dim_b; repeat
@@ -45,7 +46,12 @@ def support(rowptr, col, x, alpha=ALPHA, topk=NBR_TOPK):
     if nb.size > topk:  # the heap keeps the topk largest (weight, id) tuples; all weights are equal here
         nb = np.sort(nb)[-topk:]
     w = np.full(nb.size, np.e ** (-1.0 ** 2))
-    s = w.sum()
+    # The weights are normalised by their sum added left to right, one weight at a time: GraphRicciCurvature adds them
+    # with python's sum(), which does exactly that on CPython <= 3.11 (the reference pins 3.7).  Neither numpy's
+    # pairwise w.sum() nor the compensated sum() of CPython >= 3.12 gives the same bits for k = 120, 121, 1024, 3000.
+    s = 0.0
+    for t in w.tolist():
+        s += t
     dist = (1.0 - alpha) * w / s
     return np.concatenate([dist, [alpha]]), np.concatenate([nb, [x]])
 
@@ -80,6 +86,23 @@ def hop_costs(rowptr, col, src, tgt):
     return d
 
 
+def support_costs(rowptr, col, src, tgt):
+    """hop_costs for the two supports of an edge, built from the sparse adjacency instead of one BFS per source: with
+    B = A + I, the distance is 0 on the diagonal, 1 where B[a, b] > 0, 2 where (B B)[a, b] > 0, else 3.  Valid only
+    where every distance is at most 3 -- true for an edge's supports (neighbour - x - y - neighbour)."""
+    import scipy.sparse as sp
+    N = len(rowptr) - 1
+    A = sp.csr_matrix((np.ones(len(col)), np.asarray(col), np.asarray(rowptr)), shape=(N, N))
+    B = (A + sp.identity(N, format="csr")).tocsr()
+    src = np.asarray(src, dtype=np.int64)
+    tgt = np.asarray(tgt, dtype=np.int64)
+    bs, bt = B[src], B[tgt]
+    one = bs[:, tgt].toarray() > 0
+    two = (bs @ bt.T).toarray() > 0                    # B is symmetric: (B B)[src][:, tgt] = B[src] B[tgt]^T
+    same = src[:, None] == tgt[None, :]
+    return 3.0 - one - two - same
+
+
 def sinkhorn2(a, b, M, reg=REG, num_iter_max=NUM_ITER_MAX, stop_thr=STOP_THR):
     """POT's sinkhorn_knopp loss for one pair of histograms (ot/bregman.py)"""
     a = np.asarray(a, dtype=np.float64)
@@ -88,27 +111,29 @@ def sinkhorn2(a, b, M, reg=REG, num_iter_max=NUM_ITER_MAX, stop_thr=STOP_THR):
     u = np.ones(len(a)) / len(a)
     v = np.ones(len(b)) / len(b)
     K = np.exp(M / (-reg))
-    Kp = (1.0 / a).reshape(-1, 1) * K
     cpt, err = 0, 1.0
-    while err > stop_thr and cpt < num_iter_max:
-        uprev, vprev = u, v
-        KtU = K.T @ u
-        v = b / KtU
-        u = 1.0 / (Kp @ v)
-        if (np.any(KtU == 0) or np.any(np.isnan(u)) or np.any(np.isnan(v)) or np.any(np.isinf(u)) or np.any(np.isinf(v))):
-            u, v = uprev, vprev
-            break
-        if cpt % 10 == 0:
-            tmp2 = np.einsum("i,ij,j->j", u, K, v)
-            err = np.linalg.norm(tmp2 - b)
-        cpt += 1
+    with np.errstate(divide="ignore", invalid="ignore"):   # a zero mass (alpha = 0 or 1) ends the loop through inf * 0
+        Kp = (1.0 / a).reshape(-1, 1) * K
+        while err > stop_thr and cpt < num_iter_max:
+            uprev, vprev = u, v
+            KtU = K.T @ u
+            v = b / KtU
+            u = 1.0 / (Kp @ v)
+            if (np.any(KtU == 0) or np.any(np.isnan(u)) or np.any(np.isnan(v)) or np.any(np.isinf(u))
+                    or np.any(np.isinf(v))):
+                u, v = uprev, vprev
+                break
+            if cpt % 10 == 0:
+                tmp2 = np.einsum("i,ij,j->j", u, K, v)
+                err = np.linalg.norm(tmp2 - b)
+            cpt += 1
     return float(np.sum(u.reshape(-1, 1) * K * v.reshape(1, -1) * M)), cpt
 
 
 def edge_curvature(rowptr, col, x, y):
     a, src = support(rowptr, col, x)
     b, tgt = support(rowptr, col, y)
-    d = hop_costs(rowptr, col, src, tgt)
+    d = support_costs(rowptr, col, src, tgt)
     m, _ = sinkhorn2(a, b, d)
     return 1.0 - m / 1.0
 

@@ -3,6 +3,7 @@ import os
 
 import numpy as np
 
+import ricci_oracle as ro
 from tlc_b200 import graphgen as gg
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -56,6 +57,49 @@ def kd_seg(c, name, k):
     off = c["kd_%s_off" % name]
     w = 2 if name in ("ord0", "ext1", "edge_index") else 1  # offsets count rows; these are [rows, 2] flattened
     return c["kd_%s" % name][w * off[k]:w * off[k + 1]]
+
+
+def ricci_hub_graph():
+    """graph for kernel 6's three launch classes (support = min(degree, 3000) + 1; an edge's class comes from its larger
+    support: <= 120, <= 1024, <= 3001).  Deterministic, N = 3621 (not a multiple of 32).  Returns (rowptr, col, ids):
+      h3500 = N - 1 (the last bitmap word; always the larger endpoint), h3001, h3000 (mid-range ids: the smaller endpoint
+      of some edges, the larger of others), d1024, d1023, d120, d119: nodes of exactly that degree;
+      boundary pairs h3500-h3001 and h3001-h3000 (3001 x 3001 codes), d1024-d1023, d120-d119;
+      cut: a node adjacent to h3500 and to 8 of the 500 smallest neighbours of h3500 -- the ones the cut to 3000 drops;
+    every other node is plain, adjacent to a random subset of the above plus a sparse random background (degree <= 30)."""
+    N = 3621
+    rs = np.random.RandomState(5)
+    ids = dict(h3500=N - 1, h3001=1801, h3000=1200, d1024=2400, d1023=600, d120=3000, d119=300, cut=2999)
+    deg = dict(h3500=3500, h3001=3001, h3000=3000, d1024=1024, d1023=1023, d120=120, d119=119)
+    pairs = [("h3500", "h3001"), ("h3001", "h3000"), ("d1024", "d1023"), ("d120", "d119")]
+    edges = [(ids[p], ids[q]) for p, q in pairs]
+    plain = np.setdiff1d(np.arange(N), list(ids.values()))
+    for name, d in deg.items():
+        need = d - sum(name in pq for pq in pairs) - (name == "h3500")
+        edges += [(ids[name], int(y)) for y in np.sort(rs.choice(plain, need, replace=False))]
+    edges.append((ids["cut"], ids["h3500"]))
+    h_nb = np.sort([y for x, y in edges if x == ids["h3500"]])
+    edges += [(ids["cut"], int(y)) for y in h_nb[:8]]
+    bg = rs.choice(plain, (2 * N, 2))
+    edges += [(int(a), int(b)) for a, b in bg if a != b]
+    e = np.asarray(edges, dtype=np.int64)
+    e = np.unique(np.stack([e.min(1), e.max(1)], 1), axis=0)
+    rp, col, _ = gg.build_csr(N, e, np.zeros(len(e)))
+    dg = np.diff(rp)
+    assert all(dg[ids[k]] == d for k, d in deg.items()) and dg[plain].max() <= 30 and dg[ids["cut"]] == 9
+    assert np.all(np.isin(col[rp[ids["cut"]]:rp[ids["cut"] + 1]], np.append(h_nb[:8], ids["h3500"])))
+    return rp, col, ids
+
+
+def ricci_classes(rowptr, col):
+    """(x < y) edges in CSR order and their kernel-6 launch class: 0 (larger support <= 120), 1 (<= 1024), 2 (the rest)"""
+    deg = np.diff(np.asarray(rowptr, dtype=np.int64))
+    src = np.repeat(np.arange(len(deg)), deg)
+    keep = src < col
+    e = np.stack([src[keep], np.asarray(col, dtype=np.int64)[keep]], 1)
+    size = np.minimum(deg, ro.NBR_TOPK) + 1
+    big = np.maximum(size[e[:, 0]], size[e[:, 1]])
+    return e, np.where(big <= 120, 0, np.where(big <= 1024, 1, 2))
 
 
 def sorted_rows(a):
