@@ -156,6 +156,13 @@ __global__ void ball_mark_kernel(const int32_t* __restrict__ targets, int64_t E,
   }
 }
 
+__global__ void ball_mark_all_kernel(GraphView g, VicinityScratch vs) {  // every node with an edge whose ball is not cached yet
+  for (int x = blockIdx.x * blockDim.x + threadIdx.x; x < g.N; x += gridDim.x * blockDim.x) {
+    if (g.rowptr[x + 1] == g.rowptr[x]) continue;
+    if (vs.ball_state[x] == 0 && atomicCAS(&vs.ball_state[x], 0, 1) == 0) vs.ball_list[atomicAdd(vs.ball_count, 1)] = x;
+  }
+}
+
 __global__ void __launch_bounds__(K1_BLOCK)
 ball_build_kernel(GraphView g, Params p, VicinityScratch vs, int W, int bm_in_smem) {
   extern __shared__ uint32_t dyn_smem[];
@@ -460,15 +467,20 @@ static void set_smem(const void* fn, size_t bytes) {
   if (bytes > 48 * 1024) cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
+// targets == nullptr: the ball of every node with an edge (kernel 1t's table build needs them all)
 void launch_ball_cache(const GraphView& g, const Params& p, const int32_t* targets, int64_t E, const VicinityScratch& vs,
                        cudaStream_t st) {
-  if (!vs.ball_cache || E <= 0) return;
+  if (!vs.ball_cache || (targets && E <= 0)) return;
   const int W = (g.N + 31) / 32;
   const bool smem = vs.bitmaps == nullptr;
   const size_t bytes = smem ? (size_t)2 * W * 4 : 0;
   cudaMemsetAsync(vs.ball_count, 0, sizeof(int), st);
-  const int mgrid = (int)std::min<int64_t>((2 * E + 255) / 256, 4096);
-  ball_mark_kernel<<<mgrid, 256, 0, st>>>(targets, E, p.mode == TLC_MODE_NODE ? 1 : 0, g, vs);
+  if (targets) {
+    const int mgrid = (int)std::min<int64_t>((2 * E + 255) / 256, 4096);
+    ball_mark_kernel<<<mgrid, 256, 0, st>>>(targets, E, p.mode == TLC_MODE_NODE ? 1 : 0, g, vs);
+  } else {
+    ball_mark_all_kernel<<<(g.N + 255) / 256, 256, 0, st>>>(g, vs);
+  }
   count_launch();
   set_smem((const void*)ball_build_kernel, bytes);
   ball_build_kernel<<<vs.grid, K1_BLOCK, bytes, st>>>(g, p, vs, W, smem ? 1 : 0);

@@ -1,18 +1,28 @@
-// k1t_sssp_table.cu -- kernel 1t: the node filtration from a per-ROOT shortest-path table of the whole graph.
+// k1t_sssp_table.cu -- kernel 1t: the node filtration from a per-ROOT shortest-path table of the root's k-hop ball.
 //
 // build_fv (riccidist2dgm.py:20-61) needs, for a target (u, v), the shortest-path distances from u and from v INSIDE the
 // vicinity S.  Kernel 1b runs one Dijkstra per root and target.  On graphs small enough to afford O(N^2) entries the
-// same values come from a table that is built ONCE per graph and root r over the WHOLE graph G:
-//     D_r[x] = least fixpoint of d[y] = min_x fl(d[x] + w(x, y)) on G          (what Dijkstra returns, fl(+) monotone)
+// same values come from a table that is built ONCE per graph, hop k and root r over G'_r, the subgraph of G induced by
+// r's closed k-hop ball:
+//     D_r[x] = least fixpoint of d[y] = min_x fl(d[x] + w(x, y)) on G'_r       (what Dijkstra returns, fl(+) monotone)
 //     P_r[x] = smallest id y with fl(D_r[y] + w(y, x)) == D_r[x]               (the tree rule of kernel 1b / the oracle)
 //     Q_r[x] = python-order sum of the weights along x -> P_r[x] -> ... -> r   (:30,35, SURVEY.md F5)
 //     W_r[x] = w(x, P_r[x]), the weight of the tree edge (the walks of the vertices below need it term by term)
+// The proof below needs two facts: S is a vertex subset of G'_r, and the edges of S are edges of G'_r.  Both hold on
+// the two modes that reach this kernel: TLC_MODE_EDGE (S = ball(u) & ball(v), induced) and TLC_MODE_NODE (S = ball(u));
+// not on FORCED, UNION or REMOVEINTER, whose S leaves a root's ball (the host never gives those the tables).
 // For a vicinity S containing r call x VALID when its whole tree branch x -> ... -> r lies in S.  Then, exactly:
 //   * d_S[x] == D_r[x]: d_S >= D_r (fewer edges), and along the branch d_S[x] <= fl(d_S[p] + w) = fl(D_r[p] + w) = D_r[x];
-//   * the tree parent inside S is P_r[x]: every candidate y in S (fl(d_S[y] + w) == d_S[x]) is a candidate in G as well
-//     (D_r[y] <= d_S[y] and D_r[x] is minimal), and P_r[x], the smallest candidate of G, lies in S with d_S = D_r;
+//   * the tree parent inside S is P_r[x]: every candidate y in S (fl(d_S[y] + w) == d_S[x]) is a candidate in G'_r as
+//     well (D_r[y] <= d_S[y] and D_r[x] is minimal), and P_r[x], the smallest candidate of G'_r, lies in S with d_S = D_r;
 //   * hence the path and its python-order sum are Q_r[x].
-// The other vertices of S (their branch leaves S: 10-20 % on the Computers-shaped 2-hop vicinities, 0.3 % on the largest)
+// The ball table leaves no more vertices invalid than a table over the whole graph G would: if x's branch in G's tree
+// lies in S, then along that branch (induction from r) the G'_r values equal G's -- D' >= D (fewer edges), the G branch
+// is a path of G'_r so D' <= D, and every G'_r candidate for the parent is a G candidate, so the smallest is the same.
+// Whole-graph shortest paths often leave the ball (weights kappa + 1 lie in (0.1, 1.9): a cheap path to a 2-hop vertex
+// through a hub 3 hops away); inside the ball most of those vertices become valid.
+// The other vertices of S (their branch leaves S: 5 % of the Computers-shaped 2-hop vicinities, from 2 % on the largest
+// quarter to 17 % on the smallest -- scripts/table_census.py; 10 % with whole-graph tables)
 // get their distance from the same fixpoint restricted to them, the valid vertices acting as settled sources: ONE pass of
 // "pull" relaxations over THEIR graph rows (which also lists the adjacencies among the invalid vertices), further rounds
 // over that list only, then the tree rule and the path walk (parents and tree-edge weights of all vertices in shared
@@ -32,7 +42,7 @@ namespace tlc {
 namespace {
 
 // ---------------------------------------------------------------------------------------------------------------------
-// table build: one CTA per root, whole graph, distances + parents in shared memory
+// table build: one CTA per root, the root's ball, distances + parents in shared memory
 // ---------------------------------------------------------------------------------------------------------------------
 __global__ void sssp_mark_kernel(const int32_t* __restrict__ targets, int64_t E, int node_mode, GraphView g, SsspTables tb) {
   const int64_t total = 2 * E;
@@ -59,21 +69,29 @@ struct BuildShared {
   int32_t any;
 };
 
-__global__ void __launch_bounds__(1024) sssp_build_kernel(GraphView g, SsspTables tb, const float* __restrict__ gminw,
-                                                          double* __restrict__ pw_scratch, int plain) {
+// The graph of root r's table is G'_r, the subgraph induced by r's closed k-hop ball (the ball cache row of r, which must
+// hold the call's hop): an edge is relaxed only into a member of the ball.  Vertices outside it keep D = +inf, P = -1,
+// Q = NO_PATH_DIST, W = 0 (kernel 1t never reads them: S is a subset of the ball).  gminw, the smallest weight of a
+// vertex's WHOLE-graph row, stays a valid settling margin: the edges of G'_r into x are a subset of those of G, so their
+// smallest weight is at least gminw[x].
+__global__ void __launch_bounds__(1024) sssp_build_kernel(GraphView g, SsspTables tb, const uint32_t* __restrict__ ball_cache,
+                                                          const float* __restrict__ gminw, double* __restrict__ pw_scratch,
+                                                          int plain) {
   extern __shared__ __align__(16) unsigned long long bsm[];
   __shared__ BuildShared sh;
-  const int N = g.N;
+  const int N = g.N, W = (N + 31) / 32;
   const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, wid = tid >> 5, nw = nt >> 5;
   unsigned long long* dist = bsm;                                   // [N]
   int32_t* par = reinterpret_cast<int32_t*>(bsm + N);               // [N]
-  uint8_t* state = reinterpret_cast<uint8_t*>(par + N);             // [N]  0 far, 1 tentative, 2 done
+  uint32_t* ball = reinterpret_cast<uint32_t*>(par + N);            // [W]  the root's ball
+  uint8_t* state = reinterpret_cast<uint8_t*>(ball + W);            // [N]  0 far, 1 tentative, 2 done
   double* pw = pw_scratch + (size_t)blockIdx.x * N;                 // weight of the parent edge (global scratch of this CTA)
   const int cnt = *tb.count;
   for (int idx = blockIdx.x; idx < cnt; idx += gridDim.x) {
     const int32_t root = tb.list[idx];
     __syncthreads();
     for (int x = tid; x < N; x += nt) { dist[x] = INF_BITS; state[x] = 0; par[x] = -1; }
+    for (int w = tid; w < W; w += nt) ball[w] = ball_cache[(size_t)root * W + w];
     __syncthreads();
     if (tid == 0) { dist[root] = 0ull; state[root] = 1; }
     __syncthreads();
@@ -110,6 +128,7 @@ __global__ void __launch_bounds__(1024) sssp_build_kernel(GraphView g, SsspTable
         const int a = g.rowptr[x], b = g.rowptr[x + 1];
         for (int e = a + lane; e < b; e += 32) {
           const int y = g.col[e];
+          if (!test_bit(ball, y)) continue;
           const unsigned long long tbv = (unsigned long long)__double_as_longlong(__dadd_rn(dx, __dadd_rn(g.kappa[e], 1.0)));
           if (tbv < dist[y]) { atomicMin(&dist[y], tbv); if (state[y] == 0) state[y] = 1; }
         }
@@ -604,10 +623,11 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
 
 }  // namespace
 
-// build the table rows of the targets' endpoints that do not exist yet (once per graph and root)
+// build the table rows of the targets' endpoints that do not exist yet (once per graph, hop and root); the ball cache
+// must hold the ball of every root built
 // targets == nullptr: every node of the graph (the eager build of the first call)
 void launch_sssp_build(const GraphView& g, const Params& p, const int32_t* targets, int64_t E, const SsspTables& tb,
-                       const float* gminw, double* pw_scratch, int grid, cudaStream_t st) {
+                       const uint32_t* ball_cache, const float* gminw, double* pw_scratch, int grid, cudaStream_t st) {
   if (!tb.D) return;
   cudaMemsetAsync(tb.count, 0, sizeof(int), st);
   if (targets) {
@@ -618,14 +638,15 @@ void launch_sssp_build(const GraphView& g, const Params& p, const int32_t* targe
     sssp_mark_all_kernel<<<(g.N + 255) / 256, 256, 0, st>>>(g, tb);
   }
   count_launch();
-  const size_t bytes = (size_t)g.N * (8 + 4 + 1) + 16;
+  const size_t bytes = sssp_build_smem(g.N);
   cudaFuncSetAttribute((const void*)sssp_build_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
   cudaFuncSetAttribute((const void*)sssp_build_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  sssp_build_kernel<<<grid, 1024, bytes, st>>>(g, tb, gminw, pw_scratch, (p.flags & TLC_F_SUM_PLAIN) ? 1 : 0);
+  sssp_build_kernel<<<grid, 1024, bytes, st>>>(g, tb, ball_cache, gminw, pw_scratch, (p.flags & TLC_F_SUM_PLAIN) ? 1 : 0);
   count_launch();
 }
 
-size_t sssp_build_smem(int N) { return (size_t)N * (8 + 4 + 1) + 16; }
+// distances, parents, the root's ball bitmap, states (N = 16 384: 213 KB, 222 KB with the static BuildShared)
+size_t sssp_build_smem(int N) { return (size_t)N * (8 + 4 + 1) + (size_t)(N + 31) / 32 * 4 + 16; }
 
 void launch_filtration_table(const GraphView& g, const Params& p, const ChunkView& c, const VicinityScratch& vs,
                              const SsspTables& tb, int t0, int cnt, int block, int64_t n_max, cudaStream_t st) {

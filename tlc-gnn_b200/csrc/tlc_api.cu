@@ -188,10 +188,11 @@ struct tlc_graph {
   int small_skip = 0;              // calls left for which the small path is not tried (it handled too few rows)
   int small_hop = -1, small_mode = -1;
   double hks_time = 0.1;   // diffusion time of TLC_F_FILT_HKS (data_utils_NC.py: hks_time = 0.1)
-  // kernel 1t: per-root shortest-path tables of the whole graph (valid for sssp_plain), scratch of the build kernel
+  // kernel 1t: per-root shortest-path tables over the roots' k-hop balls (valid for sssp_plain and sssp_hop), scratch of
+  // the build kernel
   SsspTables sssp{};  // views of the sssp_* buffers, null until they exist
   DevBuf sssp_D, sssp_Q, sssp_P, sssp_PW, sssp_state, sssp_list, sssp_count, sssp_pw;
-  int sssp_plain = -1;
+  int sssp_plain = -1, sssp_hop = -1;
   bool sssp_tried = false, sssp_all = false;
   double sssp_build_ms = 0;   // device time of the (one-time) table build
   // multi-GPU exchange by peer stores: this rank's table, the mapped tables of all ranks, exchange epoch
@@ -316,7 +317,9 @@ static int prepare_call(tlc_graph* g, const Params& p, int64_t E) {
 }
 
 // kernel 1t's tables: four [N][N] arrays, allocated once when the graph is small enough (N <= 16384: the build kernel keeps a
-// root's whole distance / parent vector in shared memory) and 28 N^2 bytes fit TLC_SSSP_CACHE_GB (default 8, 0 disables)
+// root's whole distance / parent vector and ball in shared memory) and 28 N^2 bytes fit TLC_SSSP_CACHE_GB (default 8, 0
+// disables).  Their rows depend on the summation rule (path sums) and the hop (the ball each row is restricted to): a call
+// with another of either marks every row for rebuilding.
 static int ensure_sssp_tables(tlc_graph* g, const Params& p) {
   const int plain = (p.flags & TLC_F_SUM_PLAIN) ? 1 : 0;
   if (!g->sssp_tried) {
@@ -341,11 +344,13 @@ static int ensure_sssp_tables(tlc_graph* g, const Params& p) {
       g->sssp = SsspTables{g->sssp_D.as<double>(), g->sssp_Q.as<double>(), g->sssp_P.as<int32_t>(), g->sssp_PW.as<double>(),
                            g->sssp_state.as<int32_t>(), g->sssp_list.as<int32_t>(), g->sssp_count.as<int>()};
       g->sssp_plain = plain;
+      g->sssp_hop = p.hop;
     }
   }
-  if (g->sssp.D && g->sssp_plain != plain) {  // the path sums depend on the summation rule: rebuild
+  if (g->sssp.D && (g->sssp_plain != plain || g->sssp_hop != p.hop)) {
     CK(cudaMemsetAsync(g->sssp.state, 0, (size_t)g->gv.N * 4, g->stream));
     g->sssp_plain = plain;
+    g->sssp_hop = p.hop;
     g->sssp_all = false;
   }
   return TLC_OK;
@@ -597,18 +602,24 @@ static int choose_route(tlc_graph* g, const Params& p, const int32_t* d_targets,
       g->probe_hop = p.hop; g->probe_mode = p.mode; g->probe_age = 0; g->probe_direct = *direct;
     }
   }
-  if (*direct && !(p.flags & TLC_F_NO_TABLE) && !getenv("TLC_NO_TABLE")) {
+  // Kernel 1t's proof needs S to be a subset of each root's ball (the graph of the root's table row): true for EDGE
+  // (ball(u) & ball(v)) and NODE (ball(u)), not for FORCED, UNION or REMOVEINTER, which must never reach the tables.
+  const bool table_mode = p.mode == TLC_MODE_EDGE || p.mode == TLC_MODE_NODE;
+  if (*direct && table_mode && !(p.flags & TLC_F_NO_TABLE) && !getenv("TLC_NO_TABLE")) {
     int rc = ensure_sssp_tables(g, p);
     if (rc) return rc;
     if (g->sssp.D) {
       *use_table = true;
       if (!g->sssp_all) {
-        // the rows of ALL roots, once per graph (and summation rule): a full pass over a dataset touches every node anyway,
-        // and a handful of late rows would cost a whole single-CTA shortest-path run in the middle of a step
+        // the rows of ALL roots, once per graph (summation rule and hop): a full pass over a dataset touches every node
+        // anyway, and a handful of late rows would cost a whole single-CTA shortest-path run in the middle of a step.
+        // Every row needs its root's ball for this hop: prepare_call has already reset the ball cache on a hop change.
         cudaEvent_t b0 = nullptr, b1 = nullptr;
         cudaEventCreate(&b0); cudaEventCreate(&b1);
         cudaEventRecord(b0, st);
-        launch_sssp_build(g->gv, p, nullptr, 0, g->sssp, g->gminw.as<float>(), g->sssp_pw.as<double>(), g->sm_count, st);
+        launch_ball_cache(g->gv, p, nullptr, 0, vs, st);
+        launch_sssp_build(g->gv, p, nullptr, 0, g->sssp, vs.ball_cache, g->gminw.as<float>(), g->sssp_pw.as<double>(),
+                          g->sm_count, st);
         cudaEventRecord(b1, st);
         CK(cudaStreamSynchronize(st));
         float ms = 0;

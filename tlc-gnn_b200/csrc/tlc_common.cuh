@@ -369,9 +369,10 @@ void launch_gather_rows(const double* table, int64_t rows, int r2, const int64_t
 void launch_scatter_rows(const double* src_pi, const float* src_pi32, const uint8_t* src_st, const int64_t* idx, int64_t k,
                          int r2, double* dst_pi, float* dst_pi32, uint8_t* dst_st, int sm_count, cudaStream_t st);
 
-// kernel 1t (k1t_sssp_table.cu): per-root shortest-path tables of the whole graph, [N][N] each, rows built on demand
+// kernel 1t (k1t_sssp_table.cu): per-root shortest-path tables, [N][N] each, row r over the subgraph induced by r's k-hop
+// ball (the tables hold one hop at a time), rows built on demand
 struct SsspTables {
-  double* D;       // fl-distance from the root (bit pattern of the Dijkstra fixpoint), +inf where unreachable
+  double* D;       // fl-distance from the root (bit pattern of the Dijkstra fixpoint), +inf outside the ball / unreachable
   double* Q;       // python-order path sum x -> root (100 where unreachable)
   int32_t* P;      // tree parent (graph id), -1 for the root / unreachable
   double* PW;      // weight kappa + 1 of the tree edge (x, P[x])
@@ -380,7 +381,7 @@ struct SsspTables {
   int* count;
 };
 void launch_sssp_build(const GraphView& g, const Params& p, const int32_t* targets, int64_t E, const SsspTables& tb,
-                       const float* gminw, double* pw_scratch, int grid, cudaStream_t st);
+                       const uint32_t* ball_cache, const float* gminw, double* pw_scratch, int grid, cudaStream_t st);
 size_t sssp_build_smem(int N);
 void launch_filtration_table(const GraphView& g, const Params& p, const ChunkView& c, const VicinityScratch& vs,
                              const SsspTables& tb, int t0, int cnt, int block, int64_t n_max, cudaStream_t st);
@@ -449,7 +450,7 @@ void launch_peer_wait(const unsigned int* flag, unsigned int target, cudaStream_
 int64_t launch_count();
 void count_launch();
 int vicinity_grid(int device, const GraphView& g, const Params& p, size_t* bitmap_words, bool* use_smem);
-// expand (once) the balls of the targets' endpoints that are not cached yet
+// expand (once) the balls of the targets' endpoints that are not cached yet (targets == nullptr: of every node)
 void launch_ball_cache(const GraphView& g, const Params& p, const int32_t* targets, int64_t E, const VicinityScratch& vs,
                        cudaStream_t st);
 
