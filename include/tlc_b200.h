@@ -70,8 +70,8 @@ extern "C" {
 
 #define TLC_F_NO_TABLE 8192u /* graph-row route: never use the per-root shortest-path tables (kernel 1t), always run kernel 1b's
                                 Dijkstra per target.  Default: on graphs of <= 16384 nodes whose tables fit the budget
-                                (28 N^2 bytes <= TLC_SSSP_CACHE_GB, default 8) the distances, tree parents and path sums of a
-                                root over the WHOLE graph are computed once; a vicinity vertex whose tree branch stays inside
+                                (28 N^2 bytes <= TLC_SSSP_CACHE_GB GiB, default 8) the distances, tree parents and path sums of
+                                a root over its k-hop ball are computed once; a vicinity vertex whose tree branch stays inside
                                 the vicinity takes its values from the table, the others are relaxed over their own rows.
                                 Same results bit for bit */
 

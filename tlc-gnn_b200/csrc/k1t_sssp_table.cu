@@ -30,7 +30,7 @@
 // kernel 1b).
 //
 // Rows read per target drop from 2 x D_S (every row of the vicinity, once per root) to the rows of the invalid
-// vertices; the table rows of u and v (D, Q, W, P: 28 N bytes each) are streamed instead.
+// vertices; the table rows of u and v (D, P, {Q, W}: 28 N bytes each) are gathered through the vertex list instead.
 #include <cstdlib>
 
 #include <cstdio>
@@ -73,8 +73,9 @@ struct BuildShared {
 // hold the call's hop): an edge is relaxed only into a member of the ball.  Vertices outside it keep D = +inf, P = -1,
 // Q = NO_PATH_DIST, W = 0 (kernel 1t never reads them: S is a subset of the ball).  gminw, the smallest weight of a
 // vertex's WHOLE-graph row, stays a valid settling margin: the edges of G'_r into x are a subset of those of G, so their
-// smallest weight is at least gminw[x].
-__global__ void __launch_bounds__(1024) sssp_build_kernel(GraphView g, SsspTables tb, const uint32_t* __restrict__ ball_cache,
+// smallest weight is at least gminw[x].  The host launches one CTA per SM (pw_scratch has one row per CTA); saying so in
+// the launch bounds lets ptxas use up to 64 registers instead of spilling at 32.
+__global__ void __launch_bounds__(1024, 1) sssp_build_kernel(GraphView g, SsspTables tb, const uint32_t* __restrict__ ball_cache,
                                                           const float* __restrict__ gminw, double* __restrict__ pw_scratch,
                                                           int plain) {
   extern __shared__ __align__(16) unsigned long long bsm[];
@@ -161,26 +162,26 @@ __global__ void __launch_bounds__(1024) sssp_build_kernel(GraphView g, SsspTable
     }
     __threadfence_block();
     __syncthreads();
-    // outputs: D (bit pattern as double), P, Q (python-order path sum; 100 where the root does not reach x: riccidist2dgm.py:31-32)
+    // outputs: D (bit pattern as double), P, {Q (python-order path sum; 100 where the root does not reach x:
+    // riccidist2dgm.py:31-32), W}
     double* Drow = tb.D + (size_t)root * N;
-    double* Qrow = tb.Q + (size_t)root * N;
     int32_t* Prow = tb.P + (size_t)root * N;
-    double* Wrow = tb.PW + (size_t)root * N;
+    double2* QWrow = tb.QW + (size_t)root * N;
     for (int x = tid; x < N; x += nt) {
       const unsigned long long dxb = dist[x];
-      Drow[x] = __longlong_as_double((long long)dxb);
-      Prow[x] = par[x];
-      Wrow[x] = par[x] >= 0 ? pw[x] : 0.0;
+      const int32_t px = par[x];
       double res;
       if (x == root) res = 0.0;
-      else if (dxb == INF_BITS || par[x] < 0) res = NO_PATH_DIST;
+      else if (dxb == INF_BITS || px < 0) res = NO_PATH_DIST;
       else {
         PySum ps{0.0, 0.0, 0};
         int y = x, guard = 0;
         while (y != root && guard++ <= N) { pysum_add(ps, pw[y], plain != 0); y = par[y]; }
         res = pysum_get(ps, plain != 0);
       }
-      Qrow[x] = res;
+      Drow[x] = __longlong_as_double((long long)dxb);
+      Prow[x] = px;
+      QWrow[x] = make_double2(res, px >= 0 ? pw[x] : 0.0);
     }
     __syncthreads();
     if (tid == 0) { __threadfence(); tb.state[root] = 2; }
@@ -291,26 +292,38 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
       const int root = r == 0 ? lu : lv;
       const int32_t groot = r == 0 ? u : v;
       const double* __restrict__ Drow = tb.D + (size_t)groot * N;
-      const double* __restrict__ Qrow = tb.Q + (size_t)groot * N;
-      const double* __restrict__ Wrow = tb.PW + (size_t)groot * N;
       const int32_t* __restrict__ Prow = tb.P + (size_t)groot * N;
+      const double2* __restrict__ QWrow = tb.QW + (size_t)groot * N;
       double* out = r == 0 ? d1 : d2;
       int32_t* hnt = r == 0 ? hint0 : hint;
       if (tid == 0) { sh.ninv = 0; sh.nextra = 0; sh.dinv = 0; sh.nia = 0; }
       // ---- 1. classes: the branch of x stays in S <=> its table parent is in S and is valid itself ----
-      for (int x = tid; x < n; x += nt) {
-        const int32_t gx = vert[x];
-        uint8_t cl;
-        uint16_t pl = 0xffff;
-        if (x == root) cl = VALID;
-        else {
-          const int32_t gp = Prow[gx];
-          pl = gp >= 0 ? lid[gp] : (uint16_t)0xffff;
-          cl = pl == 0xffff ? INVALID : UNKNOWN;
+      // Four vertices per thread with their loads in flight together: first their graph ids, then their D and P, only
+      // then the local ids of the parents (each vertex alone would be two dependent global round trips)
+      for (int x0 = tid; x0 < n; x0 += 4 * nt) {
+        int32_t gx4[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) { const int x = x0 + k * nt; gx4[k] = x < n ? vert[x] : -1; }
+        double d4[4];
+        int32_t p4[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) { d4[k] = gx4[k] >= 0 ? Drow[gx4[k]] : 0.0; p4[k] = gx4[k] >= 0 ? Prow[gx4[k]] : -1; }
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+          const int x = x0 + k * nt;
+          if (x >= n) continue;
+          uint8_t cl;
+          uint16_t pl = 0xffff;
+          if (x == root) cl = VALID;
+          else {
+            const int32_t gp = p4[k];
+            pl = gp >= 0 ? lid[gp] : (uint16_t)0xffff;
+            cl = pl == 0xffff ? INVALID : UNKNOWN;
+          }
+          cls[x] = cl; parl[x] = pl;
+          dist[x] = (unsigned long long)__double_as_longlong(d4[k]);
+          if (r == 0) { hint[x] = -1; hint0[x] = -1; }
         }
-        cls[x] = cl; parl[x] = pl;
-        dist[x] = (unsigned long long)__double_as_longlong(Drow[gx]);
-        if (r == 0) { hint[x] = -1; hint0[x] = -1; }
       }
       __syncthreads();
       TPROF(1);
@@ -554,45 +567,59 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
       }
       __syncthreads();
       TPROF(7);
-      // parents of the invalid vertices; from here on the distances are not needed any more and every vertex's 8-byte slot
-      // holds the weight of its tree edge instead (the table's for a valid vertex), so that the walks of step 4 stay in
-      // shared memory
-      for (int x = tid; x < n; x += nt) {
-        unsigned long long wb = 0;
-        if (x != root) {
-          if (cls[x] == VALID) wb = (unsigned long long)__double_as_longlong(Wrow[vert[x]]);
-          else {
+      // ---- 4. parents and outputs (phase "parents"): from here on the distances are not needed any more and every
+      // vertex's 8-byte slot holds the weight of its tree edge instead, so that the walks below stay in shared memory.
+      // A valid vertex's {Q, W} (one 16-byte load) gives that weight and its output, the table's path sum; four valid
+      // vertices per thread with their loads in flight together.  An
+      // invalid vertex takes its parent from the tree rule's row position, or is unreachable (nx.NetworkXNoPath:
+      // disconnected vicinity, status 3 later).  The root and the unreachable vertices keep the hint -1.
+      for (int x0 = tid; x0 < n; x0 += 4 * nt) {
+        int32_t gx4[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+          const int x = x0 + k * nt;
+          gx4[k] = x < n && x != root && cls[x] == VALID ? vert[x] : -1;
+        }
+        double2 e4[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) e4[k] = gx4[k] >= 0 ? QWrow[gx4[k]] : make_double2(0.0, 0.0);
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+          const int x = x0 + k * nt;
+          if (x >= n) continue;
+          unsigned long long wb = 0;
+          if (x == root) out[x] = 0.0;
+          else if (gx4[k] >= 0) {
+            wb = (unsigned long long)__double_as_longlong(e4[k].y);
+            out[x] = e4[k].x;
+            hnt[x] = (int32_t)parl[x];
+          } else {
             const int pos = bpos[x];
             if (dist[x] != INF_BITS && pos != 0x7fffffff) {
               const uint4 rc = __ldg(g.rec + pos);
-              parl[x] = lid[rc.x];
+              const uint16_t pl = lid[rc.x];
+              parl[x] = pl;
+              hnt[x] = (int32_t)pl;
               wb = ((unsigned long long)rc.w << 32) | rc.z;
-            } else cls[x] = UNREACH;
+            } else { cls[x] = UNREACH; out[x] = NO_PATH_DIST; }
           }
+          dist[x] = wb;
         }
-        dist[x] = wb;
       }
       __syncthreads();
       TPROF(8);
-      // ---- 4. path sums: the table's for valid vertices, a walk in python order for the others   :30,35 ----
-      for (int x = tid; x < n; x += nt) {
-        double res;
-        const uint8_t cl = cls[x];
-        if (x == root) res = 0.0;
-        else if (cl == VALID) { res = Qrow[vert[x]]; hnt[x] = (int32_t)parl[x]; }
-        else if (cl == UNREACH) res = NO_PATH_DIST;  // nx.NetworkXNoPath (disconnected vicinity; status 3 later)
-        else {
-          hnt[x] = (int32_t)parl[x];
-          PySum ps{0.0, 0.0, 0};
-          int y = x, guard = 0;
-          while (y != root && guard++ <= n) {
-            const int py = (int)parl[y];
-            pysum_add(ps, __longlong_as_double((long long)dist[y]), plain);
-            y = py;
-          }
-          res = pysum_get(ps, plain);
+      // ---- 5. path sums of the invalid vertices (phase "path_sums"): a walk in python order   :30,35 ----
+      for (int i = tid; i < ninv; i += nt) {
+        const int x = inv[i] & 0xffff;  // (without the rescan flag)
+        if (cls[x] == UNREACH) continue;
+        PySum ps{0.0, 0.0, 0};
+        int y = x, guard = 0;
+        while (y != root && guard++ <= n) {
+          const int py = (int)parl[y];
+          pysum_add(ps, __longlong_as_double((long long)dist[y]), plain);
+          y = py;
         }
-        out[x] = res;
+        out[x] = pysum_get(ps, plain);
       }
       __syncthreads();
       TPROF(9);
@@ -603,7 +630,7 @@ __global__ void __launch_bounds__(1024) filtration_table_kernel(Params p, ChunkV
   }
   __syncthreads();
 
-  // ---- 5. descriptors + normalisation   riccidist2dgm.py:47-56 ; data_utils_NC.py:52-54 ----
+  // ---- 6. descriptors + normalisation   riccidist2dgm.py:47-56 ; data_utils_NC.py:52-54 ----
   double mx = -1.0, sm = -1.0;
   for (int x = tid; x < n; x += nt) {
     const double a = d1[x], b = d2[x];

@@ -191,7 +191,7 @@ struct tlc_graph {
   // kernel 1t: per-root shortest-path tables over the roots' k-hop balls (valid for sssp_plain and sssp_hop), scratch of
   // the build kernel
   SsspTables sssp{};  // views of the sssp_* buffers, null until they exist
-  DevBuf sssp_D, sssp_Q, sssp_P, sssp_PW, sssp_state, sssp_list, sssp_count, sssp_pw;
+  DevBuf sssp_D, sssp_P, sssp_QW, sssp_state, sssp_list, sssp_count, sssp_pw;
   int sssp_plain = -1, sssp_hop = -1;
   bool sssp_tried = false, sssp_all = false;
   double sssp_build_ms = 0;   // device time of the (one-time) table build
@@ -316,10 +316,10 @@ static int prepare_call(tlc_graph* g, const Params& p, int64_t E) {
   return rc ? rc : ensure_vicinity_scratch(g, p);
 }
 
-// kernel 1t's tables: four [N][N] arrays, allocated once when the graph is small enough (N <= 16384: the build kernel keeps a
-// root's whole distance / parent vector and ball in shared memory) and 28 N^2 bytes fit TLC_SSSP_CACHE_GB (default 8, 0
-// disables).  Their rows depend on the summation rule (path sums) and the hop (the ball each row is restricted to): a call
-// with another of either marks every row for rebuilding.
+// kernel 1t's tables: three [N][N] arrays (D, P, {Q, W}), allocated once when the graph is small enough (N <= 16384: the
+// build kernel keeps a root's whole distance / parent vector and ball in shared memory) and 28 N^2 bytes fit
+// TLC_SSSP_CACHE_GB (default 8, 0 disables).  Their rows depend on the summation rule (path sums) and the hop (the ball
+// each row is restricted to): a call with another of either marks every row for rebuilding.
 static int ensure_sssp_tables(tlc_graph* g, const Params& p) {
   const int plain = (p.flags & TLC_F_SUM_PLAIN) ? 1 : 0;
   if (!g->sssp_tried) {
@@ -327,21 +327,20 @@ static int ensure_sssp_tables(tlc_graph* g, const Params& p) {
     const char* env = getenv("TLC_SSSP_CACHE_GB");
     const double gb = env ? atof(env) : 8.0;
     const size_t N = (size_t)g->gv.N;
-    const size_t need = N * N * 28;
+    const size_t need = N * N * (8 + 4 + 16);
     size_t free_b = 0, total_b = 0;
     cudaMemGetInfo(&free_b, &total_b);
     if (gb > 0 && N <= 16384 && (double)need <= gb * (double)(1ull << 30) && need <= free_b / 3 &&
         sssp_build_smem((int)N) <= 227 * 1024) {
       CK(g->sssp_D.reserve(N * N * 8));
-      CK(g->sssp_Q.reserve(N * N * 8));
       CK(g->sssp_P.reserve(N * N * 4));
-      CK(g->sssp_PW.reserve(N * N * 8));
+      CK(g->sssp_QW.reserve(N * N * 16));
       CK(g->sssp_state.reserve(N * 4));
       CK(g->sssp_list.reserve(N * 4));
       CK(g->sssp_count.reserve(64));
       CK(g->sssp_pw.reserve((size_t)g->sm_count * N * 8));
       CK(cudaMemset(g->sssp_state.p, 0, N * 4));
-      g->sssp = SsspTables{g->sssp_D.as<double>(), g->sssp_Q.as<double>(), g->sssp_P.as<int32_t>(), g->sssp_PW.as<double>(),
+      g->sssp = SsspTables{g->sssp_D.as<double>(), g->sssp_P.as<int32_t>(), g->sssp_QW.as<double2>(),
                            g->sssp_state.as<int32_t>(), g->sssp_list.as<int32_t>(), g->sssp_count.as<int>()};
       g->sssp_plain = plain;
       g->sssp_hop = p.hop;

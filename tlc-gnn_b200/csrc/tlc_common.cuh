@@ -369,13 +369,15 @@ void launch_gather_rows(const double* table, int64_t rows, int r2, const int64_t
 void launch_scatter_rows(const double* src_pi, const float* src_pi32, const uint8_t* src_st, const int64_t* idx, int64_t k,
                          int r2, double* dst_pi, float* dst_pi32, uint8_t* dst_st, int sm_count, cudaStream_t st);
 
-// kernel 1t (k1t_sssp_table.cu): per-root shortest-path tables, [N][N] each, row r over the subgraph induced by r's k-hop
-// ball (the tables hold one hop at a time), rows built on demand
+// kernel 1t (k1t_sssp_table.cu): per-root shortest-path tables, [N][N] entries, row r over the subgraph induced by r's
+// k-hop ball (the tables hold one hop at a time), rows built on demand.  Three arrays, split by the pass that reads them:
+// kernel 1t's class pass reads D and P of every vertex of S (dense rows: neighbouring vertices of S share their sectors),
+// only the valid vertices' output pass reads Q and W, together in one 16-byte load.
 struct SsspTables {
   double* D;       // fl-distance from the root (bit pattern of the Dijkstra fixpoint), +inf outside the ball / unreachable
-  double* Q;       // python-order path sum x -> root (100 where unreachable)
   int32_t* P;      // tree parent (graph id), -1 for the root / unreachable
-  double* PW;      // weight kappa + 1 of the tree edge (x, P[x])
+  double2* QW;     // {Q, W}: python-order path sum x -> root (100 where unreachable), weight kappa + 1 of the tree edge
+                   // (x, P[x]) (0 without one)
   int32_t* state;  // [N] 0 row not built, 1 claimed in this call, 2 built
   int32_t* list;   // [N] roots to build in this call
   int* count;
