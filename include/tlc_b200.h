@@ -236,6 +236,28 @@ int tlc_union_find(int device, int32_t n, int32_t m, const double *fval, const i
  * dgm[K][2] (birth, death) float64 -> out[res*res] float64, runs kernel 4 on `device`. */
 int tlc_pimg_transform(int device, const double *dgm, int64_t K, int32_t resolution, double *out);
 
+/* The same imager for a batch of D diagrams already on the device, and its gradient: the batched form of
+ * Knowledge_Distillation/pimg.py `transform` (:354-414), the torch copy of PersistenceImager(resolution).transform(dgm,
+ * skew=True) (PersistenceImager.pyx:352-388) that PDGNN differentiates through.  Diagram t is the points
+ * poff[t] .. poff[t+1] of birth[] / death[]; poff[0] need not be 0 (a slice of a larger diagram array works).  poff must be
+ * non-decreasing with every entry in [0, len(birth)]: a decreasing segment is treated as empty, and no point outside
+ * [poff[t], poff[t+1]) is read for diagram t.  kind (may be NULL: every point counts) selects the points whose kind k is
+ * < 32 with bit k of img_mask set.  out[D][res*res] float64, birth-major; an empty diagram gives a zero row.
+ * Gradient: with p = death - birth, w = clamp(p, 0, 1), A_i(b) = Phi(x_{i+1} - b) - Phi(x_i - b), B_j(p) likewise and
+ * G = grad_out[t]:  grad_death = A^T G (w' B + w B'),  grad_birth = w A'^T G B - grad_death,  where w' = 1 on the CLOSED
+ * interval 0 <= p <= 1 and 0 elsewhere (torch.clamp's own backward), so zero-persistence points get a nonzero
+ * grad_death.  Points whose kind is masked out get 0.  grad_birth[k] / grad_death[k] are written for every k in
+ * [poff[0], poff[D]) and nowhere else; either pointer may be NULL (not computed).
+ * Every pointer is a DEVICE pointer on `device`; `stream` is a cudaStream_t (NULL: default stream).  Neither call
+ * allocates or synchronises: both only enqueue.  Results are bit-identical from call to call and independent of the
+ * rest of the batch (a batch split over sliced poff gives the same rows).  TLC_E_INVALID: D outside [0, 2^31),
+ * resolution outside 1..16, or a NULL required pointer with D > 0. */
+int tlc_pimg_batch_dev(int device, int64_t D, const int64_t *dev_poff, const double *dev_birth, const double *dev_death,
+                       const uint8_t *dev_kind, uint32_t img_mask, int32_t resolution, double *dev_out, void *stream);
+int tlc_pimg_batch_grad_dev(int device, int64_t D, const int64_t *dev_poff, const double *dev_birth,
+                            const double *dev_death, const uint8_t *dev_kind, uint32_t img_mask, int32_t resolution,
+                            const double *dev_grad_out, double *dev_grad_birth, double *dev_grad_death, void *stream);
+
 /* Hand-off of the cached image table to the decoder (baselines/TLCGNN.py:35-53): the table float64[rows][r2]
  * (the .npy cache layout, loaddatas.py:62-64,102) stays resident in HBM; out[i][:] = (float) table[row(i)][:],
  * row(i) = dev_index ? dev_index[i] : start + i -- what `torch.Tensor(PI[...]).cuda()` yields per decode call

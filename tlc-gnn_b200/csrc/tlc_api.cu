@@ -1821,12 +1821,54 @@ int tlc_pimg_transform(int device, const double* dgm, int64_t K, int32_t resolut
   if (!out || (K > 0 && !dgm) || resolution < 1 || resolution > 16) return fail(TLC_E_INVALID, "bad arguments");
   int rc = select_device(device);
   if (rc) return rc;
-  DevBuf b_dgm, b_out;
-  CK(b_dgm.reserve(std::max<size_t>((size_t)K * 16, 16)));
+  // one diagram of the batch imager: poff {0, K}, then the births and the deaths, uploaded in one copy
+  std::vector<double> h(2 * (size_t)K + 2);
+  const int64_t off[2] = {0, K};
+  std::memcpy(h.data(), off, sizeof off);
+  for (int64_t k = 0; k < K; k++) { h[2 + k] = dgm[2 * k]; h[2 + K + k] = dgm[2 * k + 1]; }
+  DevBuf b_in, b_out;
+  CK(b_in.reserve(h.size() * 8));
   CK(b_out.reserve((size_t)resolution * resolution * 8));
-  if (K) CK(cudaMemcpy(b_dgm.p, dgm, (size_t)K * 16, cudaMemcpyHostToDevice));
-  launch_pimg_single(b_dgm.as<double>(), K, resolution, b_out.as<double>(), nullptr);
+  CK(cudaMemcpy(b_in.p, h.data(), h.size() * 8, cudaMemcpyHostToDevice));
+  const double* d_in = b_in.as<double>();
+  launch_pimg_batch(b_in.as<int64_t>(), d_in + 2, d_in + 2 + K, nullptr, 0u, resolution, 1, b_out.as<double>(), nullptr);
   CK(cudaMemcpy(out, b_out.p, (size_t)resolution * resolution * 8, cudaMemcpyDeviceToHost));
+  CK(cudaGetLastError());
+  return TLC_OK;
+}
+
+// the checks both batch imager calls make before any CUDA call
+static int check_pimg_batch(int64_t D, const int64_t* poff, const double* birth, const double* death, int32_t resolution) {
+  if (D < 0 || D >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "D must be in [0, 2^31)");
+  if (resolution < 1 || resolution > 16) return fail(TLC_E_INVALID, "resolution must be in 1..16");
+  if (D > 0 && !poff) return fail(TLC_E_INVALID, "dev_poff is NULL");
+  if (D > 0 && !birth) return fail(TLC_E_INVALID, "dev_birth is NULL");
+  if (D > 0 && !death) return fail(TLC_E_INVALID, "dev_death is NULL");
+  return TLC_OK;
+}
+
+int tlc_pimg_batch_dev(int device, int64_t D, const int64_t* dev_poff, const double* dev_birth, const double* dev_death,
+                       const uint8_t* dev_kind, uint32_t img_mask, int32_t resolution, double* dev_out, void* stream) {
+  int rc = check_pimg_batch(D, dev_poff, dev_birth, dev_death, resolution);
+  if (rc) return rc;
+  if (D > 0 && !dev_out) return fail(TLC_E_INVALID, "dev_out is NULL");
+  if (D == 0) return TLC_OK;
+  if ((rc = select_device(device))) return rc;
+  launch_pimg_batch(dev_poff, dev_birth, dev_death, dev_kind, img_mask, resolution, D, dev_out, (cudaStream_t)stream);
+  CK(cudaGetLastError());
+  return TLC_OK;
+}
+
+int tlc_pimg_batch_grad_dev(int device, int64_t D, const int64_t* dev_poff, const double* dev_birth,
+                            const double* dev_death, const uint8_t* dev_kind, uint32_t img_mask, int32_t resolution,
+                            const double* dev_grad_out, double* dev_grad_birth, double* dev_grad_death, void* stream) {
+  int rc = check_pimg_batch(D, dev_poff, dev_birth, dev_death, resolution);
+  if (rc) return rc;
+  if (D > 0 && !dev_grad_out) return fail(TLC_E_INVALID, "dev_grad_out is NULL");
+  if (D == 0 || (!dev_grad_birth && !dev_grad_death)) return TLC_OK;
+  if ((rc = select_device(device))) return rc;
+  launch_pimg_batch_grad(dev_poff, dev_birth, dev_death, dev_kind, img_mask, resolution, D, dev_grad_out,
+                         dev_grad_birth, dev_grad_death, (cudaStream_t)stream);
   CK(cudaGetLastError());
   return TLC_OK;
 }

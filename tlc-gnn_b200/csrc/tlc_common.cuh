@@ -303,6 +303,9 @@ __device__ __forceinline__ int uf_find(PT* p, int x) {
 __device__ __forceinline__ double norm_cdf(double x) {  // erfc(-x / sqrt(2)) / 2   :60
   return erfc(-x / 1.4142135623730951) * 0.5;
 }
+__device__ __forceinline__ double norm_pdf(double x) {  // d norm_cdf / dx = exp(-x^2 / 2) / sqrt(2 pi)
+  return exp(-0.5 * x * x) * 0.3989422804014327;
+}
 __device__ __forceinline__ double ramp_weight(double pers) {  // linear_ramp defaults  :22-28
   return pers < 0.0 ? 0.0 : (pers > 1.0 ? 1.0 : pers);
 }
@@ -361,7 +364,11 @@ void launch_sweep(const Params& p, const ChunkView& c, int t0, int cnt, int64_t 
 void launch_loops(const Params& p, const ChunkView& c, int block, int smem_ints, int64_t n_max, cudaStream_t st);
 void launch_pimg(const Params& p, const ChunkView& c, double* out_pi, float* out_pi_f32, uint8_t* out_status,
                  int block, cudaStream_t st);
-void launch_pimg_single(const double* dgm, int64_t K, int res, double* out, cudaStream_t st);
+void launch_pimg_batch(const int64_t* poff, const double* birth, const double* death, const uint8_t* kind,
+                       uint32_t img_mask, int res, int64_t D, double* out, cudaStream_t st);
+void launch_pimg_batch_grad(const int64_t* poff, const double* birth, const double* death, const uint8_t* kind,
+                            uint32_t img_mask, int res, int64_t D, const double* grad_out, double* grad_birth,
+                            double* grad_death, cudaStream_t st);
 
 void launch_gather_rows(const double* table, int64_t rows, int r2, const int64_t* index, int64_t start, int64_t n,
                         float* out, int* bad, int sm_count, cudaStream_t st);

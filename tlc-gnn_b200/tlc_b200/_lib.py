@@ -30,7 +30,7 @@ EXPORTS = ["tlc_graph_create", "tlc_graph_destroy", "tlc_vicinity_pi", "tlc_vici
            "tlc_last_counts", "tlc_last_direct", "tlc_pi_gather", "tlc_last_small", "tlc_small_diagrams",
            "tlc_table_create", "tlc_table_attach", "tlc_vicinity_pi_exchange", "tlc_last_table",
            "tlc_ollivier_ricci", "tlc_graph_set_hks_time", "tlc_table_build_ms", "tlc_vicinity_diagrams",
-           "tlc_vicinity_diagrams_dev"]
+           "tlc_vicinity_diagrams_dev", "tlc_pimg_batch_dev", "tlc_pimg_batch_grad_dev"]
 
 
 class Params(C.Structure):
@@ -92,6 +92,10 @@ def lib():
     L.tlc_union_find.argtypes = [C.c_int, i32, i32, vp, vp, vp, u32] + [vp] * 11
     L.tlc_pimg_transform.restype = C.c_int
     L.tlc_pimg_transform.argtypes = [C.c_int, vp, i64, i32, vp]
+    L.tlc_pimg_batch_dev.restype = C.c_int
+    L.tlc_pimg_batch_dev.argtypes = [C.c_int, i64, vp, vp, vp, vp, u32, i32, vp, vp]
+    L.tlc_pimg_batch_grad_dev.restype = C.c_int
+    L.tlc_pimg_batch_grad_dev.argtypes = [C.c_int, i64, vp, vp, vp, vp, u32, i32, vp, vp, vp, vp]
     L.tlc_last_error.restype = C.c_char_p
     L.tlc_version.restype = C.c_char_p
     L.tlc_launch_count.restype = i64

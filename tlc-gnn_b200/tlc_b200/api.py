@@ -14,17 +14,21 @@ from . import _lib as L
 _CUDA_STREAM_LEGACY = 0x1  # cudaStreamLegacy (driver_types.h): an explicit handle of the legacy default stream
 
 
-def _dev_ptr(t, dtype_name, shape, device_index, what):
-    """data pointer of a torch CUDA tensor that crosses the C-ABI: dtype, shape, contiguity and device are checked here,
-    because the library can only see a raw address."""
-    if t is None:
-        return None
+def _check_layout(t, dtype_name, shape, what):
     if str(t.dtype) != "torch." + dtype_name:
         raise TypeError("%s must be %s, got %s" % (what, dtype_name, t.dtype))
     if tuple(t.shape) != tuple(shape):
         raise ValueError("%s must have shape %s, got %s" % (what, tuple(shape), tuple(t.shape)))
     if not t.is_contiguous():
         raise ValueError("%s must be contiguous" % what)
+
+
+def _dev_ptr(t, dtype_name, shape, device_index, what):
+    """data pointer of a torch CUDA tensor that crosses the C-ABI: dtype, shape, contiguity and device are checked here,
+    because the library can only see a raw address."""
+    if t is None:
+        return None
+    _check_layout(t, dtype_name, shape, what)
     if t.device.type != "cuda" or (t.device.index is not None and t.device.index != device_index):
         raise ValueError("%s must live on cuda:%d, got %s" % (what, device_index, t.device))
     return t.data_ptr()
@@ -354,6 +358,83 @@ def pimg_transform(dgm, resolution=5, device=0):
     out = np.zeros(resolution * resolution)
     L.check(L.lib().tlc_pimg_transform(device, d.ctypes.data, d.shape[0], resolution, out.ctypes.data))
     return out.reshape(resolution, resolution)
+
+
+_ImagesFn = None
+
+
+def _images_fn():
+    """the torch.autograd.Function over tlc_pimg_batch_dev / tlc_pimg_batch_grad_dev (built on first use: torch is only
+    imported by the calls that take tensors)"""
+    global _ImagesFn
+    if _ImagesFn is not None:
+        return _ImagesFn
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    def stream(dev):
+        return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+
+    class PersistenceImages(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, poff, birth, death, kind, img_mask, resolution):
+            dev = birth.device
+            D, r2 = poff.shape[0] - 1, resolution * resolution
+            out = torch.empty((D, r2), dtype=torch.float64, device=dev)
+            L.check(L.lib().tlc_pimg_batch_dev(dev.index, D, poff.data_ptr(), birth.data_ptr(), death.data_ptr(),
+                                               kind.data_ptr() if kind is not None else None, img_mask, resolution,
+                                               out.data_ptr(), stream(dev)))
+            ctx.save_for_backward(poff, birth, death, kind)
+            ctx.img_mask, ctx.resolution = img_mask, resolution
+            return out
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_out):
+            poff, birth, death, kind = ctx.saved_tensors
+            dev = birth.device
+            D, r2 = poff.shape[0] - 1, ctx.resolution * ctx.resolution
+            g = grad_out.contiguous()
+            _dev_ptr(g, "float64", (D, r2), dev.index, "grad_out")
+            # the kernel writes [poff[0], poff[D]); the points outside every segment keep their zero
+            gb = torch.zeros_like(birth) if ctx.needs_input_grad[1] else None
+            gd = torch.zeros_like(death) if ctx.needs_input_grad[2] else None
+            L.check(L.lib().tlc_pimg_batch_grad_dev(
+                dev.index, D, poff.data_ptr(), birth.data_ptr(), death.data_ptr(),
+                kind.data_ptr() if kind is not None else None, ctx.img_mask, ctx.resolution, g.data_ptr(),
+                gb.data_ptr() if gb is not None else None, gd.data_ptr() if gd is not None else None, stream(dev)))
+            return None, gb, gd, None, None, None
+
+    _ImagesFn = PersistenceImages
+    return _ImagesFn
+
+
+def persistence_images(poff, birth, death, kind=None, img_mask=None, resolution=5):
+    """persistence images of a batch of diagrams on the GPU, differentiable in birth and death: the batched
+    Knowledge_Distillation/pimg.py `transform` (PersistenceImager(resolution).transform, PersistenceImager.pyx:352-388).
+    poff int64[D+1], birth / death float64[P], kind uint8[P] (optional): CUDA tensors on one device; diagram t is the
+    points poff[t] .. poff[t+1], which must be non-decreasing and lie in [0, P].  img_mask: bit k set -> points of kind k
+    count (None: every kind; needs `kind`).  Returns float64[D, res^2], birth-major.  Forward and backward run on the
+    current stream of the device.  The output of VicinityGraph.vicinity_diagrams_dev plugs in directly:
+    persistence_images(d["poff"], d["birth"], d["death"], d["kind"], mask)."""
+    if img_mask is not None and kind is None:
+        raise ValueError("img_mask selects kinds: pass kind as well")
+    resolution = int(resolution)
+    if not 1 <= resolution <= 16:
+        raise ValueError("resolution must be in 1..16, got %d" % resolution)
+    if getattr(birth, "dim", lambda: 0)() != 1 or getattr(poff, "dim", lambda: 0)() != 1 or poff.shape[0] < 1:
+        raise ValueError("poff must be 1-D with D + 1 >= 1 entries and birth 1-D")
+    dev = birth.device.index if birth.device.type == "cuda" else 0
+    P = int(birth.shape[0])
+    specs = [(poff, "int64", (int(poff.shape[0]),), "poff"), (birth, "float64", (P,), "birth"),
+             (death, "float64", (P,), "death"), (kind, "uint8", (P,), "kind")]
+    for t, dtype_name, shape, what in specs:  # the layout of all of them first: a bad one is named wherever they live
+        if t is not None:
+            _check_layout(t, dtype_name, shape, what)
+    for spec in specs:
+        _dev_ptr(spec[0], spec[1], spec[2], dev, spec[3])
+    mask = 0xFFFFFFFF if img_mask is None else int(img_mask) & 0xFFFFFFFF
+    return _images_fn().apply(poff, birth, death, kind, mask, resolution)
 
 
 def launch_count():
