@@ -258,6 +258,47 @@ int tlc_pimg_batch_grad_dev(int device, int64_t D, const int64_t *dev_poff, cons
                             const double *dev_death, const uint8_t *dev_kind, uint32_t img_mask, int32_t resolution,
                             const double *dev_grad_out, double *dev_grad_birth, double *dev_grad_death, void *stream);
 
+/* Exact Wasserstein distances between D pairs of diagrams already on the device, and their gradient: the batched form
+ * of Knowledge_Distillation/wasserstein.py (gudhi's wasserstein_distance(X, Y, order=q, internal_p=p,
+ * enable_autodiff=True), :93, :198), PDGNN's training loss.  Pair t is X = points poff_x[t] .. poff_x[t+1] of
+ * birth_x / death_x and Y = points poff_y[t] .. poff_y[t+1] of birth_y / death_y, in the batch imager's ragged layout:
+ * poff[0] need not be 0, poff must be non-decreasing with entries in [0, Px] (resp. Py), a decreasing segment is empty.
+ * kind_x / kind_y (either may be NULL: every point of that side counts) select the points whose kind k is < 32 with
+ * bit k of kind_mask set.  q = order >= 1 finite, p = internal_p >= 1 or +inf.
+ *   ground cost ||x - y||_p; distance of a point to the diagonal delta(x) = |d - b| * 2^(1/p - 1) (|d - b| / 2 for
+ *   p = inf; the absolute value keeps PD_down and [max,min] points, which lie below the diagonal, at their distance);
+ *   dist[t] = (sum c)^(1/q) minimised over partial matchings, c = ||x - y||_p^q for a matched pair and delta^q for a
+ *   point matched to the diagonal -- gudhi's (n+1) x (m+1) transport problem, solved exactly (a shortest-augmenting-path
+ *   assignment solver per pair, every loop bounded by the pair's point count).  Points with b == d go to the diagonal.
+ *   A pair with a selected non-finite coordinate is not solved: dist NaN, all its matches -1.
+ *   match_x[k] = the global index into the Y arrays of the point matched to X point k, -1 the diagonal, -2 a point
+ *   masked out; match_y likewise from the Y side.  Both are written for every k in [poff[0], poff[D]) and nowhere else;
+ *   either may be NULL.  A pair's matching and distance are the same bits from call to call and whatever the batch.
+ * Workspace: dev_workspace of at least tlc_wasserstein_workspace_bytes(D, Px, Py) bytes (64 (Px + Py); Px, Py: the
+ * lengths of the X and Y point arrays), 16-byte aligned; pair t uses the slice at 64 ((poff_x[t] - poff_x[0]) +
+ * (poff_y[t] - poff_y[0])).  Neither call allocates or synchronises: both only enqueue on `stream`.
+ * Gradient: with S = dist^q and G = grad_out[t], a point's gradient is G (1/q) S^(1/q - 1) dc/d(b, d) of the term it
+ * appears in (the forward's matching), with torch.linalg.vector_norm's conventions: 0 for a zero-length difference,
+ * sgn(0) = 0, ties of the p = inf max share the gradient evenly, S = 0 gives 0; NaN for the selected points of an
+ * unsolved pair; 0 for masked points.  Written for every k in [poff[0], poff[D]) and nowhere else; any of the four
+ * gradient pointers may be NULL.
+ * TLC_E_INVALID: D outside [0, 2^31), Px or Py outside [0, 2^56), q < 1 or not finite, p < 1 or NaN, a NULL required
+ * pointer with D > 0, or a workspace smaller than the query's size.  D = 0 with NULL pointers returns 0. */
+int tlc_wasserstein_workspace_bytes(int64_t D, int64_t Px, int64_t Py, uint64_t *bytes);
+int tlc_wasserstein_batch_dev(int device, int64_t D, int64_t Px, int64_t Py, const int64_t *dev_poff_x,
+                              const double *dev_birth_x, const double *dev_death_x, const uint8_t *dev_kind_x,
+                              const int64_t *dev_poff_y, const double *dev_birth_y, const double *dev_death_y,
+                              const uint8_t *dev_kind_y, uint32_t kind_mask, double order, double internal_p,
+                              void *dev_workspace, uint64_t workspace_bytes, double *dev_dist, int64_t *dev_match_x,
+                              int64_t *dev_match_y, void *stream);
+int tlc_wasserstein_batch_grad_dev(int device, int64_t D, const int64_t *dev_poff_x, const double *dev_birth_x,
+                                   const double *dev_death_x, const uint8_t *dev_kind_x, const int64_t *dev_poff_y,
+                                   const double *dev_birth_y, const double *dev_death_y, const uint8_t *dev_kind_y,
+                                   uint32_t kind_mask, double order, double internal_p, const double *dev_dist,
+                                   const int64_t *dev_match_x, const int64_t *dev_match_y, const double *dev_grad_out,
+                                   double *dev_grad_birth_x, double *dev_grad_death_x, double *dev_grad_birth_y,
+                                   double *dev_grad_death_y, void *stream);
+
 /* Hand-off of the cached image table to the decoder (baselines/TLCGNN.py:35-53): the table float64[rows][r2]
  * (the .npy cache layout, loaddatas.py:62-64,102) stays resident in HBM; out[i][:] = (float) table[row(i)][:],
  * row(i) = dev_index ? dev_index[i] : start + i -- what `torch.Tensor(PI[...]).cuda()` yields per decode call

@@ -1873,6 +1873,77 @@ int tlc_pimg_batch_grad_dev(int device, int64_t D, const int64_t* dev_poff, cons
   return TLC_OK;
 }
 
+int tlc_wasserstein_workspace_bytes(int64_t D, int64_t Px, int64_t Py, uint64_t* bytes) {
+  if (D < 0 || D >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "D must be in [0, 2^31)");
+  if (Px < 0 || Py < 0 || Px >= ((int64_t)1 << 56) || Py >= ((int64_t)1 << 56))
+    return fail(TLC_E_INVALID, "Px and Py must be in [0, 2^56)");
+  if (!bytes) return fail(TLC_E_INVALID, "bytes is NULL");
+  *bytes = wasserstein_workspace_bytes(D, Px, Py);
+  return TLC_OK;
+}
+
+// the checks both Wasserstein calls make before any CUDA call
+static int check_wasserstein(int64_t D, const int64_t* poff_x, const double* bx, const double* dx, const int64_t* poff_y,
+                             const double* by, const double* dy, double order, double internal_p) {
+  if (D < 0 || D >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "D must be in [0, 2^31)");
+  if (!(order >= 1.0) || std::isinf(order)) return fail(TLC_E_INVALID, "order must be finite and >= 1");
+  if (!(internal_p >= 1.0)) return fail(TLC_E_INVALID, "internal_p must be >= 1 or +inf");
+  const char* names[6] = {"dev_poff_x", "dev_birth_x", "dev_death_x", "dev_poff_y", "dev_birth_y", "dev_death_y"};
+  const void* ptrs[6] = {poff_x, bx, dx, poff_y, by, dy};
+  for (int k = 0; k < 6; k++)
+    if (D > 0 && !ptrs[k]) return fail(TLC_E_INVALID, std::string(names[k]) + " is NULL");
+  return TLC_OK;
+}
+
+int tlc_wasserstein_batch_dev(int device, int64_t D, int64_t Px, int64_t Py, const int64_t* dev_poff_x,
+                              const double* dev_birth_x, const double* dev_death_x, const uint8_t* dev_kind_x,
+                              const int64_t* dev_poff_y, const double* dev_birth_y, const double* dev_death_y,
+                              const uint8_t* dev_kind_y, uint32_t kind_mask, double order, double internal_p,
+                              void* dev_workspace, uint64_t workspace_bytes, double* dev_dist, int64_t* dev_match_x,
+                              int64_t* dev_match_y, void* stream) {
+  int rc = check_wasserstein(D, dev_poff_x, dev_birth_x, dev_death_x, dev_poff_y, dev_birth_y, dev_death_y, order,
+                             internal_p);
+  if (rc) return rc;
+  uint64_t need = 0;
+  if ((rc = tlc_wasserstein_workspace_bytes(D, Px, Py, &need))) return rc;
+  if (workspace_bytes < need)
+    return fail(TLC_E_INVALID, "workspace_bytes is " + std::to_string(workspace_bytes) + ", the call needs " +
+                                   std::to_string(need));
+  if (D > 0 && need > 0 && !dev_workspace) return fail(TLC_E_INVALID, "dev_workspace is NULL");
+  if (D > 0 && !dev_dist) return fail(TLC_E_INVALID, "dev_dist is NULL");
+  if (D == 0) return TLC_OK;
+  if ((rc = select_device(device))) return rc;
+  launch_wasserstein(dev_poff_x, dev_birth_x, dev_death_x, dev_kind_x, dev_poff_y, dev_birth_y, dev_death_y,
+                     dev_kind_y, kind_mask, order, internal_p, D, dev_workspace, workspace_bytes, dev_dist,
+                     dev_match_x, dev_match_y, (cudaStream_t)stream);
+  CK(cudaGetLastError());
+  return TLC_OK;
+}
+
+int tlc_wasserstein_batch_grad_dev(int device, int64_t D, const int64_t* dev_poff_x, const double* dev_birth_x,
+                                   const double* dev_death_x, const uint8_t* dev_kind_x, const int64_t* dev_poff_y,
+                                   const double* dev_birth_y, const double* dev_death_y, const uint8_t* dev_kind_y,
+                                   uint32_t kind_mask, double order, double internal_p, const double* dev_dist,
+                                   const int64_t* dev_match_x, const int64_t* dev_match_y, const double* dev_grad_out,
+                                   double* dev_grad_birth_x, double* dev_grad_death_x, double* dev_grad_birth_y,
+                                   double* dev_grad_death_y, void* stream) {
+  int rc = check_wasserstein(D, dev_poff_x, dev_birth_x, dev_death_x, dev_poff_y, dev_birth_y, dev_death_y, order,
+                             internal_p);
+  if (rc) return rc;
+  if (D > 0 && !dev_dist) return fail(TLC_E_INVALID, "dev_dist is NULL");
+  if (D > 0 && !dev_match_x) return fail(TLC_E_INVALID, "dev_match_x is NULL");
+  if (D > 0 && !dev_match_y) return fail(TLC_E_INVALID, "dev_match_y is NULL");
+  if (D > 0 && !dev_grad_out) return fail(TLC_E_INVALID, "dev_grad_out is NULL");
+  if (D == 0 || (!dev_grad_birth_x && !dev_grad_death_x && !dev_grad_birth_y && !dev_grad_death_y)) return TLC_OK;
+  if ((rc = select_device(device))) return rc;
+  launch_wasserstein_grad(dev_poff_x, dev_birth_x, dev_death_x, dev_kind_x, dev_poff_y, dev_birth_y, dev_death_y,
+                          dev_kind_y, kind_mask, order, internal_p, D, dev_dist, dev_match_x, dev_match_y,
+                          dev_grad_out, dev_grad_birth_x, dev_grad_death_x, dev_grad_birth_y, dev_grad_death_y,
+                          (cudaStream_t)stream);
+  CK(cudaGetLastError());
+  return TLC_OK;
+}
+
 int tlc_pi_gather(int device, const double* dev_table, int64_t rows, int32_t r2, const int64_t* dev_index, int64_t start,
                   int64_t n, float* dev_out_f32, void* stream) {
   if (rows < 0 || r2 < 1 || n < 0 || (n > 0 && (!dev_table || !dev_out_f32))) return fail(TLC_E_INVALID, "bad arguments");

@@ -369,6 +369,16 @@ void launch_pimg_batch(const int64_t* poff, const double* birth, const double* d
 void launch_pimg_batch_grad(const int64_t* poff, const double* birth, const double* death, const uint8_t* kind,
                             uint32_t img_mask, int res, int64_t D, const double* grad_out, double* grad_birth,
                             double* grad_death, cudaStream_t st);
+uint64_t wasserstein_workspace_bytes(int64_t D, int64_t Px, int64_t Py);
+void launch_wasserstein(const int64_t* poff_x, const double* bx, const double* dx, const uint8_t* kx,
+                        const int64_t* poff_y, const double* by, const double* dy, const uint8_t* ky, uint32_t mask,
+                        double order, double internal_p, int64_t D, void* ws, uint64_t ws_bytes, double* dist,
+                        int64_t* match_x, int64_t* match_y, cudaStream_t st);
+void launch_wasserstein_grad(const int64_t* poff_x, const double* bx, const double* dx, const uint8_t* kx,
+                             const int64_t* poff_y, const double* by, const double* dy, const uint8_t* ky,
+                             uint32_t mask, double order, double internal_p, int64_t D, const double* dist,
+                             const int64_t* match_x, const int64_t* match_y, const double* grad_out, double* gbx,
+                             double* gdx, double* gby, double* gdy, cudaStream_t st);
 
 void launch_gather_rows(const double* table, int64_t rows, int r2, const int64_t* index, int64_t start, int64_t n,
                         float* out, int* bad, int sm_count, cudaStream_t st);

@@ -30,7 +30,8 @@ EXPORTS = ["tlc_graph_create", "tlc_graph_destroy", "tlc_vicinity_pi", "tlc_vici
            "tlc_last_counts", "tlc_last_direct", "tlc_pi_gather", "tlc_last_small", "tlc_small_diagrams",
            "tlc_table_create", "tlc_table_attach", "tlc_vicinity_pi_exchange", "tlc_last_table",
            "tlc_ollivier_ricci", "tlc_graph_set_hks_time", "tlc_table_build_ms", "tlc_vicinity_diagrams",
-           "tlc_vicinity_diagrams_dev", "tlc_pimg_batch_dev", "tlc_pimg_batch_grad_dev"]
+           "tlc_vicinity_diagrams_dev", "tlc_pimg_batch_dev", "tlc_pimg_batch_grad_dev",
+           "tlc_wasserstein_workspace_bytes", "tlc_wasserstein_batch_dev", "tlc_wasserstein_batch_grad_dev"]
 
 
 class Params(C.Structure):
@@ -96,6 +97,13 @@ def lib():
     L.tlc_pimg_batch_dev.argtypes = [C.c_int, i64, vp, vp, vp, vp, u32, i32, vp, vp]
     L.tlc_pimg_batch_grad_dev.restype = C.c_int
     L.tlc_pimg_batch_grad_dev.argtypes = [C.c_int, i64, vp, vp, vp, vp, u32, i32, vp, vp, vp, vp]
+    L.tlc_wasserstein_workspace_bytes.restype = C.c_int
+    L.tlc_wasserstein_workspace_bytes.argtypes = [i64, i64, i64, C.POINTER(u64)]
+    L.tlc_wasserstein_batch_dev.restype = C.c_int
+    L.tlc_wasserstein_batch_dev.argtypes = ([C.c_int, i64, i64, i64] + [vp] * 8 + [u32, C.c_double, C.c_double, vp, u64]
+                                            + [vp] * 4)
+    L.tlc_wasserstein_batch_grad_dev.restype = C.c_int
+    L.tlc_wasserstein_batch_grad_dev.argtypes = [C.c_int, i64] + [vp] * 8 + [u32, C.c_double, C.c_double] + [vp] * 9
     L.tlc_last_error.restype = C.c_char_p
     L.tlc_version.restype = C.c_char_p
     L.tlc_launch_count.restype = i64

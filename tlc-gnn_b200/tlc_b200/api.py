@@ -5,6 +5,7 @@ curvature uploaded once (graph2pi.__init__, riccidist2dgm.py:216-226), then one 
 of targets (get_pimg_for_all_edges, :362-370).
 """
 import ctypes as C
+import math
 
 import numpy as np
 
@@ -435,6 +436,110 @@ def persistence_images(poff, birth, death, kind=None, img_mask=None, resolution=
         _dev_ptr(spec[0], spec[1], spec[2], dev, spec[3])
     mask = 0xFFFFFFFF if img_mask is None else int(img_mask) & 0xFFFFFFFF
     return _images_fn().apply(poff, birth, death, kind, mask, resolution)
+
+
+_WassersteinFn = None
+
+
+def _wasserstein_fn():
+    """the torch.autograd.Function over tlc_wasserstein_batch_dev / tlc_wasserstein_batch_grad_dev (built on first use)"""
+    global _WassersteinFn
+    if _WassersteinFn is not None:
+        return _WassersteinFn
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    def stream(dev):
+        return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+
+    def ptr(t):
+        return t.data_ptr() if t is not None else None
+
+    class WassersteinDistances(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, poff_x, birth_x, death_x, kind_x, poff_y, birth_y, death_y, kind_y, mask, order, internal_p):
+            dev = birth_x.device
+            D, Px, Py = poff_x.shape[0] - 1, birth_x.shape[0], birth_y.shape[0]
+            nbytes = C.c_uint64()
+            L.check(L.lib().tlc_wasserstein_workspace_bytes(D, Px, Py, C.byref(nbytes)))
+            ws = torch.empty(max(nbytes.value, 1), dtype=torch.uint8, device=dev)
+            dist = torch.empty(D, dtype=torch.float64, device=dev)
+            # the kernel writes [poff[0], poff[D]); the points outside every segment keep -2 (not in any pair)
+            mx = torch.full((Px,), -2, dtype=torch.int64, device=dev)
+            my = torch.full((Py,), -2, dtype=torch.int64, device=dev)
+            L.check(L.lib().tlc_wasserstein_batch_dev(
+                dev.index, D, Px, Py, ptr(poff_x), ptr(birth_x), ptr(death_x), ptr(kind_x), ptr(poff_y), ptr(birth_y),
+                ptr(death_y), ptr(kind_y), mask, order, internal_p, ws.data_ptr(), nbytes.value, dist.data_ptr(),
+                mx.data_ptr(), my.data_ptr(), stream(dev)))
+            ctx.save_for_backward(poff_x, birth_x, death_x, kind_x, poff_y, birth_y, death_y, kind_y, dist, mx, my)
+            ctx.mask, ctx.order, ctx.internal_p = mask, order, internal_p
+            ctx.mark_non_differentiable(mx, my)
+            return dist, mx, my
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, grad_dist, _gmx, _gmy):
+            poff_x, birth_x, death_x, kind_x, poff_y, birth_y, death_y, kind_y, dist, mx, my = ctx.saved_tensors
+            dev = birth_x.device
+            D = poff_x.shape[0] - 1
+            g = grad_dist.contiguous()
+            _dev_ptr(g, "float64", (D,), dev.index, "grad_out")
+            # the kernel writes [poff[0], poff[D]); the points outside every segment keep their zero
+            need = ctx.needs_input_grad
+            grads = [torch.zeros_like(t) if need[k] else None
+                     for k, t in ((1, birth_x), (2, death_x), (5, birth_y), (6, death_y))]
+            L.check(L.lib().tlc_wasserstein_batch_grad_dev(
+                dev.index, D, ptr(poff_x), ptr(birth_x), ptr(death_x), ptr(kind_x), ptr(poff_y), ptr(birth_y),
+                ptr(death_y), ptr(kind_y), ctx.mask, ctx.order, ctx.internal_p, dist.data_ptr(), mx.data_ptr(),
+                my.data_ptr(), g.data_ptr(), *[ptr(t) for t in grads], stream(dev)))
+            gbx, gdx, gby, gdy = grads
+            return None, gbx, gdx, None, None, gby, gdy, None, None, None, None
+
+    _WassersteinFn = WassersteinDistances
+    return _WassersteinFn
+
+
+def wasserstein_distances(poff_x, birth_x, death_x, poff_y, birth_y, death_y, kind_x=None, kind_y=None, kind_mask=None,
+                          order=1.0, internal_p=math.inf, return_matching=False):
+    """exact Wasserstein distances between D pairs of diagrams on the GPU, differentiable in the four point tensors:
+    the batched gudhi wasserstein_distance(X, Y, order, internal_p, enable_autodiff=True) of
+    Knowledge_Distillation/wasserstein.py.  Pair t is X = points poff_x[t] .. poff_x[t+1] of birth_x / death_x and
+    Y = points poff_y[t] .. poff_y[t+1] of birth_y / death_y (poff int64[D+1], non-decreasing; birth / death float64;
+    kind uint8, optional): CUDA tensors on one device.  kind_mask: bit k set -> points of kind k count (None: every
+    kind); a side without `kind` counts all its points.  The defaults are gudhi's (order 1, internal_p inf).
+    Returns float64[D], and with return_matching=True also (match_x int64[len(birth_x)], match_y int64[len(birth_y)]):
+    the global index of the matched point of the other side, -1 the diagonal, -2 masked out or in no pair.  A pair with
+    a non-finite selected point gives NaN.  Runs on the current stream of the device.  The output of
+    VicinityGraph.vicinity_diagrams_dev plugs in directly: wasserstein_distances(a["poff"], a["birth"], a["death"],
+    b["poff"], b["birth"], b["death"], a["kind"], b["kind"], mask)."""
+    if kind_mask is not None and kind_x is None and kind_y is None:
+        raise ValueError("kind_mask selects kinds: pass kind_x or kind_y as well")
+    order, internal_p = float(order), float(internal_p)
+    if not (order >= 1.0 and math.isfinite(order)):
+        raise ValueError("order must be finite and >= 1, got %r" % order)
+    if not internal_p >= 1.0:
+        raise ValueError("internal_p must be >= 1 or inf, got %r" % internal_p)
+    for po, b, what in ((poff_x, birth_x, "x"), (poff_y, birth_y, "y")):
+        if getattr(b, "dim", lambda: 0)() != 1 or getattr(po, "dim", lambda: 0)() != 1 or po.shape[0] < 1:
+            raise ValueError("poff_%s must be 1-D with D + 1 >= 1 entries and birth_%s 1-D" % (what, what))
+    if poff_x.shape[0] != poff_y.shape[0]:
+        raise ValueError("poff_x and poff_y must have the same length, got %d and %d"
+                         % (poff_x.shape[0], poff_y.shape[0]))
+    dev = birth_x.device.index if birth_x.device.type == "cuda" else 0
+    Px, Py, D1 = int(birth_x.shape[0]), int(birth_y.shape[0]), int(poff_x.shape[0])
+    specs = [(poff_x, "int64", (D1,), "poff_x"), (birth_x, "float64", (Px,), "birth_x"),
+             (death_x, "float64", (Px,), "death_x"), (kind_x, "uint8", (Px,), "kind_x"),
+             (poff_y, "int64", (D1,), "poff_y"), (birth_y, "float64", (Py,), "birth_y"),
+             (death_y, "float64", (Py,), "death_y"), (kind_y, "uint8", (Py,), "kind_y")]
+    for t, dtype_name, shape, what in specs:  # the layout of all of them first: a bad one is named wherever they live
+        if t is not None:
+            _check_layout(t, dtype_name, shape, what)
+    for spec in specs:
+        _dev_ptr(spec[0], spec[1], spec[2], dev, spec[3])
+    mask = 0xFFFFFFFF if kind_mask is None else int(kind_mask) & 0xFFFFFFFF
+    dist, mx, my = _wasserstein_fn().apply(poff_x, birth_x, death_x, kind_x, poff_y, birth_y, death_y, kind_y, mask,
+                                           order, internal_p)
+    return (dist, (mx, my)) if return_matching else dist
 
 
 def launch_count():
