@@ -358,6 +358,9 @@ int64_t tlc_last_direct(tlc_graph *g);
  * those targets of a BATCH call the induced edges are not counted (no kernel reads all their rows any more): they are
  * missing from tlc_last_counts' sum m and from the 16 m term of tlc_last_algorithmic_bytes; tlc_vicinity_sizes counts them. */
 int64_t tlc_last_table(tlc_graph *g);
+/* of those, the targets kernel 1t ran with both roots u and v in the same passes (their two states fit its shared memory;
+ * TLC_TABLE_ONE_ROOT=1 runs every target one root at a time) */
+int64_t tlc_last_table_two_root(tlc_graph *g);
 /* device ms the one-time build of the shortest-path tables took (all N roots, at the first graph-row call that uses them) */
 double tlc_table_build_ms(tlc_graph *g);
 /* kernel S in the last call: out[0..2] = device ms of the class A (warp per target, n <= 64) / class B (128-thread CTA,

@@ -86,6 +86,7 @@ struct CallStats {
   int64_t live = 0, sum_n = 0, sum_m = 0;                    // targets with status <= TRIVIAL, their vertices / edges
   int64_t handed_back = 0, general = 0, rowcheck = 0, blocks = 0;  // sweep counters of kernels 2v / 3v
   int64_t direct = 0, table = 0;  // targets that took the graph-row route, those of them filtered from the tables
+  int64_t two_root = 0;            // ... and those kernel 1t ran with both roots in the same passes
   double bytes = 0;               // compulsory bytes (SURVEY.md 8d)
   double small_ms[3] = {0, 0, 0};
   int64_t small_rows[4] = {0, 0, 0, 0};  // rows finished by kernel S's class A / B / C, rows handed to the staged pipeline
@@ -95,6 +96,7 @@ struct CallStats {
     for (int i = 0; i < 4; i++) small_rows[i] += o.small_rows[i];
     chunks += o.chunks; live += o.live; sum_n += o.sum_n; sum_m += o.sum_m; handed_back += o.handed_back;
     general += o.general; rowcheck += o.rowcheck; blocks += o.blocks; direct += o.direct; table += o.table;
+    two_root += o.two_root;
     bytes += o.bytes;
     return *this;
   }
@@ -460,7 +462,7 @@ struct StageTimer {
 // kernels whose shared-memory footprint follows the vicinity size are launched per SUB-RANGE of the chunk's
 // (size-sorted) targets, each with the capacity of its own largest vicinity: smaller vicinities get more
 // resident CTAs per SM
-struct SubRange { int t0, cnt; int64_t n_max; };
+struct SubRange { int t0, cnt; int64_t n_min, n_max; };
 
 // launch(range, stream) for every sub-range; sub-ranges 1 - 3 run on the side streams, forked from / joined to `st`
 template <typename F_>
@@ -497,7 +499,7 @@ static int64_t run_stages(tlc_graph* g, const Params& p, const ChunkView& c, int
   else {
     for_subranges(g, subs, st, [&](const SubRange& r, cudaStream_t s) {
       if (c.dbm && takes_table(g, use_table, r)) {
-        launch_filtration_table(g->gv, p, c, vs, g->sssp, r.t0, r.cnt, block, r.n_max, s);
+        launch_filtration_table(g->gv, p, c, vs, g->sssp, g->d_n.as<int32_t>(), r.t0, r.cnt, block, r.n_min, r.n_max, s);
         from_table += r.cnt;
       } else if (c.dbm) launch_filtration_direct(g->gv, p, c, vs, g->gminw.as<float>(), r.t0, r.cnt, block, r.n_max, s);
       else launch_filtration(p, c, r.t0, r.cnt, block, r.n_max, s);
@@ -722,9 +724,9 @@ static std::vector<SubRange> split_subranges(const tlc_graph* g, const std::vect
     int64_t b = first;
     while (b < T && smem_class(h_n[order[pos + b]]) == cls) b++;
     if (b > first) {
-      int64_t nm = 0;
-      for (int64_t k = first; k < b; k++) nm = std::max<int64_t>(nm, h_n[order[pos + k]]);
-      subs.push_back(SubRange{(int)first, (int)(b - first), nm});
+      int64_t n0 = INT64_MAX, nm = 0;
+      for (int64_t k = first; k < b; k++) { n0 = std::min<int64_t>(n0, h_n[order[pos + k]]); nm = std::max<int64_t>(nm, h_n[order[pos + k]]); }
+      subs.push_back(SubRange{(int)first, (int)(b - first), n0, nm});
       first = b;
     }
   }
@@ -732,9 +734,9 @@ static std::vector<SubRange> split_subranges(const tlc_graph* g, const std::vect
   for (int gi = 0; gi < groups && rest > 0; gi++) {
     const int64_t a = first + rest * gi / groups, b = first + rest * (gi + 1) / groups;
     if (b <= a) continue;
-    int64_t nm = 0;
-    for (int64_t k = a; k < b; k++) nm = std::max<int64_t>(nm, h_n[order[pos + k]]);
-    subs.push_back(SubRange{(int)a, (int)(b - a), nm});
+    int64_t n0 = INT64_MAX, nm = 0;
+    for (int64_t k = a; k < b; k++) { n0 = std::min<int64_t>(n0, h_n[order[pos + k]]); nm = std::max<int64_t>(nm, h_n[order[pos + k]]); }
+    subs.push_back(SubRange{(int)a, (int)(b - a), n0, nm});
   }
   return subs;
 }
@@ -853,8 +855,8 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
   const Params p = to_params(up);
   const int r2 = p.resolution * p.resolution;
   cudaStream_t st = g->stream;
-  int* fb_counters = g->work_counter.as<int>() + 4;
-  CK(cudaMemsetAsync(fb_counters, 0, 4 * sizeof(int), st));
+  int* fb_counters = g->work_counter.as<int>() + 4;  // handed back, general, rowcheck, blocks | kernel 1t two-root targets
+  CK(cudaMemsetAsync(fb_counters, 0, 5 * sizeof(int), st));
   if (cnt_compute) *cnt_compute = 0;
   if (E == 0) return TLC_OK;
   const bool bad_desc = p.descriptor < 0 || p.descriptor > 2;
@@ -947,17 +949,18 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
       c.count_m = light ? 1 : 0;
       // tm: counted by kernel 1b (batch call) or known from the full counting pass (detail call)
       if (!light) CK(cudaMemcpyAsync((void*)c.tm, h.tm + pos, (size_t)k.T * 4, cudaMemcpyHostToDevice, st));
-      int fb0 = 0, fb1 = 0;
+      int fb0 = 0, fb1[5] = {0, 0, 0, 0, 0};
       CK(cudaMemcpyAsync(&fb0, fb_counters, sizeof(int), cudaMemcpyDeviceToHost, st));
       s.table += run_stages(g, p, c, k.n_max, k.m_max, subs, d_pi, d_pi32, d_status, want_pairs, tm, use_table);
-      CK(cudaMemcpyAsync(&fb1, fb_counters, sizeof(int), cudaMemcpyDeviceToHost, st));
+      CK(cudaMemcpyAsync(fb1, fb_counters, 5 * sizeof(int), cudaMemcpyDeviceToHost, st));
       if (light) CK(cudaMemcpyAsync(h.tm + pos, c.tm, (size_t)k.T * 4, cudaMemcpyDeviceToHost, st));
       CK(cudaStreamSynchronize(st));
       s.direct += k.T;
+      s.two_root = fb1[4];  // (a running count over the call's chunks; a redo of handed-back targets below resets the counter)
       if (light) {  // the exact edge counts: totals and the 16 m term of the compulsory bytes (SURVEY.md 8d)
         for (int64_t t = 0; t < k.T; t++) { s.sum_m += h.tm[pos + t]; s.bytes += 16.0 * (double)h.tm[pos + t]; }
       }
-      if (fb1 != fb0) {
+      if (fb1[0] != fb0) {
         // kernel 3v handed targets back: their edge-sorted sweep needs the adjacency
         if (light) {  // no adjacency space was reserved: those targets are redone on the materialised route below
           fbv.resize((size_t)k.T);
@@ -2069,6 +2072,7 @@ int tlc_last_counts(tlc_graph* g, int64_t* out5) {  // out5: 8 slots
 int64_t tlc_last_direct(tlc_graph* g) { return g ? g->last.direct : 0; }
 
 int64_t tlc_last_table(tlc_graph* g) { return g ? g->last.table : 0; }
+int64_t tlc_last_table_two_root(tlc_graph* g) { return g ? g->last.two_root : 0; }
 double tlc_table_build_ms(tlc_graph* g) { return g ? g->sssp_build_ms : 0.0; }
 
 int tlc_last_small(tlc_graph* g, double* out7) {

@@ -403,7 +403,8 @@ void launch_sssp_build(const GraphView& g, const Params& p, const int32_t* targe
                        const uint32_t* ball_cache, const float* gminw, double* pw_scratch, int grid, cudaStream_t st);
 size_t sssp_build_smem(int N);
 void launch_filtration_table(const GraphView& g, const Params& p, const ChunkView& c, const VicinityScratch& vs,
-                             const SsspTables& tb, int t0, int cnt, int block, int64_t n_max, cudaStream_t st);
+                             const SsspTables& tb, const int32_t* n_of, int t0, int cnt, int block, int64_t n_min,
+                             int64_t n_max, cudaStream_t st);
 size_t filtration_table_smem(int N, int64_t n_max);
 
 // kernel 6 (k6_ricci.cu): Ollivier-Ricci curvature (Sinkhorn) of a host-prepared edge list

@@ -29,6 +29,7 @@ EXPORTS = ["tlc_graph_create", "tlc_graph_destroy", "tlc_vicinity_pi", "tlc_vici
            "tlc_launch_count", "tlc_last_stage_ms", "tlc_last_algorithmic_bytes", "tlc_graph_set_stream",
            "tlc_last_counts", "tlc_last_direct", "tlc_pi_gather", "tlc_last_small", "tlc_small_diagrams",
            "tlc_table_create", "tlc_table_attach", "tlc_vicinity_pi_exchange", "tlc_last_table",
+           "tlc_last_table_two_root",
            "tlc_ollivier_ricci", "tlc_graph_set_hks_time", "tlc_table_build_ms", "tlc_vicinity_diagrams",
            "tlc_vicinity_diagrams_dev", "tlc_pimg_batch_dev", "tlc_pimg_batch_grad_dev",
            "tlc_wasserstein_workspace_bytes", "tlc_wasserstein_batch_dev", "tlc_wasserstein_batch_grad_dev"]
@@ -127,6 +128,8 @@ def lib():
     L.tlc_table_build_ms.argtypes = [vp]
     L.tlc_last_table.restype = i64
     L.tlc_last_table.argtypes = [vp]
+    L.tlc_last_table_two_root.restype = i64
+    L.tlc_last_table_two_root.argtypes = [vp]
     L.tlc_last_small.restype = C.c_int
     L.tlc_last_small.argtypes = [vp, vp]
     L.tlc_table_create.restype = C.c_int

@@ -323,7 +323,8 @@ class VicinityGraph:
         L.lib().tlc_last_counts(self._h, out.ctypes.data)
         return dict(live=int(out[0]), sum_n=int(out[1]), sum_m=int(out[2]), chunks=int(out[3]), handed_back=int(out[4]),
                     blocks_general=int(out[5]), blocks_rowcheck=int(out[6]), blocks=int(out[7]),
-                    graph_row_route=int(L.lib().tlc_last_direct(self._h)), table_route=int(L.lib().tlc_last_table(self._h)))
+                    graph_row_route=int(L.lib().tlc_last_direct(self._h)), table_route=int(L.lib().tlc_last_table(self._h)),
+                    table_two_root=int(L.lib().tlc_last_table_two_root(self._h)))
 
     def last_algorithmic_bytes(self):
         tot = C.c_double(0)
