@@ -105,6 +105,7 @@ extern "C" {
 #define TLC_ST_UNKNOWN_NODE 5   /* id not in the graph / isolated          riccidist2dgm.py:353 */
 #define TLC_ST_BAD_DESCRIPTOR 6 /* attribute missing                       accelerated_PD.py:13 */
 #define TLC_ST_NO_TREE_EDGES 7  /* single vertex + extended flag           accelerated_PD.py:122 */
+#define TLC_ST_NONFINITE 8      /* tlc_graph_batch_diagrams_dev: a NaN or +-inf filtration value, no pairs */
 
 typedef struct {
   int32_t hop;        /* BFS depth limit                                   riccidist2dgm.py:310 */
@@ -298,6 +299,53 @@ int tlc_wasserstein_batch_grad_dev(int device, int64_t D, const int64_t *dev_pof
                                    const int64_t *dev_match_x, const int64_t *dev_match_y, const double *dev_grad_out,
                                    double *dev_grad_birth_x, double *dev_grad_death_x, double *dev_grad_birth_y,
                                    double *dev_grad_death_y, void *stream);
+
+/* Persistence diagrams of a batch of CALLER-SUPPLIED graphs under a filtration already on the device, and their gradient
+ * in that filtration: Union_find + Accelerate_PD (accelerated_PD.py:26,115) per graph, batched -- the step in front of the
+ * batch imager and the Wasserstein distances for a learnable filtration (Knowledge_Distillation/ConvCurv_GIN.py,
+ * mode='filtration') or whole-graph persistence over a dataloader batch (Knowledge_Distillation/data_utils_GC.py:95-167).
+ * The structure is uploaded and checked once; only f changes from call to call.
+ *
+ * tlc_graph_batch_create: D graphs; graph t owns vertices noff[t] .. noff[t+1] and edges eoff[t] .. eoff[t+1] of (ea, eb),
+ * batch-global vertex ids (PyG's Batch.ptr / edge_index numbering).  HOST pointers, copied to `device`.  The order of a
+ * graph's edges is the tie-break of the sweeps, as in tlc_union_find.  TLC_E_INVALID, with a message naming the first
+ * offending graph or edge, unless noff and eoff start at 0 and are monotone, noff[D] < 2^31 and eoff[D] < 2^31, every edge
+ * of graph t has both endpoints in [noff[t], noff[t+1]), no edge is a self-loop and no undirected edge appears twice (in
+ * either direction).  Vertices without edges are allowed.  The call plans every graph's route from its size and allocates
+ * every device buffer the diagram and gradient calls need: those never allocate.
+ * tlc_graph_batch_pair_bound: N + M + D (N = noff[D], M = eoff[D]), the pair capacity every diagram call needs.
+ *
+ * tlc_graph_batch_diagrams_dev: dev_f float64[N].  Graph t's pairs and status are exactly what the pipeline gives for a
+ * node-mode vicinity equal to that graph with filtration values f[noff[t] .. noff[t+1]] (tlc_vicinity_diagrams): PD_up,
+ * [min,max], PD_down, [max,min], then PD_one with TLC_F_EXTENDED, birth / death values bit for bit, bv / dv batch-global
+ * vertex ids; status DISCONNECTED (no pairs: no per-component diagrams), NO_TREE_EDGES (one vertex with TLC_F_EXTENDED,
+ * keeps its 0-dim pairs), EMPTY (n = 0), and TLC_ST_NONFINITE (no pairs) for a graph with a NaN or +-inf value.  No
+ * normalisation: the caller scales f (in torch, where it stays differentiable).  out->cap >= the pair bound; out->poff
+ * [D+1] receives the exclusive offsets of the graphs' segments, compact and in graph order (poff[D] = pairs in total);
+ * out->npairs [D] (may be NULL); kind / bv / dv / birth / death [cap] (each may be NULL: not written; entries past poff[D]
+ * are left as they are); dev_status uint8[D] (may be NULL).  flags: TLC_F_EXTENDED, TLC_F_KEEP_ZERO, TLC_F_ASC_ONLY (not
+ * with TLC_F_EXTENDED), TLC_F_NO_SMALL (every graph through the staged kernels 2 + 3 + 3b instead of kernel 9's fused
+ * per-graph teams, which take graphs of <= 1024 vertices / <= 4096 edges; same results bit for bit).  Output is bit-identical
+ * from call to call and independent of the rest of the batch.
+ *
+ * tlc_graph_batch_grad_dev: for the diagrams d of the last diagram call (device pointers: poff, bv, dv required),
+ * grad_f[v] = sum over points k in [poff[0], poff[D]) with bv[k] == v of grad_birth[k] + with dv[k] == v of grad_death[k],
+ * added in increasing k, birth term before death term, starting from 0.0; every v in [0, N) is written.  grad_birth /
+ * grad_death may each be NULL (treated as 0).  Bit-reproducible: no floating-point atomics.
+ *
+ * All pointers of the two calls are DEVICE pointers on the batch's device; `stream` is a cudaStream_t (NULL: the legacy
+ * default stream).  Both only enqueue (no synchronisation, no allocation, no host<->device traffic) and share the batch's
+ * scratch: calls on one batch must be ordered (one stream, or the caller's events).  TLC_E_INVALID (bad flags, a NULL
+ * required pointer) and TLC_E_CAPACITY (cap < bound) are returned before any CUDA call. */
+typedef struct tlc_graph_batch tlc_graph_batch;
+int tlc_graph_batch_create(int device, int64_t D, const int64_t *noff, const int64_t *eoff, const int32_t *ea,
+                           const int32_t *eb, tlc_graph_batch **out);
+int tlc_graph_batch_destroy(tlc_graph_batch *b);
+int tlc_graph_batch_pair_bound(const tlc_graph_batch *b, int64_t *bound);
+int tlc_graph_batch_diagrams_dev(tlc_graph_batch *b, const double *dev_f, uint32_t flags, tlc_diagrams *out,
+                                 uint8_t *dev_status, void *stream);
+int tlc_graph_batch_grad_dev(tlc_graph_batch *b, const tlc_diagrams *d, const double *dev_grad_birth,
+                             const double *dev_grad_death, double *dev_grad_f, void *stream);
 
 /* Hand-off of the cached image table to the decoder (baselines/TLCGNN.py:35-53): the table float64[rows][r2]
  * (the .npy cache layout, loaddatas.py:62-64,102) stays resident in HBM; out[i][:] = (float) table[row(i)][:],

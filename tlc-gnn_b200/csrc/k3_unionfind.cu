@@ -200,7 +200,7 @@ __global__ void union_find_kernel(Params p, ChunkView c, int smem_ints, int buil
 void launch_union_find(const Params& p, const ChunkView& c, int block, int smem_ints, int build_lists, int sweep_mask,
                        int fb_only, cudaStream_t st) {
   const size_t bytes = (size_t)smem_ints * 4;
-  if (bytes > 48 * 1024)
+  if (bytes + sizeof(UfShared) > 48 * 1024)  // (the static part counts towards the 48 KiB a launch gets without opting in)
     cudaFuncSetAttribute((const void*)union_find_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
   union_find_kernel<<<c.T, block, bytes, st>>>(p, c, smem_ints, build_lists, sweep_mask, fb_only);
   count_launch();

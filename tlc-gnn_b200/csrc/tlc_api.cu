@@ -2098,3 +2098,245 @@ int tlc_last_algorithmic_bytes(tlc_graph* g, double* bytes_total, double* bytes_
 }
 
 }  // extern "C"
+
+// ---- graph batches: persistence diagrams of caller-supplied graphs (tlc_graph_batch_*, kernel 9) ----
+// Each graph takes one route, fixed at creation from its size: kernel 9's fused teams (classes A / B / C) or the staged
+// kernels 2 + 3 (+ 3b) over a ChunkView whose segments are the graphs'.  Two such views are carved from one arena: `large`
+// (the graphs no class takes, the default route) and `all` (every graph: TLC_F_NO_SMALL).  Their per-graph tables (graph
+// id, vertex / edge offsets) are uploaded once; the fill kernel writes the per-call state.
+struct StagedView {
+  ChunkView c{};
+  int64_t n_max = 0, m_max = 0;
+};
+
+struct tlc_graph_batch {
+  int device = 0, sm_count = 0;
+  int64_t D = 0, N = 0, M = 0;
+  DevBuf noff, eoff, soff, ea, eb;  // structure; soff[t] = noff[t] + eoff[t] + t: graph t's staging segment
+  DevBuf lists;                     // the graph ids of fused classes A, B, C, one after the other
+  int counts[3] = {0, 0, 0};
+  DevBuf kind, bv, dv, birth, death;  // staging pairs [N + M + D]
+  DevBuf np, status;                  // [D] pairs per graph, status (when the caller passes none)
+  DevBuf arena, tables;
+  StagedView all, large;
+  DevBuf gcnt, glst;  // gradient scratch: [N], [2 (N + M + D)]
+  int64_t bound() const { return N + M + D; }
+};
+
+static constexpr uint32_t GRAPH_BATCH_FLAGS = TLC_F_EXTENDED | TLC_F_KEEP_ZERO | TLC_F_ASC_ONLY | TLC_F_NO_SMALL;
+
+// 0..2: the fused class that takes a graph of n vertices and m edges, 3: the staged kernels
+static int graph_route(int64_t n, int64_t m) {
+  if (n <= GRAPH_A_N && m <= GRAPH_A_M) return 0;
+  if (n <= GRAPH_B_N && m <= GRAPH_B_M) return 1;
+  if (n <= GRAPH_C_N && m <= GRAPH_C_M) return 2;
+  return 3;
+}
+
+static int check_graph_batch(int64_t D, const int64_t* noff, const int64_t* eoff, const int32_t* ea, const int32_t* eb) {
+  if (D < 0 || D >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "D must be in [0, 2^31)");
+  if (!noff || !eoff) return fail(TLC_E_INVALID, "noff and eoff are required");
+  if (noff[0] != 0 || eoff[0] != 0) return fail(TLC_E_INVALID, "noff[0] and eoff[0] must be 0");
+  for (int64_t t = 0; t < D; t++) {
+    if (noff[t + 1] < noff[t]) return fail(TLC_E_INVALID, "noff is not monotone at graph " + std::to_string(t));
+    if (eoff[t + 1] < eoff[t]) return fail(TLC_E_INVALID, "eoff is not monotone at graph " + std::to_string(t));
+  }
+  if (noff[D] >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "noff[D] must be < 2^31");
+  if (eoff[D] >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "eoff[D] must be < 2^31");
+  const int64_t M = eoff[D];
+  if (M > 0 && (!ea || !eb)) return fail(TLC_E_INVALID, "ea and eb are required when there are edges");
+  std::vector<std::pair<uint64_t, int64_t>> keys((size_t)M);
+  for (int64_t t = 0; t < D; t++)
+    for (int64_t k = eoff[t]; k < eoff[t + 1]; k++) {
+      const int64_t a = ea[k], b = eb[k];
+      const std::string what = "edge " + std::to_string(k) + " (" + std::to_string(a) + ", " + std::to_string(b) +
+                               ") of graph " + std::to_string(t);
+      if (a < noff[t] || a >= noff[t + 1] || b < noff[t] || b >= noff[t + 1])
+        return fail(TLC_E_INVALID, what + " has an endpoint outside the graph's vertices [" + std::to_string(noff[t]) +
+                                       ", " + std::to_string(noff[t + 1]) + ")");
+      if (a == b) return fail(TLC_E_INVALID, what + " is a self-loop");
+      keys[(size_t)k] = {((uint64_t)std::min(a, b) << 32) | (uint64_t)std::max(a, b), k};
+    }
+  std::sort(keys.begin(), keys.end());
+  int64_t dup = -1, first = -1;
+  for (size_t i = 1; i < keys.size(); i++)
+    if (keys[i].first == keys[i - 1].first && (dup < 0 || keys[i].second < dup)) {  // the earliest repetition
+      dup = keys[i].second;
+      first = keys[i - 1].second;
+    }
+  if (dup >= 0) {
+    const int64_t t = std::upper_bound(eoff, eoff + D + 1, dup) - eoff - 1;
+    return fail(TLC_E_INVALID, "edge " + std::to_string(dup) + " (" + std::to_string(ea[dup]) + ", " +
+                                   std::to_string(eb[dup]) + ") of graph " + std::to_string(t) + " repeats edge " +
+                                   std::to_string(first));
+  }
+  return TLC_OK;
+}
+
+static GraphBatchView batch_view(const tlc_graph_batch* b, const double* f, uint32_t flags, uint8_t* status) {
+  GraphBatchView v{};
+  v.D = b->D;
+  v.noff = b->noff.as<int64_t>(); v.eoff = b->eoff.as<int64_t>(); v.soff = b->soff.as<int64_t>();
+  v.ea = b->ea.as<int32_t>(); v.eb = b->eb.as<int32_t>();
+  v.f = f;
+  v.flags = flags;
+  v.stage = DiagArea{b->kind.as<uint8_t>(), b->bv.as<int32_t>(), b->dv.as<int32_t>(), b->birth.as<double>(),
+                     b->death.as<double>()};
+  v.np = b->np.as<int32_t>();
+  v.status = status;
+  return v;
+}
+
+// the structure's device side; *b owns every allocation as soon as it exists
+static int graph_batch_upload(tlc_graph_batch* b, const int64_t* noff, const int64_t* eoff, const int32_t* ea,
+                              const int32_t* eb) {
+  const int64_t D = b->D, N = b->N, M = b->M, P = b->bound();
+  cudaDeviceProp prop;
+  CK(cudaGetDeviceProperties(&prop, b->device));
+  b->sm_count = prop.multiProcessorCount;
+  std::vector<int64_t> soff((size_t)D);
+  std::vector<int32_t> lists[3];
+  std::vector<int64_t> l_tidx, l_voff{0}, l_eoff{0};
+  for (int64_t t = 0; t < D; t++) {
+    const int64_t n = noff[t + 1] - noff[t], m = eoff[t + 1] - eoff[t];
+    soff[(size_t)t] = noff[t] + eoff[t] + t;
+    b->all.n_max = std::max(b->all.n_max, n); b->all.m_max = std::max(b->all.m_max, m);
+    const int r = graph_route(n, m);
+    if (r < 3) { lists[r].push_back((int32_t)t); continue; }
+    l_tidx.push_back(t); l_voff.push_back(l_voff.back() + n); l_eoff.push_back(l_eoff.back() + m);
+    b->large.n_max = std::max(b->large.n_max, n); b->large.m_max = std::max(b->large.m_max, m);
+  }
+  const int64_t DL = (int64_t)l_tidx.size();
+  auto up = [&](DevBuf& buf, const void* src, size_t bytes) -> cudaError_t {
+    cudaError_t e = buf.reserve(bytes);
+    if (e == cudaSuccess && bytes) e = cudaMemcpy(buf.p, src, bytes, cudaMemcpyHostToDevice);
+    return e;
+  };
+  CK(up(b->noff, noff, (size_t)(D + 1) * 8));
+  CK(up(b->eoff, eoff, (size_t)(D + 1) * 8));
+  CK(up(b->soff, soff.data(), (size_t)D * 8));
+  CK(up(b->ea, ea, (size_t)M * 4));
+  CK(up(b->eb, eb, (size_t)M * 4));
+  std::vector<int32_t> all_lists;
+  for (int c = 0; c < 3; c++) { b->counts[c] = (int)lists[c].size(); all_lists.insert(all_lists.end(), lists[c].begin(), lists[c].end()); }
+  CK(up(b->lists, all_lists.data(), all_lists.size() * 4));
+  CK(b->kind.reserve((size_t)P));
+  CK(b->bv.reserve((size_t)P * 4)); CK(b->dv.reserve((size_t)P * 4));
+  CK(b->birth.reserve((size_t)P * 8)); CK(b->death.reserve((size_t)P * 8));
+  CK(b->np.reserve((size_t)D * 4)); CK(b->status.reserve((size_t)D));
+  CK(b->gcnt.reserve((size_t)N * 4)); CK(b->glst.reserve((size_t)P * 8));
+  // staged views: `all` needs the larger arena; `large` is carved from the same bytes (the two never run in one call)
+  CK(b->arena.reserve(chunk_bytes(D, N, M, 0)));
+  b->all.c = carve(b->arena.as<char>(), D, N, M, 0, nullptr);
+  b->large.c = carve(b->arena.as<char>(), DL, l_voff.back(), l_eoff.back(), 0, nullptr);
+  // their per-graph tables: all (tidx, voff, eoff), large (tidx, voff, eoff)
+  std::vector<int64_t> tab;
+  for (int64_t t = 0; t < D; t++) tab.push_back(t);
+  tab.insert(tab.end(), noff, noff + D + 1);
+  tab.insert(tab.end(), eoff, eoff + D + 1);
+  tab.insert(tab.end(), l_tidx.begin(), l_tidx.end());
+  tab.insert(tab.end(), l_voff.begin(), l_voff.end());
+  tab.insert(tab.end(), l_eoff.begin(), l_eoff.end());
+  CK(up(b->tables, tab.data(), tab.size() * 8));
+  const int64_t* d_tab = b->tables.as<int64_t>();
+  b->all.c.tidx = d_tab; b->all.c.voff = d_tab + D; b->all.c.eoff = d_tab + 2 * D + 1;
+  const int64_t* d_l = d_tab + 3 * D + 2;
+  b->large.c.tidx = d_l; b->large.c.voff = d_l + DL; b->large.c.eoff = d_l + 2 * DL + 1;
+  return TLC_OK;
+}
+
+// kernels 2 + 3 (+ 3b) over one staged view, between the fill and the export
+static void run_graph_staged(const tlc_graph_batch* b, const GraphBatchView& v, const StagedView& s, uint32_t flags,
+                             cudaStream_t st) {
+  const ChunkView& c = s.c;
+  if (c.T <= 0) return;
+  launch_graph_fill(v, c, b->sm_count, st);
+  const Params p{0, TLC_MODE_NODE, TLC_DESC_SUM, 5, flags, 0};
+  const bool ext = (flags & TLC_F_EXTENDED) != 0;
+  const int mask = (flags & TLC_F_ASC_ONLY) ? 1 : 3;
+  const int block = block_for(s.m_max);
+  launch_sort(p, c, block, mask, 0, st);
+  const int64_t uf_ints = 2 * s.n_max * 4 <= 96 * 1024 ? 2 * s.n_max : 0;
+  launch_union_find(p, c, block, (int)uf_ints, ext ? 1 : 0, mask, 0, st);
+  if (ext) {
+    const int64_t lp_ints = 3 * s.n_max * 4 <= 200 * 1024 ? 3 * s.n_max : 0;
+    launch_loops(p, c, std::min(block, 128), (int)lp_ints, s.n_max, st);
+  }
+  launch_graph_export(v, c, b->sm_count, st);
+}
+
+extern "C" {
+
+int tlc_graph_batch_create(int device, int64_t D, const int64_t* noff, const int64_t* eoff, const int32_t* ea,
+                           const int32_t* eb, tlc_graph_batch** out) {
+  if (!out) return fail(TLC_E_INVALID, "out is NULL");
+  int rc = check_graph_batch(D, noff, eoff, ea, eb);
+  if (rc || (rc = select_device(device))) return rc;
+  tlc_graph_batch* b = new tlc_graph_batch();
+  b->device = device;
+  b->D = D; b->N = noff[D]; b->M = eoff[D];
+  rc = graph_batch_upload(b, noff, eoff, ea, eb);
+  if (rc != TLC_OK) { delete b; return rc; }
+  *out = b;
+  return TLC_OK;
+}
+
+int tlc_graph_batch_destroy(tlc_graph_batch* b) {
+  if (!b) return TLC_OK;
+  cudaSetDevice(b->device);
+  delete b;
+  return TLC_OK;
+}
+
+int tlc_graph_batch_pair_bound(const tlc_graph_batch* b, int64_t* bound) {
+  if (!b || !bound) return fail(TLC_E_INVALID, "NULL argument");
+  *bound = b->bound();
+  return TLC_OK;
+}
+
+int tlc_graph_batch_diagrams_dev(tlc_graph_batch* b, const double* dev_f, uint32_t flags, tlc_diagrams* out,
+                                 uint8_t* dev_status, void* stream) {
+  if (flags & ~GRAPH_BATCH_FLAGS)
+    return fail(TLC_E_INVALID, "flags may only hold TLC_F_EXTENDED, TLC_F_KEEP_ZERO, TLC_F_ASC_ONLY and TLC_F_NO_SMALL");
+  if ((flags & TLC_F_ASC_ONLY) && (flags & TLC_F_EXTENDED))
+    return fail(TLC_E_INVALID, "TLC_F_ASC_ONLY excludes TLC_F_EXTENDED (the loops need the descending sweep)");
+  if (!out || !out->poff) return fail(TLC_E_INVALID, "out and out->poff are required");
+  if (!b) return fail(TLC_E_INVALID, "batch is NULL");
+  if (b->N > 0 && !dev_f) return fail(TLC_E_INVALID, "dev_f is NULL");
+  if (out->cap < b->bound())
+    return fail(TLC_E_CAPACITY, "out->cap is " + std::to_string(out->cap) + ", the batch's pair bound is " +
+                                    std::to_string(b->bound()));
+  CK(cudaSetDevice(b->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const GraphBatchView v = batch_view(b, dev_f, flags, dev_status ? dev_status : b->status.as<uint8_t>());
+  if (flags & TLC_F_NO_SMALL) {
+    run_graph_staged(b, v, b->all, flags, st);
+  } else {
+    const int32_t* l = b->lists.as<int32_t>();
+    const int32_t* const lists[3] = {l, l + b->counts[0], l + b->counts[0] + b->counts[1]};
+    launch_graph_pd_small(v, lists, b->counts, st);
+    run_graph_staged(b, v, b->large, flags, st);
+  }
+  launch_scan_counts(v.np, b->D, out->poff, st);
+  const DiagArea dst{out->kind, out->bv, out->dv, out->birth, out->death};
+  launch_gather_pairs(v.np, v.soff, out->poff, b->D, v.stage, v.stage, INT64_MAX, dst, b->sm_count, st);
+  if (out->npairs && b->D > 0) CK(cudaMemcpyAsync(out->npairs, v.np, (size_t)b->D * 4, cudaMemcpyDeviceToDevice, st));
+  CK(cudaGetLastError());
+  return TLC_OK;
+}
+
+int tlc_graph_batch_grad_dev(tlc_graph_batch* b, const tlc_diagrams* d, const double* dev_grad_birth,
+                             const double* dev_grad_death, double* dev_grad_f, void* stream) {
+  if (!d || !d->poff || !d->bv || !d->dv) return fail(TLC_E_INVALID, "d, d->poff, d->bv and d->dv are required");
+  if (!b) return fail(TLC_E_INVALID, "batch is NULL");
+  if (b->N > 0 && !dev_grad_f) return fail(TLC_E_INVALID, "dev_grad_f is NULL");
+  if (b->D == 0) return TLC_OK;
+  CK(cudaSetDevice(b->device));
+  const GraphBatchView v = batch_view(b, nullptr, 0, nullptr);
+  launch_graph_grad(v, d->poff, d->bv, d->dv, dev_grad_birth, dev_grad_death, b->gcnt.as<int32_t>(),
+                    b->glst.as<int32_t>(), dev_grad_f, b->sm_count, (cudaStream_t)stream);
+  CK(cudaGetLastError());
+  return TLC_OK;
+}
+
+}  // extern "C"

@@ -456,6 +456,30 @@ void launch_scan_counts(const int32_t* np, int64_t E, int64_t* poff, cudaStream_
 void launch_gather_pairs(const int32_t* np, const int64_t* soff, const int64_t* poff, int64_t E, const DiagArea& a,
                          const DiagArea& b, int64_t split_at, const DiagArea& out, int sm_count, cudaStream_t st);
 
+// kernel 9 (k9_graph_pd.cu): diagrams of a batch of caller-supplied graphs (tlc_graph_batch_*).  Graph t owns vertices
+// noff[t] .. noff[t+1] and edges eoff[t] .. eoff[t+1] of (ea, eb), batch-global ids; its pairs are staged at soff[t] =
+// noff[t] + eoff[t] + t (capacity n + m + 1), np[t] / status[t] are its pair count (0 unless the status has pairs) and status
+struct GraphBatchView {
+  int64_t D;
+  const int64_t *noff, *eoff, *soff;
+  const int32_t *ea, *eb;
+  const double* f;
+  uint32_t flags;
+  DiagArea stage;
+  int32_t* np;
+  uint8_t* status;
+};
+// the fused route's size classes (kernel S's): a warp per graph, a 128-thread CTA, a 256-thread CTA
+constexpr int GRAPH_A_N = 64, GRAPH_A_M = 256, GRAPH_B_N = 256, GRAPH_B_M = 2048, GRAPH_C_N = 1024, GRAPH_C_M = 4096;
+// lists[c] / counts[c]: the graphs of class c
+void launch_graph_pd_small(const GraphBatchView& b, const int32_t* const lists[3], const int counts[3], cudaStream_t st);
+// staged route: c.tidx[s] = graph of staged entry s, c.voff / c.eoff its segments in the arena
+void launch_graph_fill(const GraphBatchView& b, const ChunkView& c, int sm_count, cudaStream_t st);
+void launch_graph_export(const GraphBatchView& b, const ChunkView& c, int sm_count, cudaStream_t st);
+// cnt int32[N], lst int32[2 (N + M + D)]: scratch
+void launch_graph_grad(const GraphBatchView& b, const int64_t* poff, const int32_t* bv, const int32_t* dv, const double* gb,
+                       const double* gd, int32_t* cnt, int32_t* lst, double* grad_f, int sm_count, cudaStream_t st);
+
 // multi-GPU exchange by peer stores (k5_gather.cu): the tables of all ranks, this rank's own included
 constexpr int PEER_MAX = 16;
 constexpr size_t PEER_HEADER_BYTES = 256;  // [u32 arrival counter | pad] in front of the float32 rows

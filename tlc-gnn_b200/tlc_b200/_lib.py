@@ -22,7 +22,9 @@ ST_NOT_SMALL = 255
 E_INVALID, E_CUDA, E_NOMEM, E_NODEVICE, E_CAPACITY = -1, -2, -3, -4, -5
 K_UP, K_ESS, K_DOWN, K_ESS_REV, K_ONE = 0, 1, 2, 3, 4
 ST_OK, ST_TRIVIAL, ST_EMPTY, ST_DISCONNECTED, ST_DEGENERATE, ST_UNKNOWN_NODE, ST_BAD_DESCRIPTOR, ST_NO_TREE_EDGES = range(8)
-ST_NAMES = ["OK", "TRIVIAL", "EMPTY", "DISCONNECTED", "DEGENERATE", "UNKNOWN_NODE", "BAD_DESCRIPTOR", "NO_TREE_EDGES"]
+ST_NONFINITE = 8
+ST_NAMES = ["OK", "TRIVIAL", "EMPTY", "DISCONNECTED", "DEGENERATE", "UNKNOWN_NODE", "BAD_DESCRIPTOR", "NO_TREE_EDGES",
+            "NONFINITE"]
 
 EXPORTS = ["tlc_graph_create", "tlc_graph_destroy", "tlc_vicinity_pi", "tlc_vicinity_pi_dev", "tlc_vicinity_sizes",
            "tlc_vicinity_detail", "tlc_union_find", "tlc_pimg_transform", "tlc_last_error", "tlc_version",
@@ -32,7 +34,9 @@ EXPORTS = ["tlc_graph_create", "tlc_graph_destroy", "tlc_vicinity_pi", "tlc_vici
            "tlc_last_table_two_root",
            "tlc_ollivier_ricci", "tlc_graph_set_hks_time", "tlc_table_build_ms", "tlc_vicinity_diagrams",
            "tlc_vicinity_diagrams_dev", "tlc_pimg_batch_dev", "tlc_pimg_batch_grad_dev",
-           "tlc_wasserstein_workspace_bytes", "tlc_wasserstein_batch_dev", "tlc_wasserstein_batch_grad_dev"]
+           "tlc_wasserstein_workspace_bytes", "tlc_wasserstein_batch_dev", "tlc_wasserstein_batch_grad_dev",
+           "tlc_graph_batch_create", "tlc_graph_batch_destroy", "tlc_graph_batch_pair_bound",
+           "tlc_graph_batch_diagrams_dev", "tlc_graph_batch_grad_dev"]
 
 
 class Params(C.Structure):
@@ -105,6 +109,16 @@ def lib():
                                             + [vp] * 4)
     L.tlc_wasserstein_batch_grad_dev.restype = C.c_int
     L.tlc_wasserstein_batch_grad_dev.argtypes = [C.c_int, i64] + [vp] * 8 + [u32, C.c_double, C.c_double] + [vp] * 9
+    L.tlc_graph_batch_create.restype = C.c_int
+    L.tlc_graph_batch_create.argtypes = [C.c_int, i64, vp, vp, vp, vp, C.POINTER(vp)]
+    L.tlc_graph_batch_destroy.restype = C.c_int
+    L.tlc_graph_batch_destroy.argtypes = [vp]
+    L.tlc_graph_batch_pair_bound.restype = C.c_int
+    L.tlc_graph_batch_pair_bound.argtypes = [vp, C.POINTER(i64)]
+    L.tlc_graph_batch_diagrams_dev.restype = C.c_int
+    L.tlc_graph_batch_diagrams_dev.argtypes = [vp, vp, u32, C.POINTER(Diagrams), vp, vp]
+    L.tlc_graph_batch_grad_dev.restype = C.c_int
+    L.tlc_graph_batch_grad_dev.argtypes = [vp, C.POINTER(Diagrams), vp, vp, vp, vp]
     L.tlc_last_error.restype = C.c_char_p
     L.tlc_version.restype = C.c_char_p
     L.tlc_launch_count.restype = i64

@@ -543,6 +543,151 @@ def wasserstein_distances(poff_x, birth_x, death_x, poff_y, birth_y, death_y, ki
     return (dist, (mx, my)) if return_matching else dist
 
 
+def _to_numpy(a, dtype):
+    if hasattr(a, "detach"):  # a CPU torch tensor
+        a = a.detach().cpu().numpy()
+    return np.ascontiguousarray(a, dtype=dtype)
+
+
+def normalize_edge_index(ptr, edge_index):
+    """the C-ABI's edge lists from PyG's Batch.ptr int[D+1] and edge_index int[2, E] (numpy or CPU tensors): the first
+    occurrence of every undirected edge is kept, as given, and later ones (either direction) are dropped; the kept edges
+    are grouped by the graph of their first endpoint, in input order inside a graph (that order is the sweeps'
+    tie-break).  Self-loops and out-of-range or cross-graph edges are kept for tlc_graph_batch_create to reject.
+    Returns (noff int64[D+1], eoff int64[D+1], ea int32[M], eb int32[M])."""
+    noff = _to_numpy(ptr, np.int64).reshape(-1)
+    ei = _to_numpy(edge_index, np.int64)
+    if noff.size < 1:
+        raise ValueError("ptr must have D + 1 >= 1 entries")
+    if ei.size == 0:
+        ei = ei.reshape(2, 0)
+    if ei.ndim != 2 or ei.shape[0] != 2:
+        raise ValueError("edge_index must have shape [2, E], got %s" % (ei.shape,))
+    a, b = ei[0], ei[1]
+    lo, hi = np.minimum(a, b), np.maximum(a, b)
+    span = int(max(int(noff[-1]), int(hi.max(initial=0)) + 1, 1))
+    _, first = np.unique((lo - int(lo.min(initial=0))) * span + hi, return_index=True)
+    keep = np.sort(first)
+    a, b = a[keep], b[keep]
+    D = noff.size - 1
+    g = np.clip(np.searchsorted(noff, a, side="right") - 1, 0, max(D - 1, 0))
+    order = np.argsort(g, kind="stable")
+    a, b, g = a[order], b[order], g[order]
+    eoff = np.zeros(D + 1, np.int64)
+    if D > 0:
+        np.cumsum(np.bincount(g, minlength=D)[:D], out=eoff[1:])
+    elif a.size:
+        raise ValueError("edges given for a batch of no graphs")
+    return noff, eoff, a.astype(np.int32), b.astype(np.int32)
+
+
+_GraphDiagramsFn = None
+
+
+def _graph_diagrams_fn():
+    """the torch.autograd.Function over tlc_graph_batch_diagrams_dev / tlc_graph_batch_grad_dev (built on first use)"""
+    global _GraphDiagramsFn
+    if _GraphDiagramsFn is not None:
+        return _GraphDiagramsFn
+    import torch
+    from torch.autograd.function import once_differentiable
+
+    def stream(dev):
+        return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+
+    class GraphDiagrams(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, f, batch, flags):
+            dev = f.device
+            P = batch.pair_bound
+            poff = torch.empty(batch.D + 1, dtype=torch.int64, device=dev)
+            kind = torch.zeros(P, dtype=torch.uint8, device=dev)
+            bv = torch.zeros(P, dtype=torch.int32, device=dev)
+            dv = torch.zeros(P, dtype=torch.int32, device=dev)
+            birth = torch.zeros(P, dtype=torch.float64, device=dev)
+            death = torch.zeros(P, dtype=torch.float64, device=dev)
+            status = torch.empty(batch.D, dtype=torch.uint8, device=dev)
+            d = L.Diagrams(P, poff.data_ptr(), None, kind.data_ptr(), bv.data_ptr(), dv.data_ptr(), birth.data_ptr(),
+                           death.data_ptr())
+            L.check(L.lib().tlc_graph_batch_diagrams_dev(batch._h, f.data_ptr(), flags, C.byref(d),
+                                                         status.data_ptr() if batch.D else None, stream(dev)))
+            ctx.save_for_backward(poff, bv, dv)
+            ctx.batch = batch
+            ctx.set_materialize_grads(False)  # an unused birth / death gradient reaches the library as NULL
+            ctx.mark_non_differentiable(poff, kind, bv, dv, status)
+            return poff, kind, bv, dv, birth, death, status
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, _gp, _gk, _gbv, _gdv, grad_birth, grad_death, _gs):
+            poff, bv, dv = ctx.saved_tensors
+            batch = ctx.batch
+            dev = bv.device
+            gb = grad_birth.contiguous() if grad_birth is not None else None
+            gd = grad_death.contiguous() if grad_death is not None else None
+            for g, what in ((gb, "grad_birth"), (gd, "grad_death")):
+                _dev_ptr(g, "float64", (batch.pair_bound,), dev.index, what)
+            grad_f = torch.empty(batch.N, dtype=torch.float64, device=dev)
+            d = L.Diagrams(batch.pair_bound, poff.data_ptr(), None, None, bv.data_ptr(), dv.data_ptr(), None, None)
+            L.check(L.lib().tlc_graph_batch_grad_dev(batch._h, C.byref(d), gb.data_ptr() if gb is not None else None,
+                                                     gd.data_ptr() if gd is not None else None, grad_f.data_ptr(),
+                                                     stream(dev)))
+            return grad_f, None, None
+
+    _GraphDiagramsFn = GraphDiagrams
+    return _GraphDiagramsFn
+
+
+class GraphBatch:
+    """A batch of graphs resident on one GPU, for persistence diagrams under a filtration that changes from call to
+    call (a learnable filtration, or whole-graph persistence over a dataloader batch).  ptr int[D+1] and edge_index
+    int[2, E] are PyG's Batch.ptr / edge_index (numpy or CPU tensors); edge_index may list both directions of an edge
+    (see normalize_edge_index).  The structure is checked and uploaded once."""
+
+    def __init__(self, ptr, edge_index, device=0):
+        self.noff, self.eoff, self.ea, self.eb = normalize_edge_index(ptr, edge_index)
+        self.D = int(self.noff.size - 1)
+        self.N = int(self.noff[-1])
+        self.M = int(self.eoff[-1])
+        self.device = int(device)
+        self._h = C.c_void_p()
+        L.check(L.lib().tlc_graph_batch_create(self.device, self.D, self.noff.ctypes.data, self.eoff.ctypes.data,
+                                               self.ea.ctypes.data, self.eb.ctypes.data, C.byref(self._h)))
+        bound = C.c_int64(0)
+        L.check(L.lib().tlc_graph_batch_pair_bound(self._h, C.byref(bound)))
+        self.pair_bound = int(bound.value)
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            L.lib().tlc_graph_batch_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def diagrams(self, f, extended=False, keep_zero=False, asc_only=False, no_small=False):
+        """persistence diagrams of every graph under the filtration f (float64 CUDA tensor [N] on the batch's device;
+        may require grad).  Returns a dict of CUDA tensors: poff int64[D+1] (graph t's pairs are [poff[t], poff[t+1]),
+        poff[D] the live length), kind uint8, bv / dv int32 (batch vertex ids), birth / death float64 -- all sized to
+        the pair bound N + M + D, so that nothing waits for the device -- and status uint8[D].  birth and death are
+        differentiable in f: the gradient of a pair value flows to the vertex that carries it.  Graph t's pairs are the
+        pipeline's for a node-mode vicinity equal to that graph (Union_find + Accelerate_PD, accelerated_PD.py:26,115):
+        PD_up, [min,max], PD_down, [max,min], then PD_one with extended; no pairs for a disconnected graph or one with a
+        non-finite value (status ST_NONFINITE).  f is not normalised.  no_small: every graph through the staged kernels
+        (same results).  Runs on the current stream.  The dict plugs into persistence_images(d["poff"], d["birth"],
+        d["death"], d["kind"], mask) and wasserstein_distances."""
+        if extended and asc_only:
+            raise ValueError("asc_only excludes extended (the loops need the descending sweep)")
+        _dev_ptr(f, "float64", (self.N,), self.device, "f")
+        flags = ((L.F_EXTENDED if extended else 0) | (L.F_KEEP_ZERO if keep_zero else 0)
+                 | (L.F_ASC_ONLY if asc_only else 0) | (L.F_NO_SMALL if no_small else 0))
+        poff, kind, bv, dv, birth, death, status = _graph_diagrams_fn().apply(f, self, flags)
+        return dict(poff=poff, kind=kind, bv=bv, dv=dv, birth=birth, death=death, status=status)
+
+
 def launch_count():
     return int(L.lib().tlc_launch_count())
 
