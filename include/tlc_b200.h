@@ -214,6 +214,42 @@ int tlc_vicinity_diagrams_dev(tlc_graph *g, const int32_t *dev_targets, int64_t 
 int tlc_vicinity_diagrams(tlc_graph *g, const int32_t *targets, int64_t E, const tlc_params *p, tlc_diagrams *out,
                           double *out_pi, uint8_t *out_status, int64_t *total_pairs);
 
+/* The vicinities of a batch and their filtration in graph-batch layout (PyG Batch: ptr / edge_index), straight into device
+ * buffers: the input of tlc_graph_batch_create_dev for the GPU-resident chain vicinity -> learned filtration -> diagrams ->
+ * images / Wasserstein -> backward (the student input of Knowledge_Distillation/data_utils_NC.py:183 / data_utils_LP.py:196,
+ * `filtration_val` and `edge_index` of the generator's 9-tuple; ConvCurv_GIN.py, mode='filtration').
+ *   voff / eoff [E+1] (required): exclusive offsets of the targets' vertex and edge segments, in TARGET order;
+ *     voff[t+1] - voff[t] and eoff[t+1] - eoff[t] are tlc_vicinity_sizes' n[t] and m[t] for every target.
+ *   vert [cap_v]: graph ids (tlc_graph_create numbering), ascending inside each target (kernel 1's vertex order).
+ *   ea / eb [cap_e]: one entry per undirected induced edge, batch-global vertex ids voff[t] + local id, ea < eb,
+ *     lexicographic inside each target -- the edge order the pipeline's sweeps use as their tie-break.
+ *   fval [cap_v]: the filtration value of every vertex; for a target whose status is OK or TRIVIAL bit-identical to
+ *     tlc_vicinity_detail's fval with the same params, NaN for every other target's vertices (tlc_graph_batch_diagrams_dev
+ *     reports those as TLC_ST_NONFINITE).  NULL: no filtration is computed.
+ * Any of vert / ea / eb / fval may be NULL (not written).  dev_status uint8[E] (may be NULL): tlc_vicinity_pi_dev's status
+ * for the same targets and params -- except that without fval a vicinity the filtration would find DEGENERATE (a zero
+ * normaliser) reports OK or TRIVIAL, since that status is a property of the filtration values.
+ * flags: TLC_F_NORM, TLC_F_NORM_EPS, TLC_F_SUM_PLAIN and the TLC_F_FILT_* filtrations, with their meanings in the batch
+ * calls; resolution and img_mask are ignored.  Any other flag and every argument error return TLC_E_INVALID before any
+ * CUDA call; E must lie in [0, 2^31), and batch ids are int32, so the call fails with TLC_E_INVALID when ea / eb are asked
+ * for and *total_v >= 2^31.
+ * Capacity: voff, eoff, *total_v, *total_e and the statuses are always written; if *total_v > cap_v or *total_e > cap_e the
+ * call returns TLC_E_CAPACITY after kernel 1's counting pass alone and leaves the other arrays untouched (cap = 0: a
+ * sizing call; again with the totals as capacities it succeeds).  Output is bit-identical from run to run.
+ * The call always takes the materialised route (kernel 1 fill, the filtration, kernel 1c's edge list, then kernel 10's
+ * export): the fused small-vicinity kernels and the graph-row route never write a vicinity's structure to memory.  It
+ * runs on the graph's stream (tlc_graph_set_stream) and, like the diagram calls, SYNCHRONISES with it (the chunk plan
+ * needs the counting pass on the host); every pointer is a DEVICE pointer on the graph's device. */
+typedef struct {
+  int64_t cap_v, cap_e;   /* capacities of the vertex / edge arrays                                     */
+  int64_t *voff, *eoff;   /* [E+1] exclusive offsets, TARGET order (required)                           */
+  int32_t *vert;          /* [cap_v] graph ids, ascending inside each target               (may be NULL) */
+  int32_t *ea, *eb;       /* [cap_e] batch-global vertex ids, ea < eb, lexicographic       (may be NULL) */
+  double *fval;           /* [cap_v] filtration value of each vertex (NULL: no filtration is computed)   */
+} tlc_vicinity_batch;
+int tlc_vicinity_batch_dev(tlc_graph *g, const int32_t *dev_targets, int64_t E, const tlc_params *p,
+                           tlc_vicinity_batch *out, uint8_t *dev_status, int64_t *total_v, int64_t *total_e);
+
 /* compute_ricci_curvature (loaddatas.py:105-123): OllivierRicci(G, alpha, method="Sinkhorn").compute_ricci_curvature() on the
  * unweighted graph given as a symmetric CSR (ascending rows, no self-loops) -- the step BEFORE the path, whose output is
  * the `kappa` of tlc_graph_create.  out_kappa[nnz] receives the curvature of every directed entry (both directions of an
@@ -340,6 +376,18 @@ int tlc_wasserstein_batch_grad_dev(int device, int64_t D, const int64_t *dev_pof
 typedef struct tlc_graph_batch tlc_graph_batch;
 int tlc_graph_batch_create(int device, int64_t D, const int64_t *noff, const int64_t *eoff, const int32_t *ea,
                            const int32_t *eb, tlc_graph_batch **out);
+/* tlc_graph_batch_create_dev: the same batch from structure already on the device (dev_noff / dev_eoff int64[D+1],
+ * dev_ea / dev_eb int32[M], M = eoff[D]; e.g. tlc_vicinity_batch_dev's voff / eoff / ea / eb), in CANONICAL FORM: within
+ * each graph ea < eb and the edges strictly ascending in (ea, eb) -- that order, not an input order, is then the sweeps'
+ * tie-break.  The offsets are copied to the host once (route planning needs them) and checked there as in
+ * tlc_graph_batch_create; a device kernel checks the edges (endpoints inside their graph, no self-loop, ea < eb, strictly
+ * after the graph's previous edge) and the TLC_E_INVALID message names the graph and the FIRST offending edge in
+ * tlc_graph_batch_create's wording.  No sort: O(M).  D = 0 and graphs without edges are allowed.  The work runs on
+ * `stream` (a cudaStream_t, NULL: the legacy default stream), which the call SYNCHRONISES with (after the offset copy and
+ * after the check); like tlc_graph_batch_create it allocates every buffer of the batch.  The diagram and gradient calls
+ * are the same for both creations. */
+int tlc_graph_batch_create_dev(int device, int64_t D, const int64_t *dev_noff, const int64_t *dev_eoff,
+                               const int32_t *dev_ea, const int32_t *dev_eb, void *stream, tlc_graph_batch **out);
 int tlc_graph_batch_destroy(tlc_graph_batch *b);
 int tlc_graph_batch_pair_bound(const tlc_graph_batch *b, int64_t *bound);
 int tlc_graph_batch_diagrams_dev(tlc_graph_batch *b, const double *dev_f, uint32_t flags, tlc_diagrams *out,

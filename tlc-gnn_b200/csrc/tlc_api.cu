@@ -144,6 +144,15 @@ struct DiagCollect {
   DevBuf chunk;  // per chunk: staging offset and call row of each target
 };
 
+// the outputs of a tlc_vicinity_batch_dev call while it runs: voff / eoff hold the final offsets before the first chunk,
+// every chunk's targets are exported into the arrays at those offsets
+struct BatchCollect {
+  bool on = false;
+  tlc_vicinity_batch out{};
+  uint8_t* status = nullptr;
+  int64_t total_v = 0, total_e = 0;
+};
+
 struct tlc_graph {
   int device = 0;
   GraphView gv{};  // views of rowptr / col / kappa / rec
@@ -210,6 +219,7 @@ struct tlc_graph {
   std::vector<cudaEvent_t> ev_pool;  // stage-timing events, reused from call to call
   int sm_count = 0;
   DiagCollect dg;
+  BatchCollect vb;
 
   ~tlc_graph() {
     for (void* q : peer_opened) cudaIpcCloseMemHandle(q);
@@ -483,17 +493,13 @@ static bool takes_table(const tlc_graph* g, bool use_table, const SubRange& r) {
   return use_table && filtration_table_smem(g->gv.N, r.n_max) <= 226 * 1024;
 }
 
-// returns the number of targets whose filtration came from kernel 1t's tables
-static int64_t run_stages(tlc_graph* g, const Params& p, const ChunkView& c, int64_t n_max, int64_t m_max,
-                          const std::vector<SubRange>& subs, double* d_pi, float* d_pi32, uint8_t* d_status,
-                          bool want_lists, StageTimer& tm, bool use_table) {
+// the filtration of a chunk: a structural one or HKS over the whole chunk, else kernel 1t / 1b per sub-range; returns
+// the number of targets whose filtration came from kernel 1t's tables
+static int64_t run_filtration(tlc_graph* g, const Params& p, const ChunkView& c, int64_t n_max, int block,
+                              const std::vector<SubRange>& subs, bool use_table) {
   cudaStream_t st = g->stream;
-  const int block = block_for(m_max);
   VicinityScratch vs = make_vs(g);
   int64_t from_table = 0;
-  tm.mark(1);
-  if (!c.dbm) launch_vicinity_fill(g->gv, p, c, vs, g->work_counter.as<int>(), st);
-  tm.mark(2);
   if (p.flags & TLC_F_FILT_HKS) launch_hks_filtration(p, c, g->hks_time, n_max, st);
   else if (p.flags & (TLC_F_FILT_DEGREE | TLC_F_FILT_CENTRALITY | TLC_F_FILT_CLUSTERING)) launch_degree_filtration(p, c, st);
   else {
@@ -505,6 +511,20 @@ static int64_t run_stages(tlc_graph* g, const Params& p, const ChunkView& c, int
       else launch_filtration(p, c, r.t0, r.cnt, block, r.n_max, s);
     });
   }
+  return from_table;
+}
+
+// returns the number of targets whose filtration came from kernel 1t's tables
+static int64_t run_stages(tlc_graph* g, const Params& p, const ChunkView& c, int64_t n_max, int64_t m_max,
+                          const std::vector<SubRange>& subs, double* d_pi, float* d_pi32, uint8_t* d_status,
+                          bool want_lists, StageTimer& tm, bool use_table) {
+  cudaStream_t st = g->stream;
+  const int block = block_for(m_max);
+  VicinityScratch vs = make_vs(g);
+  tm.mark(1);
+  if (!c.dbm) launch_vicinity_fill(g->gv, p, c, vs, g->work_counter.as<int>(), st);
+  tm.mark(2);
+  const int64_t from_table = run_filtration(g, p, c, n_max, block, subs, use_table);
   // ascending sweep: vertex-ordered kernels 2v + 3v; targets they hand back (tfb) and, when the descending
   // sweep is wanted (diagram output, Pos/Neg lists for the loops), the edge-sorted kernels 2 + 3.  The image
   // only needs PD_up and [min,max]: PD_down and [max,min] have death <= birth, i.e. weight 0 (SURVEY.md F6).
@@ -542,6 +562,24 @@ static int64_t run_stages(tlc_graph* g, const Params& p, const ChunkView& c, int
   launch_pimg(p, c, d_pi, d_pi32, d_status, std::max(32, std::min(block, 256)), st);
   tm.mark(-1);
   return from_table;
+}
+
+// vicinity batch call (materialised route): kernel 1's fill, the filtration when values are wanted (not with a bad
+// descriptor: no target reaches it), kernel 1c's edge list of every target, then kernel 10's export of the chunk into the
+// call's arrays at their final offsets
+static void run_structure(tlc_graph* g, const Params& p, const ChunkView& c, int64_t n_max, int64_t m_max,
+                          const std::vector<SubRange>& subs, bool bad_desc, StageTimer& tm) {
+  cudaStream_t st = g->stream;
+  const int block = block_for(m_max);
+  const tlc_vicinity_batch& o = g->vb.out;
+  tm.mark(1);
+  launch_vicinity_fill(g->gv, p, c, make_vs(g), g->work_counter.as<int>(), st);
+  tm.mark(2);
+  if (o.fval && !bad_desc) run_filtration(g, p, c, n_max, block, subs, false);
+  tm.mark(5);
+  launch_edgelist(p, c, block, 0, st);
+  tm.mark(-1);
+  launch_vicinity_export(c, o.voff, o.eoff, o.vert, o.ea, o.eb, o.fval, g->vb.status, bad_desc ? 1 : 0, st);
 }
 
 static int check_params(const tlc_params* p) {
@@ -658,7 +696,8 @@ static int plan_call(tlc_graph* g, const HostStage& h, int64_t E, bool light, in
     std::vector<uint64_t> keys;
     keys.reserve(E);
     for (int64_t i = 0; i < E; i++) {
-      if (h.st[i] != TLC_ST_OK) continue;
+      // (the vicinity batch call exports the structure of every vicinity that has vertices, whatever its status)
+      if (h.st[i] != TLC_ST_OK && !(g->vb.on && h.n[i] > 0)) continue;
       const uint64_t cls = (uint64_t)smem_class(h.n[i]);
       const uint64_t msz = (uint64_t)std::min<int64_t>(h.m[i], (1 << 28) - 1);
       keys.push_back((cls << 61) | ((((uint64_t)1 << 28) - 1 - msz) << 32) | (uint64_t)i);
@@ -874,7 +913,7 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
   // (pair output -- detail or diagram call -- wants PD_down and [max,min] unless TLC_F_ASC_ONLY)
   const bool want_pairs = detail != nullptr || g->dg.on;
   const bool want_desc_call = ((p.flags & TLC_F_EXTENDED) != 0 || want_pairs) && !(p.flags & TLC_F_ASC_ONLY);
-  const bool direct_ok = g->ball_cache.p != nullptr && g->gminw.p != nullptr && !want_desc_call && !bad_desc &&
+  const bool direct_ok = g->ball_cache.p != nullptr && g->gminw.p != nullptr && !want_desc_call && !bad_desc && !g->vb.on &&
                          p.mode <= TLC_MODE_NODE && !(p.flags & TLC_F_FILT_ANY_STRUCT) &&
                          !(p.flags & (TLC_F_NO_DIRECT | TLC_F_EDGE_SORTED)) && (size_t)Wd * 8 <= 64 * 1024;
   VicinityScratch vs = make_vs(g);
@@ -912,16 +951,31 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
   CK(cudaMemcpyAsync(h.st, d_st, (size_t)E, cudaMemcpyDeviceToHost, st));
   CK(cudaMemcpyAsync(h.bytes, d_bytes, (size_t)E * 8, cudaMemcpyDeviceToHost, st));
   // rows of targets that never reach the image kernel stay zero (riccidist2dgm.py:363)
-  CK(cudaMemsetAsync(d_pi, 0, (size_t)E * r2 * sizeof(double), st));
+  if (d_pi) CK(cudaMemsetAsync(d_pi, 0, (size_t)E * r2 * sizeof(double), st));
   if (d_pi32) CK(cudaMemsetAsync(d_pi32, 0, (size_t)E * r2 * sizeof(float), st));
   CK(cudaStreamSynchronize(st));
   if (bad_desc) {  // KeyError in perturb_filter_function for every target that got that far (accelerated_PD.py:13)
     for (int64_t i = 0; i < E; i++) if (h.st[i] == TLC_ST_OK) h.st[i] = TLC_ST_BAD_DESCRIPTOR;
     if (d_status) CK(cudaMemcpyAsync(d_status, h.st, (size_t)E, cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));
-    return TLC_OK;
+    if (!g->vb.on) return TLC_OK;  // (the vicinity batch call still exports the structure)
+  } else if (d_status) {
+    CK(cudaMemcpyAsync(d_status, d_st, (size_t)E, cudaMemcpyDeviceToDevice, st));
   }
-  if (d_status) CK(cudaMemcpyAsync(d_status, d_st, (size_t)E, cudaMemcpyDeviceToDevice, st));
+  if (g->vb.on) {  // the final offsets (kernel 7's scan of n and m) and totals; too small a capacity ends the call here
+    BatchCollect& b = g->vb;
+    launch_scan_counts(d_n, E, b.out.voff, st);
+    launch_scan_counts(d_m, E, b.out.eoff, st);
+    b.total_v = 0; b.total_e = 0;
+    for (int64_t i = 0; i < E; i++) { b.total_v += h.n[i]; b.total_e += h.m[i]; }
+    CK(cudaStreamSynchronize(st));
+    if (b.total_v > b.out.cap_v || b.total_e > b.out.cap_e)
+      return fail(TLC_E_CAPACITY, "the vicinities hold " + std::to_string(b.total_v) + " vertices and " +
+                                      std::to_string(b.total_e) + " edges, cap_v is " + std::to_string(b.out.cap_v) +
+                                      " and cap_e is " + std::to_string(b.out.cap_e));
+    if ((b.out.ea || b.out.eb) && b.total_v >= ((int64_t)1 << 31))
+      return fail(TLC_E_INVALID, "the vicinities hold " + std::to_string(b.total_v) + " vertices: int32 batch ids need < 2^31");
+  }
   for (int64_t i = 0; i < E; i++)
     if (h.st[i] == TLC_ST_OK) { s.bytes += h.bytes[i]; s.live++; s.sum_n += h.n[i]; if (!light) s.sum_m += h.m[i]; }
 
@@ -945,7 +999,9 @@ static int run_staged(tlc_graph* g, const int32_t* d_targets, int64_t E, const t
     CK(cudaMemcpyAsync((void*)(c.eoff + k.T), &k.Ne, 8, cudaMemcpyHostToDevice, st));
     const std::vector<SubRange> subs = split_subranges(g, order, pos, k.T, h.n);
     std::vector<uint8_t> fbv;  // graph-row batch call: targets kernel 3v handed back (redone below)
-    if (direct) {
+    if (g->vb.on) {
+      run_structure(g, p, c, k.n_max, k.m_max, subs, bad_desc, tm);
+    } else if (direct) {
       c.count_m = light ? 1 : 0;
       // tm: counted by kernel 1b (batch call) or known from the full counting pass (detail call)
       if (!light) CK(cudaMemcpyAsync((void*)c.tm, h.tm + pos, (size_t)k.T * 4, cudaMemcpyHostToDevice, st));
@@ -1643,6 +1699,50 @@ int tlc_vicinity_diagrams(tlc_graph* g, const int32_t* targets, int64_t E, const
   return total > out->cap ? capacity_error(total, out->cap) : TLC_OK;
 }
 
+static constexpr uint32_t VICINITY_BATCH_FLAGS = TLC_F_NORM | TLC_F_NORM_EPS | TLC_F_SUM_PLAIN | TLC_F_FILT_ANY_STRUCT;
+
+int tlc_vicinity_batch_dev(tlc_graph* g, const int32_t* dev_targets, int64_t E, const tlc_params* p,
+                           tlc_vicinity_batch* out, uint8_t* dev_status, int64_t* total_v, int64_t* total_e) {
+  if (!g) return fail(TLC_E_INVALID, "graph is NULL");
+  if (!out || !out->voff || !out->eoff) return fail(TLC_E_INVALID, "out, out->voff and out->eoff are required");
+  if (out->cap_v < 0 || out->cap_e < 0) return fail(TLC_E_INVALID, "out->cap_v and out->cap_e must be >= 0");
+  if (E < 0 || E >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "E must be in [0, 2^31)");
+  if (E > 0 && !dev_targets) return fail(TLC_E_INVALID, "targets is NULL");
+  if (!p) return fail(TLC_E_INVALID, "params is NULL");
+  if (p->flags & ~VICINITY_BATCH_FLAGS)
+    return fail(TLC_E_INVALID, "flags may only hold TLC_F_NORM, TLC_F_NORM_EPS, TLC_F_SUM_PLAIN and the TLC_F_FILT_* filtrations");
+  tlc_params q = *p;  // (resolution and img_mask are ignored)
+  q.resolution = 1;
+  q.img_mask = 0;
+  int rc = check_params(&q);
+  if (rc) return rc;
+  CK(cudaSetDevice(g->device));
+  cudaStream_t st = g->stream;
+  BatchCollect& b = g->vb;
+  b.out = *out;
+  b.status = dev_status;
+  b.total_v = 0; b.total_e = 0;
+  if (E == 0) {
+    CK(cudaMemsetAsync(out->voff, 0, 8, st));
+    CK(cudaMemsetAsync(out->eoff, 0, 8, st));
+    CK(cudaStreamSynchronize(st));
+    g->last = CallStats();
+  } else {
+    CallStats s;
+    b.on = true;
+    rc = run_staged(g, dev_targets, E, &q, nullptr, nullptr, dev_status, nullptr, nullptr, s, 0);
+    b.on = false;
+    g->last = s;
+    if (rc == TLC_OK) {
+      CK(cudaStreamSynchronize(st));
+      CK(cudaGetLastError());
+    }
+  }
+  if (total_v) *total_v = b.total_v;
+  if (total_e) *total_e = b.total_e;
+  return rc;
+}
+
 int tlc_ollivier_ricci(int device, int32_t N, int64_t nnz, const int32_t* rowptr, const int32_t* col, double alpha,
                        double* out_kappa, int32_t* out_iters) {
   if (N <= 0 || nnz < 0 || !rowptr || (nnz > 0 && (!col || !out_kappa))) return fail(TLC_E_INVALID, "bad arguments");
@@ -2133,9 +2233,8 @@ static int graph_route(int64_t n, int64_t m) {
   return 3;
 }
 
-static int check_graph_batch(int64_t D, const int64_t* noff, const int64_t* eoff, const int32_t* ea, const int32_t* eb) {
-  if (D < 0 || D >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "D must be in [0, 2^31)");
-  if (!noff || !eoff) return fail(TLC_E_INVALID, "noff and eoff are required");
+// the host-side part of both creations' checks: the offsets (host copies)
+static int check_batch_offsets(int64_t D, const int64_t* noff, const int64_t* eoff) {
   if (noff[0] != 0 || eoff[0] != 0) return fail(TLC_E_INVALID, "noff[0] and eoff[0] must be 0");
   for (int64_t t = 0; t < D; t++) {
     if (noff[t + 1] < noff[t]) return fail(TLC_E_INVALID, "noff is not monotone at graph " + std::to_string(t));
@@ -2143,6 +2242,14 @@ static int check_graph_batch(int64_t D, const int64_t* noff, const int64_t* eoff
   }
   if (noff[D] >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "noff[D] must be < 2^31");
   if (eoff[D] >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "eoff[D] must be < 2^31");
+  return TLC_OK;
+}
+
+static int check_graph_batch(int64_t D, const int64_t* noff, const int64_t* eoff, const int32_t* ea, const int32_t* eb) {
+  if (D < 0 || D >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "D must be in [0, 2^31)");
+  if (!noff || !eoff) return fail(TLC_E_INVALID, "noff and eoff are required");
+  const int rc = check_batch_offsets(D, noff, eoff);
+  if (rc) return rc;
   const int64_t M = eoff[D];
   if (M > 0 && (!ea || !eb)) return fail(TLC_E_INVALID, "ea and eb are required when there are edges");
   std::vector<std::pair<uint64_t, int64_t>> keys((size_t)M);
@@ -2209,7 +2316,7 @@ static int graph_batch_upload(tlc_graph_batch* b, const int64_t* noff, const int
   const int64_t DL = (int64_t)l_tidx.size();
   auto up = [&](DevBuf& buf, const void* src, size_t bytes) -> cudaError_t {
     cudaError_t e = buf.reserve(bytes);
-    if (e == cudaSuccess && bytes) e = cudaMemcpy(buf.p, src, bytes, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && bytes) e = cudaMemcpy(buf.p, src, bytes, cudaMemcpyDefault);  // (host or device sources)
     return e;
   };
   CK(up(b->noff, noff, (size_t)(D + 1) * 8));
@@ -2276,6 +2383,62 @@ int tlc_graph_batch_create(int device, int64_t D, const int64_t* noff, const int
   b->device = device;
   b->D = D; b->N = noff[D]; b->M = eoff[D];
   rc = graph_batch_upload(b, noff, eoff, ea, eb);
+  if (rc != TLC_OK) { delete b; return rc; }
+  *out = b;
+  return TLC_OK;
+}
+
+int tlc_graph_batch_create_dev(int device, int64_t D, const int64_t* dev_noff, const int64_t* dev_eoff,
+                               const int32_t* dev_ea, const int32_t* dev_eb, void* stream, tlc_graph_batch** out) {
+  if (!out) return fail(TLC_E_INVALID, "out is NULL");
+  if (D < 0 || D >= ((int64_t)1 << 31)) return fail(TLC_E_INVALID, "D must be in [0, 2^31)");
+  if (!dev_noff || !dev_eoff) return fail(TLC_E_INVALID, "noff and eoff are required");
+  int rc = select_device(device);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  std::vector<int64_t> noff((size_t)D + 1), eoff((size_t)D + 1);
+  CK(cudaMemcpyAsync(noff.data(), dev_noff, (size_t)(D + 1) * 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(eoff.data(), dev_eoff, (size_t)(D + 1) * 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  if ((rc = check_batch_offsets(D, noff.data(), eoff.data()))) return rc;
+  const int64_t M = eoff[(size_t)D];
+  if (M > 0 && (!dev_ea || !dev_eb)) return fail(TLC_E_INVALID, "ea and eb are required when there are edges");
+  if (M > 0) {
+    cudaDeviceProp prop;
+    CK(cudaGetDeviceProperties(&prop, device));
+    DevBuf first;
+    CK(first.reserve(8));
+    unsigned long long h_first = 0;
+    CK(cudaMemsetAsync(first.p, 0xff, 8, st));
+    launch_batch_check(D, M, dev_noff, dev_eoff, dev_ea, dev_eb, first.as<unsigned long long>(), prop.multiProcessorCount, st);
+    CK(cudaMemcpyAsync(&h_first, first.p, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaGetLastError());
+    if (h_first != ~0ull) {  // the message of tlc_graph_batch_create for the first offending edge
+      const int64_t k = (int64_t)(h_first >> 2);
+      const int reason = (int)(h_first & 3);
+      int32_t e[4] = {0, 0, 0, 0};  // ea / eb of edges k - 1 and k
+      const int64_t k0 = k > 0 ? k - 1 : k;
+      CK(cudaMemcpy(e, dev_ea + k0, (size_t)(k - k0 + 1) * 4, cudaMemcpyDeviceToHost));
+      CK(cudaMemcpy(e + 2, dev_eb + k0, (size_t)(k - k0 + 1) * 4, cudaMemcpyDeviceToHost));
+      const int64_t a = e[k - k0], bb = e[2 + k - k0];
+      const int64_t t = std::upper_bound(eoff.begin(), eoff.end(), k) - eoff.begin() - 1;
+      const std::string what = "edge " + std::to_string(k) + " (" + std::to_string(a) + ", " + std::to_string(bb) +
+                               ") of graph " + std::to_string(t);
+      if (reason == BATCH_BAD_RANGE)
+        return fail(TLC_E_INVALID, what + " has an endpoint outside the graph's vertices [" + std::to_string(noff[(size_t)t]) +
+                                       ", " + std::to_string(noff[(size_t)t + 1]) + ")");
+      if (reason == BATCH_BAD_LOOP) return fail(TLC_E_INVALID, what + " is a self-loop");
+      if (reason == BATCH_BAD_ORIENT) return fail(TLC_E_INVALID, what + " has ea > eb (canonical form needs ea < eb)");
+      if (e[0] == a && e[2] == bb) return fail(TLC_E_INVALID, what + " repeats edge " + std::to_string(k - 1));
+      return fail(TLC_E_INVALID, what + " is not after edge " + std::to_string(k - 1) + " (" + std::to_string(e[0]) + ", " +
+                                     std::to_string(e[2]) + "): canonical form needs the edges strictly ascending in (ea, eb)");
+    }
+  }
+  tlc_graph_batch* b = new tlc_graph_batch();
+  b->device = device;
+  b->D = D; b->N = noff[(size_t)D]; b->M = M;
+  rc = graph_batch_upload(b, noff.data(), eoff.data(), dev_ea, dev_eb);
   if (rc != TLC_OK) { delete b; return rc; }
   *out = b;
   return TLC_OK;

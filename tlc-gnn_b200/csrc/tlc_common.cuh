@@ -480,6 +480,21 @@ void launch_graph_export(const GraphBatchView& b, const ChunkView& c, int sm_cou
 void launch_graph_grad(const GraphBatchView& b, const int64_t* poff, const int32_t* bv, const int32_t* dv, const double* gb,
                        const double* gd, int32_t* cnt, int32_t* lst, double* grad_f, int sm_count, cudaStream_t st);
 
+// kernel 10 (k10_vicinity_batch.cu): vicinities in graph-batch layout (tlc_vicinity_batch_dev) and the device-side check
+// of a graph batch in canonical form (tlc_graph_batch_create_dev).
+// export: chunk target t's vertices, edges (local id + voff[row]) and filtration values to voff[row] / eoff[row], row =
+// c.tidx[t]; its final status (a connected check over its edges turns OK / TRIVIAL into DISCONNECTED) to status[row].
+// bad_desc: every OK / TRIVIAL target reports BAD_DESCRIPTOR (written by the host) and gets NaN values.  NULL arrays are
+// skipped.
+void launch_vicinity_export(const ChunkView& c, const int64_t* voff, const int64_t* eoff, int32_t* vert, int32_t* ea,
+                            int32_t* eb, double* fval, uint8_t* status, int bad_desc, cudaStream_t st);
+// the first edge k (in index order) that breaks canonical form, as first = k * 4 + reason (reason: 0 endpoint outside its
+// graph, 1 self-loop, 2 ea > eb, 3 not strictly after edge k - 1); first is left as it was (all ones) when there is none.
+// noff / eoff must be monotone (checked on the host).
+constexpr int BATCH_BAD_RANGE = 0, BATCH_BAD_LOOP = 1, BATCH_BAD_ORIENT = 2, BATCH_BAD_ORDER = 3;
+void launch_batch_check(int64_t D, int64_t M, const int64_t* noff, const int64_t* eoff, const int32_t* ea, const int32_t* eb,
+                        unsigned long long* first, int sm_count, cudaStream_t st);
+
 // multi-GPU exchange by peer stores (k5_gather.cu): the tables of all ranks, this rank's own included
 constexpr int PEER_MAX = 16;
 constexpr size_t PEER_HEADER_BYTES = 256;  // [u32 arrival counter | pad] in front of the float32 rows

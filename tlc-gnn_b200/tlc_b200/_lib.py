@@ -36,7 +36,8 @@ EXPORTS = ["tlc_graph_create", "tlc_graph_destroy", "tlc_vicinity_pi", "tlc_vici
            "tlc_vicinity_diagrams_dev", "tlc_pimg_batch_dev", "tlc_pimg_batch_grad_dev",
            "tlc_wasserstein_workspace_bytes", "tlc_wasserstein_batch_dev", "tlc_wasserstein_batch_grad_dev",
            "tlc_graph_batch_create", "tlc_graph_batch_destroy", "tlc_graph_batch_pair_bound",
-           "tlc_graph_batch_diagrams_dev", "tlc_graph_batch_grad_dev"]
+           "tlc_graph_batch_diagrams_dev", "tlc_graph_batch_grad_dev", "tlc_vicinity_batch_dev",
+           "tlc_graph_batch_create_dev"]
 
 
 class Params(C.Structure):
@@ -62,6 +63,12 @@ class Diagrams(C.Structure):
     """tlc_diagrams: the pair arrays of tlc_vicinity_diagrams(_dev), host or device addresses"""
     _fields_ = [("cap", C.c_int64), ("poff", C.c_void_p), ("npairs", C.c_void_p), ("kind", C.c_void_p),
                 ("bv", C.c_void_p), ("dv", C.c_void_p), ("birth", C.c_void_p), ("death", C.c_void_p)]
+
+
+class VicinityBatch(C.Structure):
+    """tlc_vicinity_batch: the graph-batch layout of tlc_vicinity_batch_dev, device addresses"""
+    _fields_ = [("cap_v", C.c_int64), ("cap_e", C.c_int64), ("voff", C.c_void_p), ("eoff", C.c_void_p),
+                ("vert", C.c_void_p), ("ea", C.c_void_p), ("eb", C.c_void_p), ("fval", C.c_void_p)]
 
 
 class TlcError(RuntimeError):
@@ -119,6 +126,11 @@ def lib():
     L.tlc_graph_batch_diagrams_dev.argtypes = [vp, vp, u32, C.POINTER(Diagrams), vp, vp]
     L.tlc_graph_batch_grad_dev.restype = C.c_int
     L.tlc_graph_batch_grad_dev.argtypes = [vp, C.POINTER(Diagrams), vp, vp, vp, vp]
+    L.tlc_vicinity_batch_dev.restype = C.c_int
+    L.tlc_vicinity_batch_dev.argtypes = [vp, vp, i64, C.POINTER(Params), C.POINTER(VicinityBatch), vp, C.POINTER(i64),
+                                         C.POINTER(i64)]
+    L.tlc_graph_batch_create_dev.restype = C.c_int
+    L.tlc_graph_batch_create_dev.argtypes = [C.c_int, i64, vp, vp, vp, vp, vp, C.POINTER(vp)]
     L.tlc_last_error.restype = C.c_char_p
     L.tlc_version.restype = C.c_char_p
     L.tlc_launch_count.restype = i64

@@ -260,6 +260,47 @@ class VicinityGraph:
         out.update(status=status, pi=pi)
         return out
 
+    # ---- vicinities in graph-batch layout (include/tlc_b200.h: tlc_vicinity_batch_dev) ----
+    _batch_cap = (0, 0)  # grow-only guess of the vertex / edge capacities
+
+    def vicinity_batch_dev(self, targets_dev, hop=2, mode=L.MODE_EDGE, descriptor="sum", flags=L.F_NORM, fval=True):
+        """the vicinities of a batch and their filtration in graph-batch (PyG Batch) layout, device buffers: targets_dev
+        int32[E, 2] (torch, this graph's device) -> dict of CUDA tensors ptr / eptr int64[E+1] (target t's vertices are
+        [ptr[t], ptr[t+1]), its edges [eptr[t], eptr[t+1])), vert int32 (graph ids, ascending inside a target),
+        edge_index int32[2, M] (batch ids, row 0 < row 1, lexicographic inside a target: canonical form, ready for
+        GraphBatch.from_device), fval float64 (the filtration tlc_vicinity_detail computes; NaN for every target whose
+        status is neither OK nor TRIVIAL) or None with fval=False (no filtration is computed), and status uint8[E].
+        flags: F_NORM, F_NORM_EPS, F_SUM_PLAIN and the F_FILT_* filtrations.  A call that needs more room than the
+        grow-only guess is repeated once with the exact totals, as vicinity_diagrams_dev does."""
+        import torch
+        E = int(targets_dev.shape[0])
+        dev = torch.device("cuda", self.device)
+        tp = _dev_ptr(targets_dev, "int32", (E, 2), self.device, "targets_dev") if E else None
+        p = make_params(hop, mode, descriptor, 5, flags, 0)
+        ptr = torch.zeros(E + 1, dtype=torch.int64, device=dev)
+        eptr = torch.zeros(E + 1, dtype=torch.int64, device=dev)
+        status = torch.zeros(E, dtype=torch.uint8, device=dev)
+        tv, te = C.c_int64(0), C.c_int64(0)
+        cap_v, cap_e = self._batch_cap
+        for attempt in range(2):
+            vert = torch.empty(cap_v, dtype=torch.int32, device=dev)
+            ei = torch.empty((2, cap_e), dtype=torch.int32, device=dev)
+            fv = torch.empty(cap_v, dtype=torch.float64, device=dev) if fval else None
+            torch.cuda.synchronize(dev)  # (the library works on its own stream)
+            b = L.VicinityBatch(cap_v, cap_e, ptr.data_ptr(), eptr.data_ptr(), vert.data_ptr(), ei[0].data_ptr(),
+                                ei[1].data_ptr(), fv.data_ptr() if fv is not None else None)
+            rc = L.lib().tlc_vicinity_batch_dev(self._h, tp, E, C.byref(p), C.byref(b), status.data_ptr() if E else None,
+                                                C.byref(tv), C.byref(te))
+            if rc == L.E_CAPACITY and attempt == 0:
+                cap_v, cap_e = int(tv.value), int(te.value)
+                continue
+            L.check(rc)
+            break
+        V, M = int(tv.value), int(te.value)
+        self._batch_cap = (max(self._batch_cap[0], cap_v), max(self._batch_cap[1], cap_e))
+        return dict(ptr=ptr, eptr=eptr, vert=vert[:V], edge_index=ei if M == cap_e else ei[:, :M].contiguous(),
+                    fval=fv[:V] if fv is not None else None, status=status)
+
     # ---- multi-GPU exchange by peer stores (include/tlc_b200.h: tlc_table_*) ----
     def table_create(self, rows, resolution=5):
         """this rank's exchange table float32[rows][res^2 + 1]: -> (device address of row 0, 64-byte CUDA IPC handle)"""
@@ -656,6 +697,55 @@ class GraphBatch:
         bound = C.c_int64(0)
         L.check(L.lib().tlc_graph_batch_pair_bound(self._h, C.byref(bound)))
         self.pair_bound = int(bound.value)
+
+    @classmethod
+    def from_device(cls, ptr, edge_index, device=0):
+        """the same batch from structure already on the GPU: ptr int64[D+1] and edge_index int32 (or int64) [2, M], CUDA
+        tensors on `device`, in CANONICAL FORM -- inside every graph edge_index[0] < edge_index[1] and the edges strictly
+        ascending in (edge_index[0], edge_index[1]), graphs one after the other.  VicinityGraph.vicinity_batch_dev's ptr /
+        edge_index are in this form.  A PyG batch (N = ptr[-1] vertices, graphs on consecutive vertex ranges) is
+        canonicalised on the device with
+            lo, hi = torch.minimum(edge_index[0], edge_index[1]), torch.maximum(edge_index[0], edge_index[1])
+            key = torch.unique(lo * N + hi)              # sorted; drops repeats and the reverse directions
+            edge_index = torch.stack([key // N, key % N]).to(torch.int32)
+        (self-loops stay, and are rejected).  That order, not the input order, is then the sweeps' tie-break, whereas
+        GraphBatch(ptr, edge_index) keeps the first occurrence of every edge in input order.  Input that is not in
+        canonical form raises TlcError with the library's message naming the graph and the first offending edge.  The
+        structure is checked on the device (O(M), no sort); the call synchronises with the current stream."""
+        import torch
+        device = int(device)
+        if getattr(ptr, "dim", lambda: 0)() != 1 or ptr.shape[0] < 1:
+            raise ValueError("ptr must be 1-D with D + 1 >= 1 entries")
+        if getattr(edge_index, "dim", lambda: 0)() != 2 or edge_index.shape[0] != 2:
+            raise ValueError("edge_index must have shape [2, M], got %s" % (tuple(getattr(edge_index, "shape", ())),))
+        D, M = int(ptr.shape[0]) - 1, int(edge_index.shape[1])
+        _dev_ptr(ptr, "int64", (D + 1,), device, "ptr")
+        if edge_index.dtype == torch.int64:
+            if M and bool(((edge_index < 0) | (edge_index >= 2 ** 31)).any()):
+                raise ValueError("edge_index holds ids outside [0, 2^31)")
+            edge_index = edge_index.to(torch.int32)
+        _dev_ptr(edge_index.contiguous(), "int32", (2, M), device, "edge_index")
+        ea, eb = edge_index[0].contiguous(), edge_index[1].contiguous()
+        # graph t's edges start at the first edge whose ea reaches ptr[t] (ea is ascending in canonical form; the library
+        # rejects edges that end up outside their graph or out of order otherwise)
+        eoff = torch.searchsorted(ea.to(torch.int64), ptr).contiguous()
+        if D >= 0:
+            eoff[0] = 0
+            eoff[D] = M
+        self = cls.__new__(cls)
+        self.noff, self.eoff, self.ea, self.eb = ptr, eoff, ea, eb
+        self.D, self.device = D, device
+        self._h = C.c_void_p()
+        st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+        L.check(L.lib().tlc_graph_batch_create_dev(device, D, ptr.data_ptr(), eoff.data_ptr(),
+                                                   ea.data_ptr() if M else None, eb.data_ptr() if M else None, st,
+                                                   C.byref(self._h)))
+        self.N = int(ptr[-1].item())
+        self.M = M
+        bound = C.c_int64(0)
+        L.check(L.lib().tlc_graph_batch_pair_bound(self._h, C.byref(bound)))
+        self.pair_bound = int(bound.value)
+        return self
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
